@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- space-time simplices tested per second (BASELINE.json metric) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c5|woven] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c5|woven] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one advance_timestep of the tracker on one new snapshot: field derivation (gradient +
 min non-zero |v|), quantisation factor, ordinal sweep at t and interval sweep over [t, t+1]
@@ -29,6 +29,10 @@ north_star names.  --only-main skips them.
 
 --impl reference times the unmodified reference CPU tracker (oracle/_ref/ftk_ref_oracle, built from
 /root/reference by oracle/build_ref.sh) on a bounded sample of the same workload.
+
+--dump-outputs DIR writes what a caller of the timed path receives after its last step: the punctured simplices the
+tracker of the main workload holds then (DIR/points_<field>.npy, float64, one file per field of the point record).  The
+inputs are generated without randomness, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -59,6 +63,9 @@ VECTOR_CONFIGS = ("c4", "c5", "c4s")
 WOVEN_CONFIGS = ("woven", "wovens")
 METRIC = "space_time_simplices_tested_per_sec"
 UNIT = "simplices/s"
+# --dump-outputs: a point is 14 float64 values (112 bytes); counting 128 bytes a point leaves room for the .npy headers
+# and keeps a dump under 64 MB
+DUMP_POINTS_MAX = (64 << 20) // 128
 
 
 def tri(g, period):
@@ -309,8 +316,20 @@ def generate_layers(env, config):
     return layers
 
 
-def run_config(env, config, K, W, e2e_steps, sample_clocks):
-    """time K sweeps of `config` on this rank (after W warm-up sweeps); returns the rank-0 record"""
+def dump_points(out_dir, pts):
+    """the punctured simplices in the element order the library returns them, one float64 array per field of the point
+    record; above DUMP_POINTS_MAX a fixed, seeded sample of them, still in that order"""
+    import numpy as np
+    if len(pts) > DUMP_POINTS_MAX:
+        pts = pts[np.sort(np.random.default_rng(0).choice(len(pts), DUMP_POINTS_MAX, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for field in pts.dtype.names:
+        np.save(os.path.join(out_dir, f"points_{field}.npy"), pts[field].astype(np.float64))
+
+
+def run_config(env, config, K, W, e2e_steps, sample_clocks, dump_dir=None):
+    """time K sweeps of `config` on this rank (after W warm-up sweeps); returns the rank-0 record.  dump_dir: write the
+    punctured simplices the tracker holds after its last timed sweep there (dump_points)"""
     import numpy as np
     import torch
     import ftk_b200
@@ -478,6 +497,8 @@ def run_config(env, config, K, W, e2e_steps, sample_clocks):
                "library": after["ms_sort_wall"] + after["ms_trace_wall"]}
     finalize_ms = 1e3 * (time.perf_counter() - t0)
     tr.close()
+    if dump_dir and rank == 0:
+        dump_points(dump_dir, pts)
 
     # ---- end-to-end measurement: host buffers through the same C-ABI calls ------------------------
     ms2, E, st2 = None, 0, None
@@ -650,23 +671,28 @@ def self_check(env):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=252)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: 252; 20 with --impl reference)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--config", default="c2", choices=sorted(CONFIGS))
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--e2e-steps", type=int, default=24)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--only-main", action="store_true", help="skip the scaling_c4 / scaling_c3 / dense_woven sub-records and the N > 1 self-check")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the punctured simplices of the main workload after its last timed step as DIR/points_<field>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
 
     if args.impl == "reference":
-        if args.steps == 252:
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the CUDA path computed; --impl reference has no such output")
+        if args.steps is None:
             args.steps = 20   # default sized so the whole run ends within a few minutes
         reference_arm(args, rank)
         return
+    if args.steps is None:
+        args.steps = 252
     if args.warmup < 3:
         args.warmup = 3
     # stdout carries exactly one JSON line: anything a library prints there (NCCL's version banner) goes to stderr
@@ -692,7 +718,7 @@ def main():
         env.dist = dist
 
     t_all = time.perf_counter()
-    line = run_config(env, args.config, args.steps, args.warmup, args.e2e_steps, sample_clocks=True)
+    line = run_config(env, args.config, args.steps, args.warmup, args.e2e_steps, sample_clocks=True, dump_dir=args.dump_outputs)
     if line is not None:
         line["config"]["host_cpus_bound_per_rank"] = int(numa_cpus)     # CPUs next to the rank's GPU (0: affinity left alone)
     extras = {}
