@@ -20,7 +20,6 @@
 #include <atomic>
 #include <vector>
 
-#include <future>
 #include <memory>
 #include "kernels.h"
 #include "online.h"
@@ -78,13 +77,10 @@ struct ftkb_ctx {
   int nbits = 0;
   int next_slot = 0;
   int sm_count = 148;
-  int scan_mode = 2;             // FTKB_SCAN=ldg|warp|tile|direct selects the fused 2D scan's staging (A/B measurements); default tile
-                                 // (direct = no shared memory, 16-byte loads + shuffles: measured 0.259 ms vs 0.188 ms on C2)
-  bool cellsV = true;            // same for vector input (field GIVEN); FTKB_VSCAN=twolayer re-reads both layers and runs the resolution pass
-  bool cells2d = true;           // same for the fused 2D tile scan; FTKB_SCAN2D=twolayer re-reads both layers every step
+  bool cellsV = true;            // vector input (field GIVEN): each layer is streamed once and keeps its range cells;
+                                 // FTKB_VSCAN=twolayer re-reads both layers every step and runs the resolution pass
   bool keys2d = true;            // 2D scalar build kernel keeps high-word keys of the differences (no fp64->fp32 conversions);
                                  // FTKB_SCAN2D=f32 (or a poisoned layer: NaN / Inf / >= 2^1000) selects the fp32-range build kernel
-  bool cells3d = true;           // fused 3D scan streams each layer once and keeps its range cells; FTKB_SCAN3D=twolayer re-reads both layers every step
   std::vector<uint4 *> freeCells;
   std::vector<uint4 *> exportedCells;   // handed to a peer process (ftkb_export_layer_cells): freed at destroy only
   size_t ncells = 0;             // cells per layer (fixed by the dims)
@@ -128,7 +124,6 @@ struct ftkb_ctx {
   std::vector<float> gaps, tl_scan_end, tl_test_end;
   cudaEvent_t dbg_prev = nullptr; bool dbg_prev_valid = false;
   double host_wait_us = 0, host_enq_us = 0; uint64_t host_wait_n = 0, host_enq_n = 0;
-  bool overlap_test = true;          // FTKB_TEST_OVERLAP=0: test kernels stay on the sweep's stream
   bool last_test_overlapped = false; // where the previous deferred step's test kernel went
   bool has_producer = false;
 
@@ -169,10 +164,6 @@ struct ftkb_ctx {
   bool streaming = false;
   std::unique_ptr<ftkb::OnlineTracer> online;
   uint64_t grown = 0;            // d_pts[0 .. grown) have been through a grow step
-  // FTKB_STREAM_GROW=async: the grow step of sweep k runs on a worker while the caller produces / pushes the next snapshot
-  // and the device sweeps step k+1; at most one is in flight, and everything that reads `online` or the host-trace time
-  // joins it first.  Default: inline.
-  std::future<double> grow_task;
   bool grow_failed = false;      // a grow step threw: every later call that depends on the trajectories reports it
 
   ftkb_stats stats{};
@@ -266,13 +257,11 @@ static void release_layer(ftkb_ctx *c, Layer &l) {
   l = Layer();
 }
 
-static int wait_grow(ftkb_ctx *c);
 static void fill_trace_params(const ftkb_ctx *c, TraceParams &tp);
 static int drain(ftkb_ctx *c);
 
 extern "C" void ftkb_destroy(ftkb_ctx *c) {
   if (!c) return;
-  (void)wait_grow(c);
   if (c->debug_timing && c->gaps.size() > 8) {
     auto med = [](std::vector<float> v) { std::sort(v.begin(), v.end()); return 1e3 * v[v.size() / 2]; };
     std::fprintf(stderr, "[ftkb] deferred steps, relative to the previous scan's end (medians over %zu): scan starts +%.1f us, ends +%.1f us, test ends +%.1f us\n",
@@ -347,20 +336,16 @@ extern "C" int ftkb_create(const ftkb_config *cfg, ftkb_ctx **out) {
   c->cfg = *cfg;
   c->slab = cfg->slab_global_dim != 0;
   c->sm_count = prop.multiProcessorCount > 0 ? prop.multiProcessorCount : 148;
-  if (const char *e = std::getenv("FTKB_SCAN")) c->scan_mode = std::string(e) == "ldg" ? 0 : (std::string(e) == "warp" ? 1 : (std::string(e) == "direct" ? 3 : 2));
   {
     // the fused 3D scan needs TMA-compatible rows (W even) and the exact early-out (robust detection on)
     const char *e = std::getenv("FTKB_SCAN3D");
     c->fused3d = n == 3 && cfg->vector_source == FTKB_SOURCE_DERIVED && cfg->robust_detection && cfg->dims[0] % 2 == 0 &&
                  !(e && std::string(e) == "plain");
-    c->cells3d = !(e && std::string(e) == "twolayer");
     const char *ev = std::getenv("FTKB_VSCAN");
     c->cellsV = cfg->vector_source == FTKB_SOURCE_GIVEN && !(n == 3 && !cfg->robust_detection) && (n == 2 || cfg->dims[0] % 2 == 0) &&
                 !(ev && std::string(ev) == "twolayer");
     const char *e2 = std::getenv("FTKB_SCAN2D");
-    c->cells2d = n == 2 && cfg->vector_source == FTKB_SOURCE_DERIVED && c->scan_mode >= 2 && !(e2 && std::string(e2) == "twolayer");
     c->keys2d = !(e2 && std::string(e2) == "f32");
-    if (n == 2 && c->scan_mode == 3 && !c->cells2d) c->scan_mode = 2;      // the direct staging exists as a cell scan only
   }
   c->n = n;
   c->nvert = (size_t)cfg->dims[0] * cfg->dims[1] * (n == 3 ? cfg->dims[2] : 1);
@@ -406,7 +391,6 @@ extern "C" int ftkb_create(const ftkb_config *cfg, ftkb_ctx **out) {
     cudaDeviceGetStreamPriorityRange(&lo, &hi);
     if ((e = cudaStreamCreateWithPriority(&c->stream2, cudaStreamNonBlocking, hi)) != cudaSuccess) return bail(std::string("cudaStreamCreate: ") + cudaGetErrorString(e), FTKB_ERR_CUDA);
     if ((e = cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming)) != cudaSuccess) return bail(std::string("cudaEventCreate: ") + cudaGetErrorString(e), FTKB_ERR_CUDA);
-    if (const char *o = std::getenv("FTKB_TEST_OVERLAP")) c->overlap_test = std::string(o) != "0";
     if (const char *o = std::getenv("FTKB_DEBUG_TIMING")) c->debug_timing = std::string(o) == "1";
     if (c->debug_timing) cudaEventCreate(&c->dbg_prev);
   }
@@ -694,8 +678,6 @@ static void fill_sweep_geometry(const ftkb_ctx *c, SweepParams &p) {
   p.coords = c->d_coords;
   p.nd = c->n;
   p.sm_count = c->sm_count;
-  static const int l2_hint = [] { const char *e = std::getenv("FTKB_K2_L2HINT"); return e ? std::atoi(e) : 0; }();
-  p.l2_hint = l2_hint;
   p.W = c->cfg.dims[0]; p.H = c->cfg.dims[1]; p.D = c->n == 3 ? c->cfg.dims[2] : 1;
   for (int j = 0; j < 3; j++) {
     const bool used = j < c->n;
@@ -707,9 +689,8 @@ static void fill_sweep_geometry(const ftkb_ctx *c, SweepParams &p) {
   }
   // scalar build kernels: key filter of the layer's min non-zero |v| against the running minimum known now (kernels.h);
   // gradient2D scales the differences by W - 1 / H - 1 (grad.hh:24-27), gradient3D halves them (grad.hh:140-144)
-  static const bool res_filter = [] { const char *e = std::getenv("FTKB_RES_FILTER"); return !(e && std::string(e) == "0"); }();
   for (int j = 0; j < 3; j++)
-    p.res_thr[j] = !res_filter ? __builtin_inff() : res_threshold_key(c->resolution, c->n == 2 ? (double)(c->cfg.dims[j < 2 ? j : 0] - 1) : 0.5);
+    p.res_thr[j] = res_threshold_key(c->resolution, c->n == 2 ? (double)(c->cfg.dims[j < 2 ? j : 0] - 1) : 0.5);
   if (c->slab) {           // a z-slab of a larger array: ranks / positions / corners in the whole lattice's frame
     p.voff[2] = c->cfg.slab_offset;
     p.rank_lb[2] = c->cfg.slab_global_lb;
@@ -717,81 +698,52 @@ static void fill_sweep_geometry(const ftkb_ctx *c, SweepParams &p) {
   }
 }
 
-// strips x row chunks of the fused 2D scan: about two equal waves of warps over the resident slots
-static void fused2d_decomposition(const ftkb_ctx *c, SweepParams &p) {
-  // bulk-async kernel: 62 corner columns per strip, 3 blocks of 8 warps per SM; register kernel: 60, 2 blocks
-  p.bulk = p.aligned16 ? c->scan_mode : 0;
-  int64_t nsy;
-  if (p.bulk == 3) {
-    // direct staging: warps = strips of 62 corner columns x row chunks (multiples of the 8-row cell block); two CTAs of
-    // 8 warps per SM, about six waves
-    const int R = VSCAN2D_CELL_ROWS;
-    p.nsx = std::max(1, (p.W + 61) / 62);
-    const int64_t want = std::max<int64_t>(1, (6 * (int64_t)c->sm_count * 16) / p.nsx);
-    p.rows = std::max(2 * R, (int)((p.H + want - 1) / want));
-    p.rows = (p.rows + R - 1) / R * R;
-    if (const char *e = std::getenv("FTKB_C2_ROWS")) p.rows = std::max(R, std::atoi(e) / R * R);   // A/B measurements
-    p.nsy = (p.H + p.rows - 1) / p.rows;
-    p.nsz = 1;
-    return;
-  }
-  if (p.bulk == 2) {      // CTA tiles of 7 x 62 corner columns, 3 CTAs per SM: about two waves of CTAs
-    p.nsx = std::max(1, (p.W + 7 * 62 - 1) / (7 * 62));
-    nsy = (2 * (int64_t)c->sm_count * 3) / p.nsx;          // floor: a few CTAs more than two waves would cost a third one
-  } else {
-    p.nsx = p.bulk ? std::max(1, (p.W + 61) / 62) : std::max(1, (p.W - 1 + 59) / 60);
-    const int64_t resident_warps = (int64_t)c->sm_count * (p.bulk ? 3 : 2) * 8;
-    nsy = (2 * resident_warps) / p.nsx;
-  }
-  nsy = std::max<int64_t>(1, std::min<int64_t>(nsy, (p.H + 31) / 32));
-  p.rows = (int)((p.H + nsy - 1) / nsy);
-  if (p.bulk == 2 && c->cells2d) {
+// strips x row chunks of the fused 2D scan.  aligned: 16-byte aligned rows, range-cell kernels on CTA tiles of 7 x 62 corner
+// columns, 3 CTAs per SM; otherwise the register kernel on strips of 60 corner columns, 2 blocks of 8 warps per SM
+static void fused2d_decomposition(const ftkb_ctx *c, SweepParams &p, bool aligned) {
+  if (aligned) {
     // just under eight waves of CTAs (costs differ: border strips, cold paths; the last, partly filled wave runs at low occupancy:
     // measured on C2, rows 36 / 45 / 54 / 63 / 90 = 9.8 / 7.8 / 6.5 / 5.6 / 3.9 waves: 0.153 / 0.145 / 0.148 / 0.150 / 0.163 ms),
     // at least two cell blocks per chunk
     const int R = SCAN2D_CELL_ROWS;
+    p.nsx = std::max(1, (p.W + 7 * 62 - 1) / (7 * 62));
     const int64_t want = std::max<int64_t>(1, (8 * (int64_t)c->sm_count * 3) / p.nsx);
     p.rows = std::max(2 * R, (int)((p.H + want - 1) / want));
     p.rows = (p.rows + R - 1) / R * R;      // chunks start on cell-block boundaries
-    if (const char *e = std::getenv("FTKB_C2_ROWS")) p.rows = std::max(R, std::atoi(e) / R * R);   // A/B measurements
     p.rows = std::min(p.rows, 64 * R);      // the key kernel keeps one fail bit per block of a chunk
+  } else {    // about two equal waves of warps over the resident slots
+    p.nsx = std::max(1, (p.W - 1 + 59) / 60);
+    int64_t nsy = (2 * (int64_t)c->sm_count * 2 * 8) / p.nsx;
+    nsy = std::max<int64_t>(1, std::min<int64_t>(nsy, (p.H + 31) / 32));
+    p.rows = (int)((p.H + nsy - 1) / nsy);
   }
   p.nsy = (p.H + p.rows - 1) / p.rows;
   p.nsz = 1;
 }
 
-// tiles x z chunks of the fused 3D scan: about two equal waves of CTAs (one CTA per SM)
-static void fused3d_decomposition(const ftkb_ctx *c, SweepParams &p, bool cells = false) {
+// tiles x z chunks of the 3D range-cell scans (scalar and vector input)
+static void fused3d_decomposition(const ftkb_ctx *c, SweepParams &p) {
   p.nsx = (p.W + F3_STRIDE - 1) / F3_STRIDE;
   p.nsy = (p.H + F3_TROWS - 1) / F3_TROWS;
   const int64_t tiles = (int64_t)p.nsx * p.nsy;
-  if (c->cells3d || cells) {
-    // two CTAs per SM.  CTA costs differ (edge tiles, cold paths), so aim for about six waves of CTAs and let the
-    // hardware scheduler balance them, but keep at least 16 planes per CTA (3 halo planes are re-read per chunk)
-    const int64_t slots = 2 * (int64_t)c->sm_count;
-    const int64_t nsz = std::max<int64_t>(1, std::min<int64_t>((6 * slots + tiles - 1) / tiles, std::max(1, p.D / 16)));
-    p.rows = (int)((p.D + nsz - 1) / nsz);
-    if (const char *e = std::getenv("FTKB_S3_ROWS")) p.rows = std::max(1, std::min(p.D, std::atoi(e)));   // A/B measurements
-    p.rows = std::min(p.rows, 63);       // the build kernels keep one fail bit per corner plane of a chunk
-    p.nsz = (p.D + p.rows - 1) / p.rows;
-    return;
-  }
-  int64_t nsz = std::max<int64_t>(1, (2 * (int64_t)c->sm_count) / tiles);
-  nsz = std::min<int64_t>(nsz, std::max(1, p.D / 8));
+  // two CTAs per SM.  CTA costs differ (edge tiles, cold paths), so aim for about six waves of CTAs and let the
+  // hardware scheduler balance them, but keep at least 16 planes per CTA (3 halo planes are re-read per chunk)
+  const int64_t slots = 2 * (int64_t)c->sm_count;
+  const int64_t nsz = std::max<int64_t>(1, std::min<int64_t>((6 * slots + tiles - 1) / tiles, std::max(1, p.D / 16)));
   p.rows = (int)((p.D + nsz - 1) / nsz);
+  p.rows = std::min(p.rows, 63);       // the build kernels keep one fail bit per corner plane of a chunk
   p.nsz = (p.D + p.rows - 1) / p.rows;
 }
 
 // vector input, range-cell scan: warps = strips of 62 corner columns x row chunks (2D), tiles x plane chunks (3D)
 static void vcells_decomposition(const ftkb_ctx *c, SweepParams &p) {
-  if (c->n == 3) { fused3d_decomposition(c, p, true); return; }
+  if (c->n == 3) { fused3d_decomposition(c, p); return; }
   // two CTAs of 8 warps per SM, about six waves; chunks are multiples of the cell block
   const int R = VSCAN2D_CELL_ROWS;
   p.nsx = std::max(1, (p.W + 61) / 62);
   const int64_t want = std::max<int64_t>(1, (6 * (int64_t)c->sm_count * 16) / p.nsx);
   p.rows = std::max(2 * R, (int)((p.H + want - 1) / want));
   p.rows = (p.rows + R - 1) / R * R;
-  if (const char *e = std::getenv("FTKB_V2_ROWS")) p.rows = std::max(R, std::atoi(e) / R * R);   // A/B measurements
   p.nsy = (p.H + p.rows - 1) / p.rows;
   p.nsz = 1;
 }
@@ -885,7 +837,6 @@ static int resolve_pending(ftkb_ctx *c, Layer &l) {
   p.has_next = 0;
   p.thrp_f = 1.f; p.thr2_f = 1.f; p.lim_f = 0.f;
   p.L[0].S = l.S; p.L[1].S = l.S;
-  p.aligned16 = rows_aligned16(c, l.S, nullptr);
   p.res_slot[0] = c->d_scalars + l.slot;
   p.wl_count = c->d_scalars + ftkb_ctx::SLOT_WL;
   p.wl = c->d_wl; p.wl_cap = 0;
@@ -896,30 +847,27 @@ static int resolve_pending(ftkb_ctx *c, Layer &l) {
     p.tmap[1] = p.tmap[0];
     CK(cudaMemsetAsync(p.poison, 0, sizeof(unsigned long long), c->stream));
     fused3d_decomposition(c, p);
-    if (c->cells3d) {
-      // stream the layer once: its range cells (with the real domain masks) and min |v|; no cube is tested
-      fill_sweep_geometry(c, p);
-      int rc = ensure_cells(c, l, p);
-      if (rc) return rc;
-      p.sum_mode = SUM_BUILD; p.build_layer = 0; p.sum_out = l.cells;
-      launch_scan3d_cells(p, c->stream);
-      l.cells_valid = true;
-    } else {
-      launch_scan(p, c->stream);
-    }
+    // stream the layer once: its range cells (with the real domain masks) and min |v|; no cube is tested
+    fill_sweep_geometry(c, p);
+    int rc = ensure_cells(c, l, p);
+    if (rc) return rc;
+    p.sum_mode = SUM_BUILD; p.build_layer = 0; p.sum_out = l.cells;
+    launch_scan3d_cells(p, c->stream);
+    l.cells_valid = true;
     c->stats.kernel_launches++;
     CK(cudaMemcpyAsync(c->h_scalars + l.slot, c->d_scalars + l.slot, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
     CK(cudaMemcpyAsync(c->h_scalars + ftkb_ctx::SLOT_POISON, p.poison, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
     c->stats.d2h_bytes += 16;
-    int rc = check_launch(c, "resolution (fused 3D)");
+    rc = check_launch(c, "resolution (fused 3D)");
     if (rc) return rc;
     CK(cudaStreamSynchronize(c->stream));
     l.res_pending = false;
     if (c->h_scalars[ftkb_ctx::SLOT_POISON]) return abandon_fused3d(c);
     return FTKB_OK;
   }
-  fused2d_decomposition(c, p);
-  if (c->cells2d && p.bulk >= 2) {
+  const bool aligned = rows_aligned16(c, l.S, nullptr);
+  fused2d_decomposition(c, p, aligned);
+  if (aligned) {
     // stream the layer once: its range cells and min |v|; no cube is tested
     fill_sweep_geometry(c, p);
     int rc = ensure_cells(c, l, p);
@@ -942,24 +890,19 @@ static int resolve_pending(ftkb_ctx *c, Layer &l) {
 // grow(), critical_point_tracker_2d_regular.hh:288-329 / ..._3d_regular.hh:173-200: the punctured simplices found since
 // the last grow step (the reference clears discrete_critical_points after each) go to the host-side online tracer
 static int wait_grow(ftkb_ctx *c) {
-  if (!c->grow_task.valid()) return c->grow_failed ? FTKB_ERR_NOMEM : FTKB_OK;
-  try { c->stats.ms_finalize_host += c->grow_task.get(); }
-  catch (const std::bad_alloc &) { c->grow_failed = true; return fail(c, FTKB_ERR_NOMEM, "streaming grow step: out of memory (trajectories are incomplete)"); }
-  catch (const std::exception &e) { c->grow_failed = true; return fail(c, FTKB_ERR_INVALID, std::string("streaming grow step: ") + e.what()); }
   return c->grow_failed ? FTKB_ERR_NOMEM : FTKB_OK;
 }
 
 static int grow_trajectories(ftkb_ctx *c) {
   const uint64_t n = c->npts - c->grown;
   if (n >= 0xffffffffull) return fail(c, FTKB_ERR_OVERFLOW, "more than 2^32 punctured simplices in one step");
-  { const int rc = wait_grow(c); if (rc) return rc; }                  // grow steps run in order; the staging buffer is free again
-  // The device prepares the batch (FTKB_STREAM_PREP=host: the host hashes the raw batch instead): element keys -> radix sort ->
-  // unique -> for every element the batch indices of its punctured neighbours, itself included (the same binary search as the
-  // offline trace).  The host walk then only chases index lists (OnlineTracer::grow_sorted).
-  static const bool host_prep = [] { const char *e = std::getenv("FTKB_STREAM_PREP"); return e && std::string(e) == "host"; }();
-  // staging: the raw records (host preparation), or {keys, nine neighbour indices, count} per element -- the records themselves stay on
-  // the device: finalize maps the trajectories' keys onto the sorted points
-  const size_t per = host_prep ? sizeof(ftkb_point) : 8 + 4 * 9 + 1;
+  { const int rc = wait_grow(c); if (rc) return rc; }
+  // The device prepares the batch: element keys -> radix sort -> unique -> for every element the batch indices of its punctured
+  // neighbours, itself included (the same binary search as the offline trace).  The host walk then only chases index lists
+  // (OnlineTracer::grow_sorted).
+  // staging: {keys, nine neighbour indices, count} per element -- the records themselves stay on the device: finalize maps the
+  // trajectories' keys onto the sorted points
+  const size_t per = 8 + 4 * 9 + 1;
   if (n && c->grow_stage_cap < per * n) {
     if (c->grow_stage) cudaFreeHost(c->grow_stage);
   for (ftkb_point *q : c->retired_pts) cudaFree(q);
@@ -968,16 +911,11 @@ static int grow_trajectories(ftkb_ctx *c) {
     if (cudaMallocHost(&c->grow_stage, want) != cudaSuccess) { cudaGetLastError(); return fail(c, FTKB_ERR_NOMEM, "streaming grow step: out of page-locked memory"); }
     c->grow_stage_cap = want;
   }
-  ftkb_point *h_pts = (ftkb_point *)c->grow_stage;
   uint64_t *h_keys = (uint64_t *)c->grow_stage;
   uint32_t *h_nb = (uint32_t *)(h_keys + n);
   uint8_t *h_cnt = (uint8_t *)(h_nb + 9 * n);
   uint64_t nu = n;
-  if (n && host_prep) {
-    CK(cudaMemcpyAsync(h_pts, c->d_pts + c->grown, sizeof(ftkb_point) * n, cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    c->stats.d2h_bytes += sizeof(ftkb_point) * n;
-  } else if (n) {
+  if (n) {
     TraceParams tp{};
     fill_trace_params(c, tp);
     unsigned long long *k0 = nullptr, *k1 = nullptr;
@@ -1010,23 +948,14 @@ static int grow_trajectories(ftkb_ctx *c) {
     c->stats.kernel_launches += 4;
     c->stats.d2h_bytes += per * n + 8;
   }
-  ftkb::OnlineTracer *tracer = c->online.get();
-  const bool prepared = n && !host_prep;
-  auto work = [tracer, prepared, h_pts, h_keys, h_nb, h_cnt, n, nu]() {
+  try {
     const auto t0 = std::chrono::steady_clock::now();
-    if (prepared) tracer->grow_sorted(nullptr, h_keys, (uint32_t)nu, h_nb, h_cnt);
-    else tracer->grow(h_pts, n);
-    return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-  };
-  // FTKB_STREAM_GROW=async: the walk of step k runs on a worker thread behind the sweep of step k+1 and the caller's next
-  // push (it reads the staging buffer, which the next grow step reuses only after joining it).  Default is inline.
-  static const bool async_grow = [] { const char *e = std::getenv("FTKB_STREAM_GROW"); return e && std::string(e) == "async"; }();
-  if (async_grow) c->grow_task = std::async(std::launch::async, work);
-  else {
-    try { c->stats.ms_finalize_host += work(); }
-    catch (const std::bad_alloc &) { c->grow_failed = true; return fail(c, FTKB_ERR_NOMEM, "streaming grow step: out of memory (trajectories are incomplete)"); }
-    catch (const std::exception &e) { c->grow_failed = true; return fail(c, FTKB_ERR_INVALID, std::string("streaming grow step: ") + e.what()); }
+    if (n) c->online->grow_sorted(nullptr, h_keys, (uint32_t)nu, h_nb, h_cnt);
+    else c->online->grow(nullptr, 0);
+    c->stats.ms_finalize_host += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
   }
+  catch (const std::bad_alloc &) { c->grow_failed = true; return fail(c, FTKB_ERR_NOMEM, "streaming grow step: out of memory (trajectories are incomplete)"); }
+  catch (const std::exception &e) { c->grow_failed = true; return fail(c, FTKB_ERR_INVALID, std::string("streaming grow step: ") + e.what()); }
   c->grown = c->npts;
   c->traced = false;
   return FTKB_OK;
@@ -1036,7 +965,6 @@ extern "C" int ftkb_set_streaming_trajectories(ftkb_ctx *c, int enable) {
   if (!c) return FTKB_ERR_INVALID;
   if (c->stats.scan_launches || c->npts) return fail(c, FTKB_ERR_INVALID, "set_streaming_trajectories: call it before the first update_timestep");
   if (c->slab && enable) return fail(c, FTKB_ERR_INVALID, "set_streaming_trajectories: not available on a spatial slab");
-  (void)wait_grow(c);
   c->streaming = enable != 0;
   c->grow_failed = false;
   c->online.reset(c->streaming ? new ftkb::OnlineTracer(c->n, c->cfg.lb, c->cfg.ub) : nullptr);
@@ -1289,6 +1217,7 @@ static int update_impl(ftkb_ctx *c, bool allow_defer) {
   if (has_next && p.scalar_source != FTKB_SOURCE_NONE && !c->layers[1].S) return fail(c, FTKB_ERR_INVALID, "update_timestep: the next snapshot has no scalar field");
   p.fused = fused;
   p.poison = c->d_scalars + ftkb_ctx::SLOT_POISON;
+  const bool aligned = rows_aligned16(c, lay[0]->S, lay[1]->S);    // 2D scalar input: the range-cell kernels need 16-byte aligned rows
   if (fused && c->n == 3) {
     if (!encode_scalar_tmap3d(lay[0]->S, p.W, p.H, p.D, &p.tmap[0]) || !encode_scalar_tmap3d(lay[1]->S, p.W, p.H, p.D, &p.tmap[1])) {
       int rc = drain(c);
@@ -1297,8 +1226,7 @@ static int update_impl(ftkb_ctx *c, bool allow_defer) {
     }
     fused3d_decomposition(c, p);
   } else if (fused) {
-    p.aligned16 = rows_aligned16(c, lay[0]->S, lay[1]->S);
-    fused2d_decomposition(c, p);
+    fused2d_decomposition(c, p, aligned);
   } else if (vcells) {
     vcells_decomposition(c, p);
   } else {
@@ -1317,7 +1245,7 @@ static int update_impl(ftkb_ctx *c, bool allow_defer) {
   p.pt_count = c->d_scalars + ftkb_ctx::SLOT_PT;
   p.ticket = c->d_scalars + ftkb_ctx::SLOT_TICKET;
   p.test_blocks = test_grid(c);
-  const bool cells_path = vcells || (fused && ((c->n == 3 && c->cells3d) || (c->n == 2 && c->cells2d && p.bulk >= 2)));
+  const bool cells_path = vcells || (fused && (c->n == 3 || aligned));
   void (*launch_cells)(const SweepParams &, cudaStream_t) = vcells ? launch_vscan_cells : (c->n == 3 ? launch_scan3d_cells : launch_scan2d_cells);
 
   // ---- deferred step: enqueue and return; the previous one is confirmed behind it ------------------------------------
@@ -1389,7 +1317,7 @@ static int update_impl(ftkb_ctx *c, bool allow_defer) {
     // a test kernel with a GPU's worth of work (feature-dense fields: 1e5 .. 1e6 surviving cubes) gains nothing next to the
     // following scan -- the two take turns on the SMs, measured 0.90 .. 1.64 ms per step against 0.95 in a row -- so only
     // the small, latency-bound ones go to the second stream
-    const bool overlap = c->overlap_test && c->wl_hint < 100000;
+    const bool overlap = c->wl_hint < 100000;
     if (!overlap && c->last_test_overlapped && !c->pend.empty())
       CK(cudaStreamWaitEvent(c->stream, c->dev[c->pend.back().evset][2], 0));     // test kernels share one ticket counter: never two at once
     c->last_test_overlapped = overlap;

@@ -266,9 +266,11 @@ __global__ void __launch_bounds__(32 * SCAN3_BY) scan3d_kernel(const SweepParams
 
 // ---- 2D, scalar input: central-difference gradient (grad.hh:10-31) fused into the scan -------------
 // The vector field is never materialised.  A warp owns a strip of 64 vertex columns (two per lane,
-// one 16-byte load per lane, row and layer) and marches along y with a four-row register window
+// two 8-byte loads per lane, row and layer) and marches along y with a four-row register window
 // per layer (three rows of stencil + one row of prefetch; the row loop is unrolled by four so the
-// window rotates without register moves); x neighbours come from warp shuffles.
+// window rotates without register moves); x neighbours come from warp shuffles.  It runs where the
+// rows are not 16-byte aligned (odd W, or a borrowed pointer off a 16-byte boundary); aligned rows
+// take the range-cell kernels below.
 //
 // Per row the kernel derives the fp64 gradient of both layers exactly as gradient2D does, rounds
 // each component to fp32 and keeps fp32 min/max ranges per component (merged over the two layers,
@@ -318,7 +320,7 @@ __device__ __forceinline__ void warp_res_commit(double m, unsigned long long *sl
 
 __device__ __forceinline__ double nz_abs_d(double v) { const double a = fabs(v); return (v != 0.0 && a < DBL_MAX) ? a : DBL_MAX; }
 
-template <bool HAS_NEXT, bool ALIGNED, bool BORDER>
+template <bool HAS_NEXT, bool BORDER>
 __device__ __forceinline__ void fused2d_strip(const SweepParams &p, const int b, const int cy, const int lane) {
   constexpr int NL = HAS_NEXT ? 2 : 1;
   const int W = p.W, H = p.H;
@@ -357,14 +359,8 @@ __device__ __forceinline__ void fused2d_strip(const SweepParams &p, const int b,
     }
 #pragma unroll
     for (int L = 0; L < NL; L++) {
-      if (ALIGNED) {
-        double2 t = make_double2(0.0, 0.0);
-        if (e_in) t = __ldg(reinterpret_cast<const double2 *>(q[L]));
-        dst[L][0] = t.x; dst[L][1] = t.y;
-      } else {
-        dst[L][0] = e_in ? __ldg(q[L]) : 0.0;
-        dst[L][1] = o_in ? __ldg(q[L] + 1) : 0.0;
-      }
+      dst[L][0] = e_in ? __ldg(q[L]) : 0.0;
+      dst[L][1] = o_in ? __ldg(q[L] + 1) : 0.0;
     }
   };
 
@@ -446,30 +442,25 @@ __device__ __forceinline__ void fused2d_strip(const SweepParams &p, const int b,
     if (want_res[L]) warp_res_commit(rmin[L], p.res_slot[L]);
 }
 
-template <bool HAS_NEXT, bool ALIGNED>
+template <bool HAS_NEXT>
 __global__ void __launch_bounds__(256, 2) scan2d_fused_kernel(const SweepParams p) {
   const int lane = threadIdx.x & 31;
   const i64 warp = (i64)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   const int sx = (int)(warp % p.nsx), cy = (int)(warp / p.nsx);
   if (cy >= p.nsy) return;
   const int b = sx * 60;                     // first loaded column of the strip (even)
-  if (b == 0 || b + 65 > p.W) fused2d_strip<HAS_NEXT, ALIGNED, true>(p, b, cy, lane);    // touches the array's left / right edge
-  else fused2d_strip<HAS_NEXT, ALIGNED, false>(p, b, cy, lane);
+  if (b == 0 || b + 65 > p.W) fused2d_strip<HAS_NEXT, true>(p, b, cy, lane);    // touches the array's left / right edge
+  else fused2d_strip<HAS_NEXT, false>(p, b, cy, lane);
 }
 
-// ---- 2D, scalar input, bulk-async staging ----------------------------------------------------------
-// Same algorithm as scan2d_fused_kernel, but the scalar rows are staged in shared memory by the
-// async copy engine (cp.async.bulk global -> shared, completion on an mbarrier: UBLKCP in SASS)
-// instead of through registers.  Every warp owns a private ring of FB_NST row stages (both layers),
-// so there is no block-level synchronisation at all: lane 0 issues the copy of row j + FB_NST as
-// soon as row j is dead, every lane waits on the stage's mbarrier before reading it.  This keeps
-// FB_NST-2 rows (x 2 layers x 544 B) per warp in flight independent of register pressure, which is
-// what an HBM-bound stencil needs; x neighbours are read from the staged row, so no shuffles either.
-// Requires 16-byte aligned rows (W even, aligned base); otherwise scan2d_fused_kernel runs.
-constexpr int FB_NST = 6;          // ring stages (rows) per warp; the row loop is unrolled by 6 = lcm(3-row window, 2 range buffers, ring)
-constexpr int FB_SEG = 68;         // doubles per staged row segment: columns c0-2 .. c0+65
+// ---- staging helpers of the range-cell scans ----------------------------------------------------------------------
+// The scalar build kernels below stage rows (2D) or planes (3D) in a shared-memory ring with the async copy engine
+// (cp.async.bulk / cp.async.bulk.tensor, completion on a stage's `full` mbarrier).  Consumer warps wait on `full` and
+// never synchronise with each other; a stage is refilled once every consumer warp has released it (2D: a producer
+// warp waits on the stage's `empty` mbarrier; 3D: the last warp to release it issues the copy).  A 2D strip owns
+// FB_STRIDE corner columns and reads FB_SEG columns of a row.
+constexpr int FB_SEG = 68;         // doubles per row segment of a strip: columns c0-2 .. c0+65
 constexpr int FB_STRIDE = 62;      // corner columns owned per strip (c0 .. c0+61)
-constexpr int FB_WARPS = 8;
 
 __device__ __forceinline__ uint32_t smem_u32(const void *q) { return (uint32_t)__cvta_generic_to_shared(q); }
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
@@ -482,22 +473,20 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void *src, uint32_t
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
-// the same copy with an L2 eviction policy (createpolicy): a layer is streamed once, so its lines may leave L2 first
-__device__ __forceinline__ unsigned long long l2_policy_evict_first() {
-  unsigned long long pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void bulk_g2s_hint(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar, unsigned long long pol) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-               ::"r"(dst), "l"(src), "r"(bytes), "r"(bar), "l"(pol) : "memory");
-}
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   uint32_t done;
   do {
     asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
                  : "=r"(done) : "r"(bar), "r"(parity) : "memory");
   } while (!done);
+}
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+
+__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *tm, int c0, int c1, int c2, uint32_t bar) {
+  asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
+               ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(bar) : "memory");
 }
 
 template <int K> struct IC { static constexpr int value = K; };
@@ -523,416 +512,18 @@ __device__ __forceinline__ void res_update4(double &m, float &mf, bool e_in, boo
   mf = fabs(m) < 1e38 ? __double2float_ru(fabs(m)) * 1.000001f : 3.4028234e38f;
 }
 
-// cold path of the bulk scan: per-corner tests of one lane's two cubes + worklist append.
-// top: the row above belongs to no cube of this corner row (domain's last row): ranges of the lower row only
-struct SlowArgs {          // what the cold path needs of SweepParams (passed by value: no stack copy of the whole block)
-  float thrp, thr2, limf;
-  int lb0, lb1, nc0;
-  unsigned long long *wl_count, *wl;
-  unsigned long long wl_cap;
-};
-
-__device__ __noinline__ void bulk_slow_tests(const SlowArgs a, bool top, bool e_act, bool o_act, int e, int y,
-                                             FRange pex, FRange pey, FRange pox, FRange poy, FRange cex, FRange cey, FRange cox, FRange coy) {
-  if (top) { cex = pex; cey = pey; cox = pox; coy = poy; }
-  const bool se = e_act && !cube_excluded2_f(fmerge(pex, cex), fmerge(pey, cey), a.thrp, a.thr2, a.limf);
-  const bool so = o_act && !cube_excluded2_f(fmerge(pox, cox), fmerge(poy, coy), a.thrp, a.thr2, a.limf);
-  if (!__any_sync(0xffffffffu, se || so)) return;
-  const int lane = threadIdx.x & 31;
-  const u64 lin = (u64)(e - a.lb0) + (u64)a.nc0 * (u64)(y - a.lb1);
-#pragma unroll
-  for (int q = 0; q < 2; q++) {
-    const bool surv = q ? so : se;
-    const unsigned b = __ballot_sync(0xffffffffu, surv);
-    if (b == 0) continue;
-    u64 base = 0;
-    if (lane == __ffs(b) - 1) base = atomicAdd(a.wl_count, (u64)__popc(b));
-    base = __shfl_sync(0xffffffffu, base, __ffs(b) - 1);
-    if (surv) {
-      const u64 i = base + __popc(b & ((1u << lane) - 1));
-      if (i < a.wl_cap) a.wl[i] = lin + q;
-    }
-  }
-}
-
-template <bool HAS_NEXT, bool BORDER>
-__device__ __forceinline__ void fused2d_bulk_strip(const SweepParams &p, const int c0, const int cy, const int lane,
-                                                   double *ring /* [FB_NST][NL][FB_SEG] */, const uint32_t bar0 /* FB_NST barriers */) {
-  constexpr int NL = HAS_NEXT ? 2 : 1;
-  constexpr uint32_t STAGE_BYTES = NL * FB_SEG * 8;
-  const int W = p.W, H = p.H;
-  const int e = c0 + 2 * lane, o = e + 1;
-  const bool e_in = !BORDER || e < W, o_in = !BORDER || o < W, o1_in = !BORDER || o + 1 < W;
-  const bool e_own = lane <= 30 && e >= p.lb[0] && e <= p.ub[0];
-  const bool o_own = lane <= 30 && o >= p.lb[0] && o <= p.ub[0];
-  const bool e_last = BORDER && e == p.ub[0], o_last = BORDER && o == p.ub[0];   // the vertex column right of the domain's last one is not part of any valid simplex
-  const int r0 = cy * p.rows;
-  const int r1 = min(r0 + p.rows - 1, H - 1);        // last corner row of the chunk
-  const int jl = r1 + 1;                             // last gradient row visited
-  const int nrows = jl - r0 + 3;                     // staged rows r0-1 .. jl+1 (ring index 0 .. nrows-1)
-  const int ytop = p.ub[1];
-  const float cwf = (float)(W - 1), chf = (float)(H - 1);
-  const float thrp = p.thrp_f, thr2 = p.thr2_f, limf = p.lim_f;
-  const bool want_res[2] = {p.res_slot[0] != nullptr, HAS_NEXT && p.res_slot[1] != nullptr};
-  double rmin[2] = {DBL_MAX, DBL_MAX};
-  float rminf[2] = {3.4028234e38f, 3.4028234e38f};
-
-  // producer side (one elected lane; every operand is warp-uniform): copy the clipped segment of one row
-  // of every layer into its stage.  The source pointers walk the rows r0-1, r0, ... with the array's
-  // index clamp (rows below 0 / above H-1 re-read the border row).
-  const int col_lo = max(c0 - 2, 0), col_hi = min(c0 + FB_SEG - 2, W);
-  const uint32_t seg_bytes = (uint32_t)(col_hi - col_lo) * 8u;
-  const uint32_t ring_u32 = smem_u32(ring) + (uint32_t)(col_lo - (c0 - 2)) * 8u;
-  const size_t row_bytes = (size_t)W * 8;
-  const char *src[NL];
-  int src_row = clampi(r0 - 1, H);
-#pragma unroll
-  for (int L = 0; L < NL; L++)
-    src[L] = reinterpret_cast<const char *>((L == 0 ? p.L[0].S : p.L[1].S) + (size_t)W * (size_t)src_row + (size_t)col_lo);
-  int rr_issue = 0;                                  // next ring row to issue; rows are issued strictly in order
-  auto issue = [&](const uint32_t stage_off, const uint32_t bar) {
-    const int want = clampi(r0 - 1 + rr_issue, H);
-    if (want != src_row) {
-      src_row = want;
-#pragma unroll
-      for (int L = 0; L < NL; L++) src[L] += row_bytes;
-    }
-    if (elect_one()) {
-      mbar_expect_tx(bar, seg_bytes * NL);
-#pragma unroll
-      for (int L = 0; L < NL; L++) bulk_g2s(ring_u32 + stage_off + (uint32_t)(L * FB_SEG) * 8u, src[L], seg_bytes, bar);
-    }
-    rr_issue++;
-  };
-  const double *lane_base = ring + 2 * lane;    // [1]: column e-1, [2..3]: e, o, [4]: o+1
-  auto centre = [&](const int st, double (&dst)[NL][2]) {
-#pragma unroll
-    for (int L = 0; L < NL; L++) {
-      const double2 t = *reinterpret_cast<const double2 *>(lane_base + (st * NL + L) * FB_SEG + 2);
-      dst[L][0] = t.x; dst[L][1] = t.y;
-    }
-  };
-
-#pragma unroll
-  for (int q = 0; q < FB_NST; q++)
-    if (q < nrows) issue(q * STAGE_BYTES, bar0 + 8u * q);
-  double win[3][NL][2];
-  FRange R[2][2][2];
-  mbar_wait(bar0, 0);
-  centre(0, win[0]);
-  mbar_wait(bar0 + 8, 0);
-  centre(1, win[1]);
-  __syncwarp();
-  if (rr_issue < nrows) issue(0, bar0);             // row 0 is dead: only its centre columns are ever needed
-#pragma unroll
-  for (int a = 0; a < 2; a++)
-#pragma unroll
-    for (int c = 0; c < 2; c++) R[1][a][c] = FRange{0.f, 0.f};   // never read: the first row has no previous row
-
-  // gradient row j = r0 + 6 i + K; ring index of row j is 1 + 6 i + K
-  auto step = [&](auto KC, const int j, const int i) {
-    constexpr int K = decltype(KC)::value;
-    constexpr int ST_J = (1 + K) % FB_NST, ST_P = (2 + K) % FB_NST;
-    double (&m1)[NL][2] = win[K % 3];
-    double (&c0v)[NL][2] = win[(K + 1) % 3];
-    double (&p1)[NL][2] = win[(K + 2) % 3];
-    FRange (&prev)[2][2] = R[(K + 1) & 1];
-    FRange (&cur)[2][2] = R[K & 1];
-    mbar_wait(bar0 + 8u * ST_P, (uint32_t)((i + (2 + K >= FB_NST ? 1 : 0)) & 1));
-    centre(ST_P, p1);
-    FRange ve[2], vo[2];   // per component, layers merged
-#pragma unroll
-    for (int L = 0; L < NL; L++) {
-      const double *rowj = lane_base + (ST_J * NL + L) * FB_SEG;
-      double left = rowj[1], right = rowj[4];
-      double mid_e = c0v[L][1];
-      if (BORDER) {
-        if (e == 0) left = c0v[L][0];
-        if (!o_in) mid_e = c0v[L][0];
-        if (!o1_in) right = c0v[L][1];
-      }
-      // exact fp64 differences; the scaling by (W-1), (H-1) is done in fp32 here (only the conservative
-      // ranges use it) and in fp64, as the reference does, wherever a value is needed exactly
-      const double dxe = mid_e - left, dxo = right - c0v[L][0], dye = p1[L][0] - m1[L][0], dyo = p1[L][1] - m1[L][1];
-      const float fxe = __double2float_rn(dxe) * cwf, fxo = __double2float_rn(dxo) * cwf;
-      const float fye = __double2float_rn(dye) * chf, fyo = __double2float_rn(dyo) * chf;
-      if (want_res[L] && j < H) {
-        // candidates for a new minimum of the non-zero |v|: decided in fp32 against a filter that sits
-        // above the fp64 minimum; exact zeros (and fp32 underflow) also take the exact path
-        float a = fminf(fminf(fabsf(fxe), fabsf(fye)), fminf(fabsf(fxo), fabsf(fyo)));
-        if (BORDER) a = fminf(e_in ? fminf(fabsf(fxe), fabsf(fye)) : 3.4028234e38f, o_in ? fminf(fabsf(fxo), fabsf(fyo)) : 3.4028234e38f);
-        if (a < rminf[L]) res_update4(rmin[L], rminf[L], e_in, o_in, dxe, dye, dxo, dyo, (double)(W - 1), (double)(H - 1));
-      }
-      if (L == 0) {
-        ve[0] = FRange{fxe, fxe}; ve[1] = FRange{fye, fye}; vo[0] = FRange{fxo, fxo}; vo[1] = FRange{fyo, fyo};
-      } else {
-        ve[0] = fmerge(ve[0], FRange{fxe, fxe}); ve[1] = fmerge(ve[1], FRange{fye, fye});
-        vo[0] = fmerge(vo[0], FRange{fxo, fxo}); vo[1] = fmerge(vo[1], FRange{fyo, fyo});
-      }
-    }
-    // x merge: corner column c covers vertex columns c and c+1 (only c when c is the domain's last column)
-#pragma unroll
-    for (int c = 0; c < 2; c++) {
-      const FRange nx = fshfl_down1(ve[c]);
-      cur[0][c] = e_last ? ve[c] : fmerge(ve[c], vo[c]);
-      cur[1][c] = o_last ? vo[c] : fmerge(vo[c], nx);
-    }
-    if (j > r0) {
-      const int y = j - 1;
-      const bool yrow = y >= p.lb[1] && y <= ytop;
-      bool slow = BORDER || y == ytop;      // masked columns / the domain's last row: per-corner path
-      if (!BORDER && y != ytop) {
-        // both cubes of the lane at once: if their union passes, each of them does
-        const FRange ux = fmerge(fmerge(prev[0][0], prev[1][0]), fmerge(cur[0][0], cur[1][0]));
-        const FRange uy = fmerge(fmerge(prev[0][1], prev[1][1]), fmerge(cur[0][1], cur[1][1]));
-        const bool ok = cube_excluded2_f(ux, uy, thrp, thr2, limf) || !(yrow && (e_own || o_own));
-        slow = __any_sync(0xffffffffu, !ok);
-      }
-      if (slow && yrow)
-        bulk_slow_tests(SlowArgs{thrp, thr2, limf, p.lb[0], p.lb[1], p.nc[0], p.wl_count, p.wl, p.wl_cap}, y == ytop, e_own, o_own, e, y,
-                        prev[0][0], prev[0][1], prev[1][0], prev[1][1], cur[0][0], cur[0][1], cur[1][0], cur[1][1]);
-    }
-    // row j is dead now (its centre went into the window one step ago, its x neighbours were read above):
-    // refill its stage with the next row in line (ring row 1 + 6 i + K + FB_NST)
-    __syncwarp();
-    if (rr_issue < nrows) issue(ST_J * STAGE_BYTES, bar0 + 8u * ST_J);
-  };
-
-  for (int j = r0, i = 0; j <= jl; j += FB_NST, i++) {
-    step(IC<0>{}, j, i);
-    if (j + 1 <= jl) step(IC<1>{}, j + 1, i);
-    if (j + 2 <= jl) step(IC<2>{}, j + 2, i);
-    if (j + 3 <= jl) step(IC<3>{}, j + 3, i);
-    if (j + 4 <= jl) step(IC<4>{}, j + 4, i);
-    if (j + 5 <= jl) step(IC<5>{}, j + 5, i);
-  }
-#pragma unroll
-  for (int L = 0; L < NL; L++)
-    if (want_res[L]) warp_res_commit(fabs(rmin[L]), p.res_slot[L]);
-}
-
-template <bool HAS_NEXT>
-__global__ void __launch_bounds__(FB_WARPS * 32, 3) scan2d_bulk_kernel(const SweepParams p) {
-  constexpr int NL = HAS_NEXT ? 2 : 1;
-  extern __shared__ __align__(128) unsigned char fb_smem[];
-  const int lane = threadIdx.x & 31;
-  const int wib = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);     // warp-uniform by construction
-  double *ring = reinterpret_cast<double *>(fb_smem) + (size_t)wib * (FB_NST * NL * FB_SEG);
-  unsigned long long *bars = reinterpret_cast<unsigned long long *>(fb_smem + (size_t)FB_WARPS * FB_NST * NL * FB_SEG * 8) + wib * FB_NST;
-  const uint32_t bar0 = smem_u32(bars);
-  if (lane == 0) {
-#pragma unroll
-    for (int q = 0; q < FB_NST; q++) mbar_init(bar0 + 8u * q, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  }
-  __syncwarp();
-  const i64 warp = (i64)blockIdx.x * FB_WARPS + wib;
-  const int sx = (int)(warp % p.nsx), cy = (int)(warp / p.nsx);
-  if (cy >= p.nsy) return;
-  const int c0 = sx * FB_STRIDE;
-  // strips that touch the array's left / right edge or hold the domain's last column take the masked path
-  const bool border = c0 == 0 || c0 + FB_SEG - 2 > p.W || (p.ub[0] >= c0 - 1 && p.ub[0] <= c0 + 63);
-  if (border) fused2d_bulk_strip<HAS_NEXT, true>(p, c0, cy, lane, ring, bar0);
-  else fused2d_bulk_strip<HAS_NEXT, false>(p, c0, cy, lane, ring, bar0);
-}
-
-// ---- 2D, scalar input, CTA-wide staging with a producer warp -----------------------------------------
-// The per-warp rings above issue two 544-byte copies per warp and row, and ncu shows the copy engine's
-// request queue (stall_mio on UBLKCP, long scoreboard behind it) as the limiter.  Here a CTA of seven
-// consumer warps + one producer warp shares ONE ring of row stages that spans all seven strips
-// (7 x 62 corner columns + halo = 442 doubles = 3.5 KB per row and layer): 7x fewer, 7x larger bulk
-// copies, no column overlap between the strips of a CTA, and no copy-issue instructions at all in the
-// consumer warps.  Classic full/empty mbarrier pipeline: the producer's elected lane waits for a
-// stage's `empty` barrier (one arrival per consumer warp), arms `full` with the byte count and issues
-// the copies; consumers wait on `full`, read, and arrive on `empty` when a row is dead for them.
-constexpr int TL_CW = 7;                               // consumer warps per CTA
-constexpr int TL_SEG = TL_CW * FB_STRIDE + 8;          // staged doubles per row: columns C0-2 .. C0+439
-constexpr int TL_NST = FB_NST;
-
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-
-template <bool HAS_NEXT, bool BORDER>
-__device__ __forceinline__ void fused2d_tile_strip(const SweepParams &p, const int c0, const int r0, const int r1, const int lane,
-                                                   const double *tile /* this warp's column 0 = c0-2 */, const uint32_t full0, const uint32_t empty0) {
-  constexpr int NL = HAS_NEXT ? 2 : 1;
-  const int W = p.W, H = p.H;
-  const int e = c0 + 2 * lane, o = e + 1;
-  const bool e_in = !BORDER || e < W, o_in = !BORDER || o < W, o1_in = !BORDER || o + 1 < W;
-  const bool e_own = lane <= 30 && e >= p.lb[0] && e <= p.ub[0];
-  const bool o_own = lane <= 30 && o >= p.lb[0] && o <= p.ub[0];
-  const bool e_last = BORDER && e == p.ub[0], o_last = BORDER && o == p.ub[0];
-  const int jl = r1 + 1;                             // last gradient row visited
-  const int ytop = p.ub[1];
-  const float cwf = (float)(W - 1), chf = (float)(H - 1);
-  const float thrp = p.thrp_f, thr2 = p.thr2_f, limf = p.lim_f;
-  const bool want_res[2] = {p.res_slot[0] != nullptr, HAS_NEXT && p.res_slot[1] != nullptr};
-  double rmin[2] = {DBL_MAX, DBL_MAX};
-  float rminf[2] = {3.4028234e38f, 3.4028234e38f};
-
-  const double *lane_base = tile + 2 * lane;    // [1]: column e-1, [2..3]: e, o, [4]: o+1
-  auto centre = [&](const int st, double (&dst)[NL][2]) {
-#pragma unroll
-    for (int L = 0; L < NL; L++) {
-      const double2 t = *reinterpret_cast<const double2 *>(lane_base + (st * NL + L) * TL_SEG + 2);
-      dst[L][0] = t.x; dst[L][1] = t.y;
-    }
-  };
-  auto release = [&](const int st) {     // this warp is done with the stage
-    __syncwarp();
-    if (elect_one()) mbar_arrive(empty0 + 8u * st);
-  };
-
-  double win[3][NL][2];
-  FRange R[2][2][2];
-  mbar_wait(full0, 0);
-  centre(0, win[0]);
-  mbar_wait(full0 + 8, 0);
-  centre(1, win[1]);
-  release(0);                                      // row r0-1: only its centre columns are ever needed
-#pragma unroll
-  for (int a = 0; a < 2; a++)
-#pragma unroll
-    for (int c = 0; c < 2; c++) R[1][a][c] = FRange{0.f, 0.f};   // never read: the first row has no previous row
-
-  // gradient row j = r0 + 6 i + K; ring index of row j is 1 + 6 i + K
-  auto step = [&](auto KC, const int j, const int i) {
-    constexpr int K = decltype(KC)::value;
-    constexpr int ST_J = (1 + K) % TL_NST, ST_P = (2 + K) % TL_NST;
-    double (&m1)[NL][2] = win[K % 3];
-    double (&c0v)[NL][2] = win[(K + 1) % 3];
-    double (&p1)[NL][2] = win[(K + 2) % 3];
-    FRange (&prev)[2][2] = R[(K + 1) & 1];
-    FRange (&cur)[2][2] = R[K & 1];
-    mbar_wait(full0 + 8u * ST_P, (uint32_t)((i + (2 + K >= TL_NST ? 1 : 0)) & 1));
-    centre(ST_P, p1);
-    FRange ve[2], vo[2];   // per component, layers merged
-#pragma unroll
-    for (int L = 0; L < NL; L++) {
-      const double *rowj = lane_base + (ST_J * NL + L) * TL_SEG;
-      double left = rowj[1], right = rowj[4];
-      double mid_e = c0v[L][1];
-      if (BORDER) {
-        if (e == 0) left = c0v[L][0];
-        if (!o_in) mid_e = c0v[L][0];
-        if (!o1_in) right = c0v[L][1];
-      }
-      const double dxe = mid_e - left, dxo = right - c0v[L][0], dye = p1[L][0] - m1[L][0], dyo = p1[L][1] - m1[L][1];
-      const float fxe = __double2float_rn(dxe) * cwf, fxo = __double2float_rn(dxo) * cwf;
-      const float fye = __double2float_rn(dye) * chf, fyo = __double2float_rn(dyo) * chf;
-      if (want_res[L] && j < H) {
-        float a = fminf(fminf(fabsf(fxe), fabsf(fye)), fminf(fabsf(fxo), fabsf(fyo)));
-        if (BORDER) a = fminf(e_in ? fminf(fabsf(fxe), fabsf(fye)) : 3.4028234e38f, o_in ? fminf(fabsf(fxo), fabsf(fyo)) : 3.4028234e38f);
-        if (a < rminf[L]) res_update4(rmin[L], rminf[L], e_in, o_in, dxe, dye, dxo, dyo, (double)(W - 1), (double)(H - 1));
-      }
-      if (L == 0) {
-        ve[0] = FRange{fxe, fxe}; ve[1] = FRange{fye, fye}; vo[0] = FRange{fxo, fxo}; vo[1] = FRange{fyo, fyo};
-      } else {
-        ve[0] = fmerge(ve[0], FRange{fxe, fxe}); ve[1] = fmerge(ve[1], FRange{fye, fye});
-        vo[0] = fmerge(vo[0], FRange{fxo, fxo}); vo[1] = fmerge(vo[1], FRange{fyo, fyo});
-      }
-    }
-#pragma unroll
-    for (int c = 0; c < 2; c++) {
-      const FRange nx = fshfl_down1(ve[c]);
-      cur[0][c] = e_last ? ve[c] : fmerge(ve[c], vo[c]);
-      cur[1][c] = o_last ? vo[c] : fmerge(vo[c], nx);
-    }
-    if (j > r0) {
-      const int y = j - 1;
-      const bool yrow = y >= p.lb[1] && y <= ytop;
-      bool slow = BORDER || y == ytop;      // masked columns / the domain's last row: per-corner path
-      if (!BORDER && y != ytop) {
-        const FRange ux = fmerge(fmerge(prev[0][0], prev[1][0]), fmerge(cur[0][0], cur[1][0]));
-        const FRange uy = fmerge(fmerge(prev[0][1], prev[1][1]), fmerge(cur[0][1], cur[1][1]));
-        const bool ok = cube_excluded2_f(ux, uy, thrp, thr2, limf) || !(yrow && (e_own || o_own));
-        slow = __any_sync(0xffffffffu, !ok);
-      }
-      if (slow && yrow)
-        bulk_slow_tests(SlowArgs{thrp, thr2, limf, p.lb[0], p.lb[1], p.nc[0], p.wl_count, p.wl, p.wl_cap}, y == ytop, e_own, o_own, e, y,
-                        prev[0][0], prev[0][1], prev[1][0], prev[1][1], cur[0][0], cur[0][1], cur[1][0], cur[1][1]);
-    }
-    release(ST_J);     // row j: its centre went into the window one step ago, its x neighbours were read above
-  };
-
-  for (int j = r0, i = 0; j <= jl; j += TL_NST, i++) {
-    step(IC<0>{}, j, i);
-    if (j + 1 <= jl) step(IC<1>{}, j + 1, i);
-    if (j + 2 <= jl) step(IC<2>{}, j + 2, i);
-    if (j + 3 <= jl) step(IC<3>{}, j + 3, i);
-    if (j + 4 <= jl) step(IC<4>{}, j + 4, i);
-    if (j + 5 <= jl) step(IC<5>{}, j + 5, i);
-  }
-#pragma unroll
-  for (int L = 0; L < NL; L++)
-    if (want_res[L]) warp_res_commit(fabs(rmin[L]), p.res_slot[L]);
-}
-
-template <bool HAS_NEXT>
-__global__ void __launch_bounds__((TL_CW + 1) * 32, 3) scan2d_tile_kernel(const SweepParams p) {
-  constexpr int NL = HAS_NEXT ? 2 : 1;
-  constexpr uint32_t STAGE_BYTES = NL * TL_SEG * 8;
-  extern __shared__ __align__(128) unsigned char fb_smem[];
-  const int lane = threadIdx.x & 31;
-  const int wib = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);     // warp-uniform by construction
-  double *ring = reinterpret_cast<double *>(fb_smem);
-  const uint32_t full0 = smem_u32(fb_smem + (size_t)TL_NST * STAGE_BYTES), empty0 = full0 + 8u * TL_NST;
-  const int W = p.W, H = p.H;
-  const int bx = blockIdx.x % p.nsx, cy = blockIdx.x / p.nsx;
-  const int C0 = bx * (TL_CW * FB_STRIDE);
-  // consumer warps whose strip starts inside the array
-  const int nactive = min(TL_CW, (W - C0 + FB_STRIDE - 1) / FB_STRIDE);
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int q = 0; q < TL_NST; q++) { mbar_init(full0 + 8u * q, 1); mbar_init(empty0 + 8u * q, (uint32_t)nactive); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  }
-  __syncthreads();
-  const int r0 = cy * p.rows;
-  const int r1 = min(r0 + p.rows - 1, H - 1);
-  const int nrows = (r1 + 1) - r0 + 3;               // staged rows r0-1 .. r1+2 (ring index 0 .. nrows-1)
-  if (wib == TL_CW) {
-    // producer: one elected lane walks the rows with the array's index clamp (rows below 0 / above H-1
-    // re-read the border row) and keeps the ring full
-    if (elect_one()) {
-      const int col_lo = max(C0 - 2, 0), col_hi = min(C0 - 2 + TL_SEG, W);
-      const uint32_t seg_bytes = (uint32_t)(col_hi - col_lo) * 8u;
-      const uint32_t dst0 = smem_u32(ring) + (uint32_t)(col_lo - (C0 - 2)) * 8u;
-      for (int rr = 0; rr < nrows; rr++) {
-        const int st = rr % TL_NST;
-        if (rr >= TL_NST) mbar_wait(empty0 + 8u * st, (uint32_t)((rr / TL_NST - 1) & 1));
-        const size_t off = (size_t)W * (size_t)clampi(r0 - 1 + rr, H) + (size_t)col_lo;
-        mbar_expect_tx(full0 + 8u * st, seg_bytes * NL);
-#pragma unroll
-        for (int L = 0; L < NL; L++)
-          bulk_g2s(dst0 + (uint32_t)st * STAGE_BYTES + (uint32_t)(L * TL_SEG) * 8u, (L == 0 ? p.L[0].S : p.L[1].S) + off, seg_bytes, full0 + 8u * st);
-      }
-    }
-    return;
-  }
-  if (wib >= nactive) return;
-  const int c0 = C0 + wib * FB_STRIDE;
-  const double *tile = ring + wib * FB_STRIDE;
-  // strips that touch the array's left / right edge or hold the domain's last column take the masked path
-  const bool border = c0 == 0 || c0 + FB_SEG - 2 > W || (p.ub[0] >= c0 - 1 && p.ub[0] <= c0 + 63);
-  if (border) fused2d_tile_strip<HAS_NEXT, true>(p, c0, r0, r1, lane, tile, full0, empty0);
-  else fused2d_tile_strip<HAS_NEXT, false>(p, c0, r0, r1, lane, tile, full0, empty0);
-}
-
 // ---- 2D, scalar input, per-layer range cells ("build once, test from cells") ---------------------------------
-// Same idea as the 3D cells below: the fp32 ranges the tile scan keeps per thread depend on one layer only, so
+// Same idea as the 3D cells below: the fp32 ranges of the register scan above depend on one layer only, so
 // a layer is streamed once -- by the step that first sees it -- and leaves a 16-byte cell {min vx, max vx, min vy,
 // max vy} per (lane, block of C2_R corner rows); the step reads the CURRENT layer's cells instead of the layer.
 // A cell spans the lane's two columns, the next lane's two, and gradient rows 9k .. 9k+9: a superset of the
 // vertices of the lane's 2 x 9 cubes.  If the union of the two layers' cells passes cube_excluded2_f, all 18 cubes
 // are excluded; otherwise they are tested one by one from global memory (cold) and survivors are appended.
-// Traffic per step: 8 B/vertex of scalars + ~1 B/vertex of cells written + ~1 B/vertex read (16 B/vertex before).
+// Traffic per step: 8 B/vertex of scalars + ~1 B/vertex of cells written + ~1 B/vertex read (16 B/vertex for a scan that re-reads both layers).
 constexpr int C2_R = 9;                                // corner rows per cell block (a multiple of 3: the row window rotates by index)
 constexpr int C2_NST = 9;                              // ring stages (rows) = unroll of the row loop = C2_R
-constexpr int C2_CW = TL_CW;
+constexpr int C2_CW = 7;                               // consumer warps per CTA (plus one producer warp)
+constexpr int C2_SEG = C2_CW * FB_STRIDE + 8;          // staged doubles per row: columns C0-2 .. C0+439
 static_assert(C2_R % 3 == 0 && C2_R == C2_NST && C2_R == SCAN2D_CELL_ROWS, "row window / ring / cell block must stay aligned");
 
 __device__ __forceinline__ size_t cells2d_index(const SweepParams &p, const int strip, const int kb, const int lane) {
@@ -944,14 +535,14 @@ __device__ __forceinline__ size_t cells2d_index(const SweepParams &p, const int 
 // one lane per cube: ranges over the vertices valid simplices can use (<= ub) from global memory, gradient exactly
 // as gradient2D indexes it (clamped at the array border); survivors are appended.
 template <int NL>
-__device__ __forceinline__ void cells2d_slow_cubes_t(const SweepParams &p, unsigned failmask, const int c0, const int y0, const int nrows, const uint32_t stage) {
+__device__ __forceinline__ void cells2d_slow_cubes_t(const SweepParams &p, unsigned failmask, const int c0, const int y0, const uint32_t stage) {
   static_assert(2 * C2_R <= 32, "one lane per cube");
   const int W = p.W, H = p.H;
   const int lane = threadIdx.x & 31;
   const float cwf = (float)(W - 1), chf = (float)(H - 1);
   const float nanf_ = __int_as_float(0x7FC00000);
-  // the 2 x nrows cubes of every failing lane, packed 32 to a pass (a failing lane alone would keep 18 of 32 lanes busy)
-  const int per = 2 * nrows, total = per * __popc(failmask);
+  // the 2 x C2_R cubes of every failing lane, packed 32 to a pass (a failing lane alone would keep 18 of 32 lanes busy)
+  const int per = 2 * C2_R, total = per * __popc(failmask);
   for (int q0 = 0; q0 < total; q0 += 32) {
     const int qi = q0 + lane;
     const bool live = qi < total;
@@ -999,16 +590,16 @@ __device__ __forceinline__ void cells2d_slow_cubes_t(const SweepParams &p, unsig
 // one lane per cube: ranges over the vertices valid simplices can use (<= ub) from global memory, gradient exactly
 // as gradient2D indexes it (clamped at the array border); survivors are appended.
 // stage: shared-memory staging of this warp's survivors (flushed by the caller at the end), or 0: append directly
-__device__ __noinline__ void cells2d_slow_cubes(const SweepParams &p, unsigned failmask, const int c0, const int y0, const int nl, const int nrows, const uint32_t stage = 0) {
-  if (nl == 1) cells2d_slow_cubes_t<1>(p, failmask, c0, y0, nrows, stage);
-  else cells2d_slow_cubes_t<2>(p, failmask, c0, y0, nrows, stage);
+__device__ __noinline__ void cells2d_slow_cubes(const SweepParams &p, unsigned failmask, const int c0, const int y0, const int nl, const uint32_t stage = 0) {
+  if (nl == 1) cells2d_slow_cubes_t<1>(p, failmask, c0, y0, stage);
+  else cells2d_slow_cubes_t<2>(p, failmask, c0, y0, stage);
 }
 
 // union of the cells of all layers for one block -> excluded, or the cold path
 __device__ __forceinline__ void cells2d_decide(const SweepParams &p, const FRange ux, const FRange uy, const bool own, const int e, const int y0, const int nl) {
   const bool fail = own && !cube_excluded2_f(ux, uy, p.thrp_f, p.thr2_f, p.lim_f);
   const unsigned fm = __ballot_sync(0xffffffffu, fail);
-  if (fm) cells2d_slow_cubes(p, fm, e - 2 * (int)(threadIdx.x & 31), y0, nl, C2_R);
+  if (fm) cells2d_slow_cubes(p, fm, e - 2 * (int)(threadIdx.x & 31), y0, nl);
 }
 
 template <bool BORDER, int NPREV, bool TEST>
@@ -1029,7 +620,7 @@ __device__ __forceinline__ void cells2d_strip(const SweepParams &p, const int c0
 
   const double *lane_base = tile + 2 * lane;    // [1]: column e-1, [2..3]: e, o, [4]: o+1
   auto centre = [&](const int st, double (&dst)[2]) {
-    const double2 t = *reinterpret_cast<const double2 *>(lane_base + st * TL_SEG + 2);
+    const double2 t = *reinterpret_cast<const double2 *>(lane_base + st * C2_SEG + 2);
     dst[0] = t.x; dst[1] = t.y;
   };
   auto release = [&](const int st) {     // this warp is done with the stage
@@ -1070,7 +661,7 @@ __device__ __forceinline__ void cells2d_strip(const SweepParams &p, const int c0
     double (&p1)[2] = win[(K + 2) % 3];
     mbar_wait(full0 + 8u * ST_P, (uint32_t)((i + (2 + K >= C2_NST ? 1 : 0)) & 1));
     centre(ST_P, p1);
-    const double *rowj = lane_base + ST_J * TL_SEG;
+    const double *rowj = lane_base + ST_J * C2_SEG;
     double left = rowj[1], right = rowj[4];
     double mid_e = c0v[1];
     if (BORDER) {
@@ -1115,7 +706,7 @@ __device__ __forceinline__ void cells2d_strip(const SweepParams &p, const int c0
 
 template <int NPREV, bool TEST>
 __global__ void __launch_bounds__((C2_CW + 1) * 32, 3) scan2d_build_kernel(const __grid_constant__ SweepParams p) {
-  constexpr uint32_t STAGE_BYTES = TL_SEG * 8;
+  constexpr uint32_t STAGE_BYTES = C2_SEG * 8;
   extern __shared__ __align__(128) unsigned char fb_smem[];
   const int lane = threadIdx.x & 31;
   const int wib = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);     // warp-uniform by construction
@@ -1139,7 +730,7 @@ __global__ void __launch_bounds__((C2_CW + 1) * 32, 3) scan2d_build_kernel(const
     // producer: one elected lane walks the rows with the array's index clamp and keeps the ring full
     if (elect_one()) {
       const double *S = p.L[p.build_layer].S;
-      const int col_lo = max(C0 - 2, 0), col_hi = min(C0 - 2 + TL_SEG, W);
+      const int col_lo = max(C0 - 2, 0), col_hi = min(C0 - 2 + C2_SEG, W);
       const uint32_t seg_bytes = (uint32_t)(col_hi - col_lo) * 8u;
       const uint32_t dst0 = smem_u32(ring) + (uint32_t)(col_lo - (C0 - 2)) * 8u;
       for (int rr = 0; rr < nrows; rr++) {
@@ -1194,9 +785,9 @@ __global__ void __launch_bounds__(256) scan2d_cells_kernel(const __grid_constant
 // Scalars >= 2^1000 / Inf / NaN cannot be ordered by the keys: they raise p.poison and the context redoes the step with
 // scan2d_build_kernel (fp32 ranges, handles them).
 constexpr int K2_R = 3;                                // rows per stage
-// CTAs per SM and ring stages are launch variants (FTKB_K2_CTAS / FTKB_K2_NST, see k2_variant): 8 stages (85 KB per CTA) at two
-// CTAs per SM, 4 - 6 stages (42 - 64 KB) at three, 4 at four
-constexpr uint32_t K2_ROW_BYTES = TL_SEG * 8;
+constexpr int K2_NST = 4;                              // ring stages (42 KB per CTA)
+constexpr int K2_CTAS = 3;                             // CTAs per SM
+constexpr uint32_t K2_ROW_BYTES = C2_SEG * 8;
 constexpr uint32_t K2_STAGE_BYTES = K2_R * K2_ROW_BYTES;
 static_assert(C2_R % K2_R == 0, "cell block = whole stages");
 
@@ -1254,7 +845,7 @@ struct K2Acc { double mdx, mdy; float big; };     // per-lane accumulators carri
 
 // one segment of one strip; a function of its own (not inlined) so that the hot loop gets the whole register file and the
 // persistent loop's bookkeeping is saved once per segment, not kept live across it
-template <bool BORDER, int NPREV, bool TEST, int K2_NST>
+template <bool BORDER, int NPREV, bool TEST>
 __device__ __forceinline__ K2Acc keys2d_strip(const SweepParams &p, const int c0, const int r0, const int r1, const int lane,
                                            const uint32_t tile_u32 /* smem address of this warp's column c0-2, stage 0, row 0 */,
                                            const uint32_t full0, const uint32_t empty0, const int strip,
@@ -1434,7 +1025,7 @@ __device__ __forceinline__ K2Acc keys2d_strip(const SweepParams &p, const int c0
     for (int b = 0; b < 64; b++) {
       if (!__any_sync(0xffffffffu, (failbits >> b) != 0)) break;
       const unsigned fm = __ballot_sync(0xffffffffu, (failbits >> b) & 1ull);
-      if (fm) cells2d_slow_cubes(p, fm, c0, (kb0 + b) * C2_R, NPREV + 1, C2_R, wl_stage);
+      if (fm) cells2d_slow_cubes(p, fm, c0, (kb0 + b) * C2_R, NPREV + 1, wl_stage);
     }
     flush_survivors(p, wl_stage);
   }
@@ -1442,7 +1033,7 @@ __device__ __forceinline__ K2Acc keys2d_strip(const SweepParams &p, const int c0
 }
 
 // One CTA per (tile of C2_CW strips, chunk of p.rows corner rows); K2_CTAS CTAs per SM.
-template <int NPREV, bool TEST, int K2_CTAS, int K2_NST>
+template <int NPREV, bool TEST>
 __global__ void __launch_bounds__((C2_CW + 1) * 32, K2_CTAS) scan2d_keys_build_kernel(const __grid_constant__ SweepParams p) {
   extern __shared__ __align__(128) unsigned char fb_smem[];
   const int lane = threadIdx.x & 31;
@@ -1471,11 +1062,9 @@ __global__ void __launch_bounds__((C2_CW + 1) * 32, K2_CTAS) scan2d_keys_build_k
     // K2_R rows (rows past the chunk's last one repeat the clamp: valid data, never used)
     if (elect_one()) {
       const double *S = p.L[p.build_layer].S;
-      const int col_lo = max(C0 - 2, 0), col_hi = min(C0 - 2 + TL_SEG, W);
+      const int col_lo = max(C0 - 2, 0), col_hi = min(C0 - 2 + C2_SEG, W);
       const uint32_t seg_bytes = (uint32_t)(col_hi - col_lo) * 8u;
       const uint32_t dst0 = ring0 + (uint32_t)(col_lo - (C0 - 2)) * 8u;
-      const bool hint = (p.l2_hint & 1) != 0;
-      const unsigned long long pol = hint ? l2_policy_evict_first() : 0ull;
       for (int s = 0; s < nstages; s++) {
         const uint32_t slot = (uint32_t)s % K2_NST;
         if (s >= K2_NST) mbar_wait(empty0 + 8u * slot, (uint32_t)((s / K2_NST - 1) & 1));
@@ -1483,8 +1072,7 @@ __global__ void __launch_bounds__((C2_CW + 1) * 32, K2_CTAS) scan2d_keys_build_k
 #pragma unroll
         for (int i = 0; i < K2_R; i++) {
           const size_t off = (size_t)W * (size_t)clampi(r0 - 1 + K2_R * s + i, H) + (size_t)col_lo;
-          if (hint) bulk_g2s_hint(dst0 + slot * K2_STAGE_BYTES + (uint32_t)i * K2_ROW_BYTES, S + off, seg_bytes, full0 + 8u * slot, pol);
-          else bulk_g2s(dst0 + slot * K2_STAGE_BYTES + (uint32_t)i * K2_ROW_BYTES, S + off, seg_bytes, full0 + 8u * slot);
+          bulk_g2s(dst0 + slot * K2_STAGE_BYTES + (uint32_t)i * K2_ROW_BYTES, S + off, seg_bytes, full0 + 8u * slot);
         }
       }
     }
@@ -1499,8 +1087,8 @@ __global__ void __launch_bounds__((C2_CW + 1) * 32, K2_CTAS) scan2d_keys_build_k
   sts64_f64(res_u32, DBL_MAX); sts64_f64(res_u32 + 8u, DBL_MAX);
   if (lane == 0) asm volatile("st.shared.s32 [%0], %1;" ::"r"(wl_stage), "r"(0) : "memory");
   __syncwarp();
-  if (border) acc = keys2d_strip<true, NPREV, TEST, K2_NST>(p, c0, r0, r1, lane, tile_u32, full0, empty0, bx * C2_CW + wib, 0u, res_u32, wl_stage, cell_stage, acc);
-  else acc = keys2d_strip<false, NPREV, TEST, K2_NST>(p, c0, r0, r1, lane, tile_u32, full0, empty0, bx * C2_CW + wib, 0u, res_u32, wl_stage, cell_stage, acc);
+  if (border) acc = keys2d_strip<true, NPREV, TEST>(p, c0, r0, r1, lane, tile_u32, full0, empty0, bx * C2_CW + wib, 0u, res_u32, wl_stage, cell_stage, acc);
+  else acc = keys2d_strip<false, NPREV, TEST>(p, c0, r0, r1, lane, tile_u32, full0, empty0, bx * C2_CW + wib, 0u, res_u32, wl_stage, cell_stage, acc);
   if (p.res_slot[p.build_layer] != nullptr) {
     const double cw = (double)(W - 1), ch = (double)(H - 1);
     const double ax = fabs(acc.mdx), ay = fabs(acc.mdy);
@@ -1510,56 +1098,22 @@ __global__ void __launch_bounds__((C2_CW + 1) * 32, K2_CTAS) scan2d_keys_build_k
   if (!(acc.big < __int_as_float(KEYF_BIG))) atomicExch(p.poison, 1ull);
 }
 
-static size_t k2_smem_bytes(int nst) { return (size_t)nst * K2_STAGE_BYTES + (size_t)2 * nst * 8 + (size_t)16 * (C2_CW + 1) * 32 + 32 + (size_t)WL_STAGE_BYTES * C2_CW + (size_t)1024 * C2_CW; }
-// FTKB_K2_CTAS (CTAs per SM: 2 | 3 | 4, default 3) and FTKB_K2_NST (ring stages at three CTAs per SM: 4 | 5 | 6, default 4)
-static int k2_variant() {
-  static const int v = [] {
-    const char *e = std::getenv("FTKB_K2_CTAS"), *n = std::getenv("FTKB_K2_NST");
-    const int ctas = e ? std::atoi(e) : 3, nst = n ? std::atoi(n) : 4;
-    if (ctas == 2) return 28;
-    if (ctas == 4) return 44;
-    return nst == 5 ? 35 : (nst == 6 ? 36 : 34);
-  }();
-  return v;
-}
-template <int CTAS, int NST>
-static void k2_launch(const SweepParams &p, unsigned grid, cudaStream_t s) {
-  const size_t sm = k2_smem_bytes(NST);
-  switch (p.sum_mode) {
-    case SUM_BUILD: scan2d_keys_build_kernel<0, false, CTAS, NST><<<grid, (C2_CW + 1) * 32, sm, s>>>(p); break;
-    case SUM_BUILD_TEST1: scan2d_keys_build_kernel<0, true, CTAS, NST><<<grid, (C2_CW + 1) * 32, sm, s>>>(p); break;
-    default: scan2d_keys_build_kernel<1, true, CTAS, NST><<<grid, (C2_CW + 1) * 32, sm, s>>>(p); break;
-  }
-}
-template <int CTAS, int NST>
-static void k2_attrs() {
-  const int sm = (int)k2_smem_bytes(NST);
-  cudaFuncSetAttribute(scan2d_keys_build_kernel<0, false, CTAS, NST>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-  cudaFuncSetAttribute(scan2d_keys_build_kernel<0, true, CTAS, NST>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-  cudaFuncSetAttribute(scan2d_keys_build_kernel<1, true, CTAS, NST>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm);
-}
+static size_t k2_smem_bytes() { return (size_t)K2_NST * K2_STAGE_BYTES + (size_t)2 * K2_NST * 8 + (size_t)16 * (C2_CW + 1) * 32 + 32 + (size_t)WL_STAGE_BYTES * C2_CW + (size_t)1024 * C2_CW; }
+static size_t c2_smem_bytes() { return (size_t)C2_NST * C2_SEG * 8 + (size_t)2 * C2_NST * 8; }
 
-static size_t c2_smem_bytes() { return (size_t)C2_NST * TL_SEG * 8 + (size_t)2 * C2_NST * 8; }
-
-size_t vscan2d_cells_per_layer(const SweepParams &p);
-void launch_scan2d_direct(const SweepParams &p, cudaStream_t s);
 size_t scan2d_cells_per_layer(const SweepParams &p) {
-  if (p.bulk == 3) return vscan2d_cells_per_layer(p);      // direct staging: strips x 8-row blocks
   return (size_t)p.nsx * C2_CW * (size_t)(p.H / C2_R + 2) * 32u;
 }
 
 void launch_scan2d_cells(const SweepParams &p, cudaStream_t s) {
-  if (p.bulk == 3) { launch_scan2d_direct(p, s); return; }
   const unsigned grid = (unsigned)((i64)p.nsx * p.nsy);
   const int nstrips = (p.W + FB_STRIDE - 1) / FB_STRIDE, nblk = (p.H + C2_R - 1) / C2_R;
   const unsigned tgrid = (unsigned)(((i64)nstrips * nblk + 7) / 8);
   if (p.keys2d && p.sum_mode <= SUM_BUILD_TEST2) {
-    switch (k2_variant()) {
-      case 28: k2_launch<2, 8>(p, grid, s); break;
-      case 44: k2_launch<4, 4>(p, grid, s); break;
-      case 35: k2_launch<3, 5>(p, grid, s); break;
-      case 36: k2_launch<3, 6>(p, grid, s); break;
-      default: k2_launch<3, 4>(p, grid, s); break;
+    switch (p.sum_mode) {
+      case SUM_BUILD: scan2d_keys_build_kernel<0, false><<<grid, (C2_CW + 1) * 32, k2_smem_bytes(), s>>>(p); break;
+      case SUM_BUILD_TEST1: scan2d_keys_build_kernel<0, true><<<grid, (C2_CW + 1) * 32, k2_smem_bytes(), s>>>(p); break;
+      default: scan2d_keys_build_kernel<1, true><<<grid, (C2_CW + 1) * 32, k2_smem_bytes(), s>>>(p); break;
     }
     return;
   }
@@ -1572,39 +1126,22 @@ void launch_scan2d_cells(const SweepParams &p, cudaStream_t s) {
   }
 }
 
-// ---- 3D, scalar input: gradient (grad.hh:130-149) fused into the scan, planes staged by TMA -----------
-// The vector field is never materialised.  A CTA owns a tile of F3_STRIDE x F3_TROWS corner columns and
-// marches along z over a chunk of planes.  One producer warp keeps a ring of F3_NST scalar planes (both
-// layers, tile + halo) in shared memory with cp.async.bulk.tensor (TMA tile mode, one 3D box per layer and
-// plane, out-of-bounds elements zero-filled, completion on a `full` mbarrier); eight consumer warps read
-// planes z-1, z, z+1, release plane z-1 through an `empty` mbarrier and never synchronise with each other.
+// ---- 3D, scalar input: gradient (grad.hh:130-149) folded into per-layer range cells, planes staged by TMA --------
+// The vector field is never materialised.  gradient3D is 1/2 (S[+1] - S[-1]) on the array interior and zero on its
+// border, so the quantised value trunc(v 2^nbits) is trunc(d 2^(nbits-1)) with d the plain difference: scaling by a
+// power of two is exact, and the HIGH WORD of the fp64 difference, reinterpreted as an fp32 bit pattern, is a monotone
+// key of d (sign-magnitude order; truncated towards zero).  The kernels therefore keep min/max of those keys with
+// FMNMX -- no conversion instruction at all -- and "every vertex >= 1 after quantisation" is the exact comparison
+// key >= key(2^(1-nbits)) because the threshold is a power of two.  NaN keys are the neutral element (FMNMX drops
+// NaN); real NaN / Inf / >= 2^1000 scalars raise p.poison instead and the host repeats the sweep with the gradient
+// materialised (scan3d_kernel).
 //
-// gradient3D is 1/2 (S[+1] - S[-1]) on the array interior and zero on its border, so the quantised value
-// trunc(v 2^nbits) is trunc(d 2^(nbits-1)) with d the plain difference: scaling by a power of two is exact,
-// and the HIGH WORD of the fp64 difference, reinterpreted as an fp32 bit pattern, is a monotone key of d
-// (sign-magnitude order; truncated towards zero).  The kernel therefore keeps min/max of those keys with
-// FMNMX -- no conversion instruction at all -- and "every vertex >= 1 after quantisation" is the exact
-// comparison key >= key(2^(1-nbits)) because the threshold is a power of two.  NaN keys are the neutral
-// element (FMNMX drops NaN); real NaN / Inf / >= 2^1000 scalars raise p.poison instead and the host
-// repeats the sweep on the unfused path.
-//
-// Exclusion is decided per THREAD first: a lane covers 2 columns x (F3_RW + 1) gradient rows per plane; the
-// union of its values, its right neighbour's and the previous plane's is a superset of the vertices of
-// the lane's 2 x F3_RW cubes, so if the union passes the exclusion test every one of them does.  Lanes whose
-// union fails (near a common zero of all three components) test their cubes one by one from global
-// memory (cold path) and append survivors to the worklist.
-//
-// By-product: min non-zero |v| (ndarray.hh:769-779) of layers whose resolution is still unknown, over the
-// whole array -- tiles cover the array, not only the tracker's domain.
+// Determinant guard, exponent form: with e_c the biased exponent of max |d_c| (at least that of 2^-nbits),
+// |quantised v_c| < 2^(e_c - 1023 + nbits) and M_c := |quantised| + 1 <= 2^(e_c - 1022 + nbits).  Every determinant of
+// the cascade is at most 48 Mx My Mz (cube_excluded3 with R <= 2 M) < 2^(6 + sum(e_c) - 3066 + 3 nbits), which stays
+// below 2^62 for sum(e_c) <= 3119 - 3 nbits.
 constexpr int F3_LAYER_BYTES = ((F3_ROWS * F3_COLS * 8 + 127) / 128) * 128;   // one staged plane of one layer
-constexpr int F3_LAYER_DOUBLES = F3_LAYER_BYTES / 8;
 constexpr uint32_t F3_BOX_BYTES = F3_ROWS * F3_COLS * 8;
-
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap *tm, int c0, int c1, int c2, uint32_t bar) {
-  asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-               ::"r"(dst), "l"(tm), "r"(c0), "r"(c1), "r"(c2), "r"(bar) : "memory");
-}
-
 
 // cold path: for every lane whose union failed (bit set in failmask), the WARP tests that lane's 2 x F3_RW cubes of
 // plane z: four lanes per cube, two vertices each (ranges over the vertices valid simplices can use, <= ub, read from
@@ -1668,219 +1205,23 @@ __device__ __forceinline__ void res_update3(double &m, const bool in, const doub
   if (vz != 0.0 && fabs(vz) < fabs(m)) m = vz;
 }
 
-// precise exclusion test of a union given as float keys (rare: the exponent bound below failed)
-__device__ __noinline__ bool fused3d_union_excluded_precise(const float mn0, const float mx0, const float mn1, const float mx1,
-                                                            const float mn2, const float mx2, const int nbits20) {
-  const KeyRange x{vertex_range(__float_as_int(mn0), nbits20).mn, vertex_range(__float_as_int(mx0), nbits20).mx};
-  const KeyRange y{vertex_range(__float_as_int(mn1), nbits20).mn, vertex_range(__float_as_int(mx1), nbits20).mx};
-  const KeyRange z{vertex_range(__float_as_int(mn2), nbits20).mn, vertex_range(__float_as_int(mx2), nbits20).mx};
-  return cube_excluded3(x, y, z);
-}
-
-template <bool HAS_NEXT, bool EDGE>
-__device__ __forceinline__ void fused3d_consume(const SweepParams &p, const unsigned char *ring, const uint32_t full0, const uint32_t empty0,
-                                                const int C0, const int Y0, const int zc0, const int zc1, const int wib, const int lane) {
-  constexpr int NL = HAS_NEXT ? 2 : 1;
-  const int W = p.W, H = p.H, D = p.D;
-  const int e = C0 + 2 * lane;                 // this lane's columns: e, e + 1
-  const int y0 = Y0 + wib * F3_RW;             // first corner row of this warp
-  const int tr0 = wib * F3_RW;                 // its row in the staged tile is tr0 + 1 (tile row 0 = Y0 - 1)
-  const float nanf_ = __int_as_float(KEYF_NAN);
-  const float kthr = __int_as_float((1023 + 1 - p.nbits) << 20);    // key of 2^(1-nbits): |d| >= 2^(1-nbits) <=> |quantised v| >= 1
-  const int esum_max = 3119 - 3 * p.nbits;     // exponent bound of the determinant guard (see below)
-  const float kfloor = __int_as_float((1023 - p.nbits) << 20);      // key of 2^-nbits: smaller magnitudes quantise to 0
-  const int nbits20 = (p.nbits - 1) << 20;
-  const bool want_res[2] = {p.res_slot[0] != nullptr, HAS_NEXT && p.res_slot[1] != nullptr};
-  double rmin[2] = {DBL_MAX, DBL_MAX};
-  float rkey[2] = {__int_as_float(0x7F800000), __int_as_float(0x7F800000)};   // key of 2 |rmin|; +Inf (as a float): nothing found yet
-  bool bad = false;
-
-  // EDGE tiles: columns / rows outside the tracker's domain stay out of the ranges (NaN key), vertices on the
-  // array border have a zero gradient, vertices outside the array interior stay out of the resolution
-  bool arr_c[2] = {true, true}, dom_c[2] = {true, true};
-  bool own_any = lane <= 30;
-  if (EDGE) {
-    bool any_col = false;
-#pragma unroll
-    for (int q = 0; q < 2; q++) {
-      arr_c[q] = e + q >= 1 && e + q <= W - 2;
-      dom_c[q] = e + q >= p.lb[0] && e + q <= p.ub[0];
-      any_col = any_col || dom_c[q];
-    }
-    own_any = own_any && any_col && y0 <= p.ub[1] && y0 + F3_RW - 1 >= p.lb[1];
-  }
-
-  float pmin[3] = {nanf_, nanf_, nanf_}, pmax[3] = {nanf_, nanf_, nanf_};   // previous plane's union (neighbour lane merged)
-  int st_m = 0, st_c = 1, st_p = 2;            // ring stages of planes zg-1, zg, zg+1
-  uint32_t par_p = 0;                          // parity of the next completion of full[st_p]
-  mbar_wait(full0, 0);
-  mbar_wait(full0 + 8, 0);
-  for (int zg = zc0; zg <= zc1 + 1; zg++) {
-    mbar_wait(full0 + 8u * st_p, par_p);
-    const bool zarr = zg >= 1 && zg <= D - 2;
-    const bool zdom = zg >= p.lb[2] && zg <= p.ub[2];
-    float umin[3] = {nanf_, nanf_, nanf_}, umax[3] = {nanf_, nanf_, nanf_};
-#pragma unroll
-    for (int L = 0; L < NL; L++) {
-      const double *Pc = reinterpret_cast<const double *>(ring + (size_t)st_c * (NL * F3_LAYER_BYTES) + (size_t)L * F3_LAYER_BYTES) + 2 * lane;
-      const double *Pm = reinterpret_cast<const double *>(ring + (size_t)st_m * (NL * F3_LAYER_BYTES) + (size_t)L * F3_LAYER_BYTES) + 2 * lane;
-      const double *Pp = reinterpret_cast<const double *>(ring + (size_t)st_p * (NL * F3_LAYER_BYTES) + (size_t)L * F3_LAYER_BYTES) + 2 * lane;
-      const bool res_now = want_res[L] && zarr;
-      double2 rm = *reinterpret_cast<const double2 *>(Pc + (tr0 + 0) * F3_COLS + 2);
-      double2 rc = *reinterpret_cast<const double2 *>(Pc + (tr0 + 1) * F3_COLS + 2);
-#pragma unroll
-      for (int r = 0; r <= F3_RW; r++) {
-        const int row = tr0 + r + 1;
-        const double2 rp = *reinterpret_cast<const double2 *>(Pc + (row + 1) * F3_COLS + 2);
-        const double left = Pc[row * F3_COLS + 1], right = Pc[row * F3_COLS + 4];
-        const double2 zm = *reinterpret_cast<const double2 *>(Pm + row * F3_COLS + 2);
-        const double2 zp = *reinterpret_cast<const double2 *>(Pp + row * F3_COLS + 2);
-        const double dxe = rc.y - left, dxo = right - rc.x;
-        const double dye = rp.x - rm.x, dyo = rp.y - rm.y;
-        const double dze = zp.x - zm.x, dzo = zp.y - zm.y;
-        float kxe = hikey(dxe), kxo = hikey(dxo), kye = hikey(dye), kyo = hikey(dyo), kze = hikey(dze), kzo = hikey(dzo);
-        bad = bad || !(fabsf(hikey(rc.x)) < __int_as_float(KEYF_BIG)) || !(fabsf(hikey(rc.y)) < __int_as_float(KEYF_BIG));
-        bool in_e = true, in_o = true;
-        if (EDGE) {
-          const int y = y0 + r;
-          const bool arr_y = y >= 1 && y <= H - 2;
-          in_e = arr_c[0] && arr_y; in_o = arr_c[1] && arr_y;
-        }
-        if (res_now) {
-          float a = fminf(fminf(fabsf(kxe), fabsf(kye)), fabsf(kze)), b = fminf(fminf(fabsf(kxo), fabsf(kyo)), fabsf(kzo));
-          if (EDGE) { a = in_e ? a : __int_as_float(0x7F800000); b = in_o ? b : __int_as_float(0x7F800000); }
-          if (fminf(a, b) <= rkey[L]) {
-            res_update3(rmin[L], in_e, dxe, dye, dze);
-            res_update3(rmin[L], in_o, dxo, dyo, dzo);
-            rkey[L] = rmin[L] == DBL_MAX ? __int_as_float(0x7F800000) : hikey(2.0 * fabs(rmin[L]));
-          }
-        }
-        if (EDGE) {
-          const int y = y0 + r;
-          const bool dom_y = y >= p.lb[1] && y <= p.ub[1];
-          const int keep_e = (in_e && dom_c[0] && dom_y) ? -1 : 0, fill_e = (dom_c[0] && dom_y) ? 0 : KEYF_NAN;
-          const int keep_o = (in_o && dom_c[1] && dom_y) ? -1 : 0, fill_o = (dom_c[1] && dom_y) ? 0 : KEYF_NAN;
-          kxe = __int_as_float((__float_as_int(kxe) & keep_e) | fill_e); kxo = __int_as_float((__float_as_int(kxo) & keep_o) | fill_o);
-          kye = __int_as_float((__float_as_int(kye) & keep_e) | fill_e); kyo = __int_as_float((__float_as_int(kyo) & keep_o) | fill_o);
-          kze = __int_as_float((__float_as_int(kze) & keep_e) | fill_e); kzo = __int_as_float((__float_as_int(kzo) & keep_o) | fill_o);
-        }
-        umin[0] = fminf(umin[0], fminf(kxe, kxo)); umax[0] = fmaxf(umax[0], fmaxf(kxe, kxo));
-        umin[1] = fminf(umin[1], fminf(kye, kyo)); umax[1] = fmaxf(umax[1], fmaxf(kye, kyo));
-        umin[2] = fminf(umin[2], fminf(kze, kzo)); umax[2] = fmaxf(umax[2], fmaxf(kze, kzo));
-        rm = rc; rc = rp;
-      }
-    }
-    // plane-level masks (warp-uniform): planes outside the domain stay out of the ranges; the array's first and
-    // last plane have a zero gradient
-    if (!zdom || !zarr) {
-#pragma unroll
-      for (int c = 0; c < 3; c++) {
-        const bool has = zdom && !(umin[c] != umin[c]);     // lanes with no in-domain vertex keep the neutral element
-        umin[c] = has ? 0.f : nanf_; umax[c] = has ? 0.f : nanf_;
-      }
-    }
-    // x neighbour: corner column e+1 also uses the next lane's first column
-#pragma unroll
-    for (int c = 0; c < 3; c++) {
-      umin[c] = fminf(umin[c], __shfl_down_sync(0xffffffffu, umin[c], 1));
-      umax[c] = fmaxf(umax[c], __shfl_down_sync(0xffffffffu, umax[c], 1));
-    }
-    if (zg > zc0) {
-      const int zc = zg - 1;                     // corner plane decided now (warp-uniform)
-      if (zc >= p.lb[2] && zc <= p.ub[2]) {
-        float cmn[3], cmx[3];
-        bool sided = false;
-        int esum = 0;
-#pragma unroll
-        for (int c = 0; c < 3; c++) {
-          cmn[c] = fminf(pmin[c], umin[c]); cmx[c] = fmaxf(pmax[c], umax[c]);
-          sided = sided || cmn[c] >= kthr || cmx[c] <= -kthr;
-          esum += (__float_as_int(fmaxf(fmaxf(fabsf(cmn[c]), fabsf(cmx[c])), kfloor)) >> 20);
-        }
-        // determinant guard, exponent form: with e_c the biased exponent of max |d_c| (at least that of 2^-nbits),
-        // |quantised v_c| < 2^(e_c - 1023 + nbits) and M_c := |quantised| + 1 <= 2^(e_c - 1022 + nbits).  Every determinant of the
-        // cascade is at most 48 Mx My Mz (cube_excluded3 with R <= 2 M) < 2^(6 + sum(e_c) - 3066 + 3 nbits), which stays
-        // below 2^62 for sum(e_c) <= 3119 - 3 nbits.
-        // A NaN union (no vertex) or Inf fails the bound and takes the precise / cold path.
-        bool excl = sided && esum <= esum_max && !(cmn[0] != cmn[0]);
-        if (sided && !excl && own_any) excl = fused3d_union_excluded_precise(cmn[0], cmx[0], cmn[1], cmx[1], cmn[2], cmx[2], nbits20);
-        const bool fail = own_any && !excl;
-        { const unsigned fm = __ballot_sync(0xffffffffu, fail); if (fm) fused3d_slow_cubes(p, fm, C0, y0, zc, NL); }
-      }
-    }
-#pragma unroll
-    for (int c = 0; c < 3; c++) { pmin[c] = umin[c]; pmax[c] = umax[c]; }
-    // plane zg-1 is dead for this warp
-    __syncwarp();
-    if (elect_one()) mbar_arrive(empty0 + 8u * st_m);
-    st_m = st_c; st_c = st_p;
-    st_p = st_p + 1 == F3_NST ? 0 : st_p + 1;
-    if (st_p == 0) par_p ^= 1u;
-  }
-#pragma unroll
-  for (int L = 0; L < NL; L++)
-    if (want_res[L]) warp_res_commit(fabs(rmin[L]), p.res_slot[L]);
-  if (bad) atomicExch(p.poison, 1ull);
-}
-
-template <bool HAS_NEXT>
-__global__ void __launch_bounds__((F3_CW + 1) * 32, 1) scan3d_fused_kernel(const __grid_constant__ SweepParams p) {
-  constexpr int NL = HAS_NEXT ? 2 : 1;
-  constexpr uint32_t STAGE_BYTES = NL * F3_LAYER_BYTES;
-  extern __shared__ __align__(128) unsigned char fb_smem[];
-  const int lane = threadIdx.x & 31;
-  const int wib = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);     // warp-uniform by construction
-  const uint32_t ring_u32 = smem_u32(fb_smem);
-  const uint32_t full0 = ring_u32 + (uint32_t)F3_NST * STAGE_BYTES, empty0 = full0 + 8u * F3_NST;
-  int b = blockIdx.x;
-  const int bx = b % p.nsx; b /= p.nsx;
-  const int by = b % p.nsy;
-  const int bz = b / p.nsy;
-  const int C0 = bx * F3_STRIDE, Y0 = by * F3_TROWS;
-  const int zc0 = bz * p.rows, zc1 = min(zc0 + p.rows - 1, p.D - 1);
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int q = 0; q < F3_NST; q++) { mbar_init(full0 + 8u * q, 1); mbar_init(empty0 + 8u * q, F3_CW); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  }
-  __syncthreads();
-  if (wib == F3_CW) {
-    // producer: scalar planes zc0-1 .. zc1+2 of every layer, one TMA box (tile + halo) each
-    if (elect_one()) {
-      const int nplanes = zc1 - zc0 + 4;
-      for (int s = 0; s < nplanes; s++) {
-        const int st = s % F3_NST;
-        if (s >= F3_NST) mbar_wait(empty0 + 8u * st, (uint32_t)((s / F3_NST - 1) & 1));
-        mbar_expect_tx(full0 + 8u * st, F3_BOX_BYTES * NL);
-#pragma unroll
-        for (int L = 0; L < NL; L++)
-          tma_load_3d(ring_u32 + (uint32_t)st * STAGE_BYTES + (uint32_t)L * F3_LAYER_BYTES, &p.tmap[L], C0 - 2, Y0 - 1, zc0 - 1 + s, full0 + 8u * st);
-      }
-    }
-    return;
-  }
-  // tiles whose 64 x (TROWS + 1) gradient vertices all lie in the array interior and in the tracker's domain skip the masks
-  const bool interior = C0 >= max(1, p.lb[0]) && C0 + 63 <= min(p.W - 2, p.ub[0]) && Y0 >= max(1, p.lb[1]) && Y0 + F3_TROWS <= min(p.H - 2, p.ub[1]);
-  if (interior) fused3d_consume<HAS_NEXT, false>(p, fb_smem, full0, empty0, C0, Y0, zc0, zc1, wib, lane);
-  else fused3d_consume<HAS_NEXT, true>(p, fb_smem, full0, empty0, C0, Y0, zc0, zc1, wib, lane);
-}
-
 // ---- 3D, scalar input, per-layer range summaries ("build once, test from summaries") -----------------------
-// The per-thread unions of the fused scan depend on ONE layer only (raw keys of the gradient, domain masks),
-// not on the quantisation factor.  A layer is therefore streamed from HBM once in its life: the step that
-// first sees it (as the "next" layer) derives its gradient keys, folds min non-zero |v|, and stores each
-// thread's union (after the x-neighbour merge) as a 16-byte cell -- six keys truncated to their upper 16
-// bits (sign, 11 exponent bits, 4 mantissa bits).  The exclusion test only compares keys against powers of
-// two and sums exponents, so truncation towards zero changes none of its decisions.  The same step reads
-// the CURRENT layer's cells (written one step earlier) instead of the layer itself: 8 B/vertex of scalars
-// + 2 B/vertex of cells written + 2 B/vertex read, against 16 B/vertex for the two-layer scan, and half the
-// arithmetic.  Re-sweeps (a stale speculated factor, worklist growth) and the final ordinal-only sweep read
-// cells only.
+// A CTA of eight warps owns a tile of F3_STRIDE x F3_TROWS corner columns and marches along z over a chunk of
+// planes; a thread covers 2 columns x S3_RW corner rows.  The per-thread unions of gradient keys depend on ONE
+// layer only (raw keys of the gradient, domain masks), not on the quantisation factor.  A layer is therefore
+// streamed from HBM once in its life: the step that first sees it (as the "next" layer) derives its gradient
+// keys, folds min non-zero |v|, and stores each thread's union (after the x-neighbour merge) as a 16-byte cell
+// -- six keys truncated to their upper 16 bits (sign, 11 exponent bits, 4 mantissa bits).  The exclusion test
+// only compares keys against powers of two and sums exponents, so truncation towards zero changes none of its
+// decisions.  The same step reads the CURRENT layer's cells (written one step earlier) instead of the layer
+// itself: 8 B/vertex of scalars + 2 B/vertex of cells written + 2 B/vertex read, against 16 B/vertex for a scan
+// that re-reads both layers, and half the arithmetic.  Re-sweeps (a stale speculated factor, worklist growth)
+// and the final ordinal-only sweep read cells only.
 //
-// Staging: as above (TMA box per plane, full/empty mbarriers, producer warp), one layer per stage.  Each
-// consumer thread keeps a three-plane register window of its 2 columns x (S3_RW + 3) rows, so a plane is read
-// from shared memory once (plus the two x-neighbour columns while it is the centre plane).
+// Staging: a ring of S3_NST planes of the layer being built, one TMA box (tile + halo, out-of-bounds elements
+// zero-filled) per plane and stage; no producer warp (see S3Build::release).  Each consumer thread keeps a
+// three-plane register window of its 2 columns x (S3_RW + 3) rows, so a plane is read from shared memory once
+// (plus the two x-neighbour columns while it is the centre plane).
 constexpr int S3_RW = F3_RW;                       // corner rows per consumer warp
 constexpr int S3_WR = S3_RW + 1;                   // window rows per plane: the gradient rows y0 .. y0+RW (the two halo rows of the
                                                    // centre plane are re-read from shared memory while it is the centre)
@@ -1904,7 +1245,7 @@ __device__ __forceinline__ S3Thresholds s3_thresholds(const int nbits, const boo
   S3Thresholds t;
   t.kthr = __int_as_float((1023 + 1 - s - nbits) << 20);   // key of 2^(1-nbits) (d) / 2^-nbits (v): at or above it |quantised v| >= 1
   t.kfloor = __int_as_float((1023 - s - nbits) << 20);     // half of that: smaller magnitudes quantise to 0
-  t.esum_max = 3119 - 3 * s - 3 * nbits;                    // determinant guard, see fused3d_consume
+  t.esum_max = 3119 - 3 * s - 3 * nbits;                    // determinant guard, see the 3D section header
   t.nbits20 = (nbits - 1 + s) << 20;
   t.half_factor = __hiloint2double((1023 + nbits - 1 + s) << 20, 0);   // v 2^nbits = d 2^(nbits-1)
   return t;
@@ -1959,7 +1300,7 @@ __device__ __forceinline__ void s3_test(const SweepParams &p, const S3Thresholds
     mag[c] = fmaxf(fabsf(cmn[c]), fabsf(cmx[c]));
     esum += (__float_as_int(fmaxf(mag[c], T.kfloor)) >> 20);
   }
-  // determinant guard, level 1 (exponents only, see fused3d_consume).  A NaN union (no vertex) fails every level and
+  // determinant guard, level 1 (exponents only, see the 3D section header).  A NaN union (no vertex) fails every level and
   // takes the cold path, which is exact.
   bool excl = sided && esum <= T.esum_max && !(cmn[0] != cmn[0]);
   if (sided && !excl && own_any && !(cmn[0] != cmn[0])) {
@@ -2535,191 +1876,6 @@ __global__ void __launch_bounds__(256) vscan2d_cells_kernel(const __grid_constan
   vcells2d_decide(p, xmn, xmx, ymn, ymx, own, c0, y0, NL);
 }
 
-// ---- 2D, scalar input, range cells, direct loads ("direct" staging, the default) ------------------------------------
-// Same cells idea as scan2d_build_kernel, without shared memory: a warp owns a strip of 62 corner columns (64 vertex
-// columns, two per lane, one 16-byte load per lane and row) and marches along y eight rows at a time -- all eight loads
-// of a batch are issued before the first is used, so every thread keeps 128 B in flight; x neighbours come from warp
-// shuffles (lanes 0 and 31 load their one outside column), y neighbours from a two-row carry.  Ranges are kept on the
-// HIGH WORDS of the fp64 differences (monotone float keys, no conversion instruction in the row loop); a cell is four
-// such keys {min dx, max dx, min dy, max dy} per lane and 8-row block.  At block end the keys are widened outwards to
-// fp64, scaled by (W-1) / (H-1) like gradient2D does, rounded outwards to fp32, and go through cube_excluded2_f.
-__device__ __forceinline__ double key_bound_lo(const float k) {     // a double <= every value whose high word is k
-  const int h = __float_as_int(k);
-  return __hiloint2double(h, h < 0 ? (int)0xffffffffu : 0);
-}
-__device__ __forceinline__ double key_bound_hi(const float k) {     // a double >= every value whose high word is k
-  const int h = __float_as_int(k);
-  return __hiloint2double(h, h < 0 ? 0 : (int)0xffffffffu);
-}
-
-__device__ __forceinline__ void dcells2d_decide(const SweepParams &p, const float xmn, const float xmx, const float ymn, const float ymx,
-                                                const bool own, const int c0, const int y0, const int nl) {
-  const double cw = (double)(p.W - 1), ch = (double)(p.H - 1);
-  // NaN keys (no vertex) give NaN bounds: cube_excluded2_f then refuses and the cold path decides
-  const FRange x{__double2float_rd(key_bound_lo(xmn) * cw), __double2float_ru(key_bound_hi(xmx) * cw)};
-  const FRange y{__double2float_rd(key_bound_lo(ymn) * ch), __double2float_ru(key_bound_hi(ymx) * ch)};
-  const bool none = xmn != xmn || ymn != ymn;      // no vertex in the union: let the cold path look
-  const bool fail = own && (none || !cube_excluded2_f(x, y, p.thrp_f, p.thr2_f, p.lim_f));
-  const unsigned fm = __ballot_sync(0xffffffffu, fail);
-  if (fm) cells2d_slow_cubes(p, fm, c0, y0, nl, V2_R);
-}
-
-// min non-zero |v| of the layer, v = d (W-1) resp. d (H-1): the scale factors are constants >= 1, so the product is
-// monotone in |d| and never underflows to zero -- the kernel keeps the exact minimum of the non-zero |dx| and |dy| per
-// axis (with the float keys as a prefilter) and scales once at the end, which gives bit for bit the minimum that
-// res_update4 finds value by value.
-__device__ __forceinline__ void dmin_nz(double &m, float &mk, const bool in, const double d) {
-  const double a = fabs(d);
-  if (in && d != 0.0 && a < m) { m = a; mk = hikey(a); }      // NaN / Inf never compare below
-}
-
-template <bool BORDER, int NPREV, bool TEST>
-__device__ __forceinline__ void dcells2d_strip(const SweepParams &p, const int strip, const int cy, const int lane) {
-  const int W = p.W, H = p.H, B = p.build_layer;
-  const int c0 = strip * FB_STRIDE, e = c0 + 2 * lane;
-  const bool e_ok = !BORDER || e < W, o_ok = !BORDER || e + 1 < W, o1_ok = !BORDER || e + 2 < W;
-  const bool e_dom = e >= p.lb[0] && e <= p.ub[0], o_dom = e + 1 >= p.lb[0] && e + 1 <= p.ub[0];
-  const bool own_cols = lane <= 30 && (e_dom || o_dom);
-  const int r0 = cy * p.rows, r1 = min(r0 + p.rows - 1, H - 1), jl = min(r1 + 1, H - 1);
-  const double *__restrict__ S = p.L[B].S;
-  const bool want_res = p.res_slot[B] != nullptr;
-  const double cw = (double)(W - 1), ch = (double)(H - 1);
-  const float nanf_ = __int_as_float(KEYF_NAN), inff_ = __int_as_float(0x7F800000);
-  double mdx = DBL_MAX, mdy = DBL_MAX;       // min non-zero |dx|, |dy| seen by this thread
-  float tkx = inff_, tky = inff_;            // their high-word keys (prefilter)
-  const uint4 *sum_prev = NPREV ? p.sum_in[0] + vcells2d_index(p, strip, 0, lane) : nullptr;
-  uint4 *sum_out = p.sum_out + vcells2d_index(p, strip, 0, lane);
-  // the one column outside the strip that this lane supplies: lane 0 the left one, lane 31 the right one (index clamped like gradient2D)
-  const bool edge_lane = lane == 0 || lane == 31;
-  const int edge_col = lane == 0 ? max(c0 - 1, 0) : min(c0 + 64, W - 1);
-
-  auto load_row = [&](const int j, double2 &v, double &ed) {
-    const size_t row = (size_t)W * (size_t)min(max(j, 0), H - 1);
-    v = e_ok ? __ldg(reinterpret_cast<const double2 *>(S + row + e)) : make_double2(0.0, 0.0);
-    ed = edge_lane ? __ldg(S + row + edge_col) : 0.0;
-  };
-  auto finish_block = [&](const int kb, float xmn, float xmx, float ymn, float ymx, const uint4 prevc) {
-    xmn = fminf(xmn, __shfl_down_sync(0xffffffffu, xmn, 1)); xmx = fmaxf(xmx, __shfl_down_sync(0xffffffffu, xmx, 1));
-    ymn = fminf(ymn, __shfl_down_sync(0xffffffffu, ymn, 1)); ymx = fmaxf(ymx, __shfl_down_sync(0xffffffffu, ymx, 1));
-    sum_out[(size_t)kb * 32u] = make_uint4(__float_as_uint(xmn), __float_as_uint(xmx), __float_as_uint(ymn), __float_as_uint(ymx));
-    if (TEST) {
-      if (NPREV) {
-        xmn = fminf(xmn, __uint_as_float(prevc.x)); xmx = fmaxf(xmx, __uint_as_float(prevc.y));
-        ymn = fminf(ymn, __uint_as_float(prevc.z)); ymx = fmaxf(ymx, __uint_as_float(prevc.w));
-      }
-      const int y0 = kb * V2_R;
-      dcells2d_decide(p, xmn, xmx, ymn, ymx, own_cols && y0 <= p.ub[1] && y0 + V2_R - 1 >= p.lb[1], c0, y0, NPREV + 1);
-    }
-  };
-
-  // carry: vertex rows g-1 (m1) and g (c0v, with its edge value) of the next gradient row g
-  double2 m1, cv;
-  double m1e, cve;
-  load_row(r0 - 1, m1, m1e);
-  load_row(r0, cv, cve);
-  float bxmn = nanf_, bxmx = nanf_, bymn = nanf_, bymx = nanf_;
-  uint4 prevc = make_uint4(0x7FC00000u, 0x7FC00000u, 0x7FC00000u, 0x7FC00000u);
-  for (int g0 = r0; g0 <= jl; g0 += V2_R) {
-    // vertex rows g0+1 .. g0+8: the rows above the gradient rows g0 .. g0+7 of this batch
-    double2 a[V2_R];
-    double ae[V2_R];
-#pragma unroll
-    for (int k = 0; k < V2_R; k++) {
-      if (g0 + k <= jl) load_row(g0 + k + 1, a[k], ae[k]);
-      else { a[k] = make_double2(0.0, 0.0); ae[k] = 0.0; }
-    }
-    uint4 prevn = prevc;
-    if (NPREV) prevn = __ldg(sum_prev + (size_t)(g0 / V2_R) * 32u);     // the block this batch opens
-#pragma unroll
-    for (int k = 0; k < V2_R; k++) {
-      const int g = g0 + k;
-      if (g > jl) break;
-      const double2 up = a[k];
-      // x neighbours: column e-1 is the previous lane's second column, column e+2 the next lane's first
-      double left = __shfl_up_sync(0xffffffffu, cv.y, 1), right = __shfl_down_sync(0xffffffffu, cv.x, 1);
-      if (lane == 0) left = cve;
-      if (lane == 31) right = cve;
-      double mid_e = cv.y;
-      if (BORDER) {
-        if (!o_ok) mid_e = cv.x;          // x+1 clamped to W-1
-        if (!o1_ok) right = cv.y;
-      }
-      const double dxe = mid_e - left, dxo = right - cv.x, dye = up.x - m1.x, dyo = up.y - m1.y;
-      float kxe = hikey(dxe), kxo = hikey(dxo), kye = hikey(dye), kyo = hikey(dyo);
-      if (want_res) {
-        float ax = fminf(fabsf(kxe), fabsf(kxo)), ay = fminf(fabsf(kye), fabsf(kyo));
-        if (BORDER) {
-          ax = fminf(e_ok ? fabsf(kxe) : inff_, o_ok ? fabsf(kxo) : inff_);
-          ay = fminf(e_ok ? fabsf(kye) : inff_, o_ok ? fabsf(kyo) : inff_);
-        }
-        if (ax <= tkx) { dmin_nz(mdx, tkx, e_ok, dxe); dmin_nz(mdx, tkx, o_ok, dxo); }
-        if (ay <= tky) { dmin_nz(mdy, tky, e_ok, dye); dmin_nz(mdy, tky, o_ok, dyo); }
-      }
-      const bool dom_y = g >= p.lb[1] && g <= p.ub[1];
-      if (!(e_dom && dom_y)) { kxe = nanf_; kye = nanf_; }
-      if (!(o_dom && dom_y)) { kxo = nanf_; kyo = nanf_; }
-      const float rxmn = fminf(kxe, kxo), rxmx = fmaxf(kxe, kxo), rymn = fminf(kye, kyo), rymx = fmaxf(kye, kyo);
-      if (k == 0) {
-        // gradient row 8 k closes block k-1 and opens block k
-        if (g > r0) finish_block(g / V2_R - 1, fminf(bxmn, rxmn), fmaxf(bxmx, rxmx), fminf(bymn, rymn), fmaxf(bymx, rymx), prevc);
-        bxmn = rxmn; bxmx = rxmx; bymn = rymn; bymx = rymx;
-        prevc = prevn;
-      } else {
-        bxmn = fminf(bxmn, rxmn); bxmx = fmaxf(bxmx, rxmx); bymn = fminf(bymn, rymn); bymx = fmaxf(bymx, rymx);
-      }
-      m1 = cv; cv = up; cve = ae[k];
-    }
-  }
-  if (jl == H - 1) finish_block(jl / V2_R, bxmn, bxmx, bymn, bymx, prevc);     // the array's last block ends at row H-1
-  if (want_res) {
-    const double vx = mdx < DBL_MAX ? mdx * cw : DBL_MAX, vy = mdy < DBL_MAX ? mdy * ch : DBL_MAX;
-    warp_res_commit(fmin(vx, vy), p.res_slot[B]);
-  }
-}
-
-template <int NPREV, bool TEST>
-__global__ void __launch_bounds__(256, 2) scan2d_direct_kernel(const __grid_constant__ SweepParams p) {
-  const int lane = threadIdx.x & 31;
-  const i64 w = (i64)blockIdx.x * 8 + (threadIdx.x >> 5);
-  const int strip = (int)(w % p.nsx), cy = (int)(w / p.nsx);
-  if (cy >= p.nsy) return;
-  const int c0 = strip * FB_STRIDE;
-  if (c0 + 66 > p.W) dcells2d_strip<true, NPREV, TEST>(p, strip, cy, lane);        // the last strip clamps its columns
-  else dcells2d_strip<false, NPREV, TEST>(p, strip, cy, lane);
-}
-
-template <int NL>
-__global__ void __launch_bounds__(256) scan2d_direct_cells_kernel(const __grid_constant__ SweepParams p, const int nstrips, const int nblk_used) {
-  const int lane = threadIdx.x & 31;
-  const long long w = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
-  if (w >= (long long)nstrips * nblk_used) return;
-  const int strip = (int)(w / nblk_used), kb = (int)(w % nblk_used);
-  const int c0 = strip * FB_STRIDE, e = c0 + 2 * lane, y0 = kb * V2_R;
-  const bool own = lane <= 30 && ((e >= p.lb[0] && e <= p.ub[0]) || (e + 1 >= p.lb[0] && e + 1 <= p.ub[0])) && y0 <= p.ub[1] && y0 + V2_R - 1 >= p.lb[1];
-  if (!__any_sync(0xffffffffu, own)) return;
-  const float nanf_ = __int_as_float(KEYF_NAN);
-  float xmn = nanf_, xmx = nanf_, ymn = nanf_, ymx = nanf_;
-#pragma unroll
-  for (int L = 0; L < NL; L++) {
-    const uint4 c = __ldg(p.sum_in[L] + vcells2d_index(p, strip, kb, lane));
-    xmn = fminf(xmn, __uint_as_float(c.x)); xmx = fmaxf(xmx, __uint_as_float(c.y));
-    ymn = fminf(ymn, __uint_as_float(c.z)); ymx = fmaxf(ymx, __uint_as_float(c.w));
-  }
-  dcells2d_decide(p, xmn, xmx, ymn, ymx, own, c0, y0, NL);
-}
-
-void launch_scan2d_direct(const SweepParams &p, cudaStream_t s) {
-  const unsigned grid = (unsigned)(((i64)p.nsx * p.nsy + 7) / 8);
-  const int nblk = (p.H + V2_R - 1) / V2_R;
-  const unsigned tgrid = (unsigned)(((i64)p.nsx * nblk + 7) / 8);
-  switch (p.sum_mode) {
-    case SUM_BUILD: scan2d_direct_kernel<0, false><<<grid, 256, 0, s>>>(p); break;
-    case SUM_BUILD_TEST1: scan2d_direct_kernel<0, true><<<grid, 256, 0, s>>>(p); break;
-    case SUM_BUILD_TEST2: scan2d_direct_kernel<1, true><<<grid, 256, 0, s>>>(p); break;
-    case SUM_TEST1: scan2d_direct_cells_kernel<1><<<tgrid, 256, 0, s>>>(p, p.nsx, nblk); break;
-    default: scan2d_direct_cells_kernel<2><<<tgrid, 256, 0, s>>>(p, p.nsx, nblk); break;
-  }
-}
 
 // 3D: CTA = 8 warps over a tile of 62 x 32 corner columns, marching along a chunk of planes; per plane a thread reads
 // its 2 columns x (S3_RW + 1) rows (three 16-byte loads per row)
@@ -2877,9 +2033,6 @@ void launch_vscan_cells(const SweepParams &p, cudaStream_t s) {
   }
 }
 
-static size_t fused3d_smem_bytes(bool has_next) {
-  return (size_t)F3_NST * (has_next ? 2 : 1) * F3_LAYER_BYTES + (size_t)2 * F3_NST * 8;
-}
 
 typedef CUresult (*TmapEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *, const cuuint32_t *,
                                  const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -2903,27 +2056,13 @@ bool encode_scalar_tmap3d(const double *S, int W, int H, int D, CUtensorMap *out
             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-static size_t tile_smem_bytes(bool has_next) {
-  return (size_t)TL_NST * (has_next ? 2 : 1) * TL_SEG * 8 + (size_t)2 * TL_NST * 8;
-}
-
-static size_t bulk_smem_bytes(bool has_next) {
-  return (size_t)FB_WARPS * FB_NST * (has_next ? 2 : 1) * FB_SEG * 8 + (size_t)FB_WARPS * FB_NST * 8;
-}
-
-static void init_carveouts();
 void init_kernel_attributes() {
-  init_carveouts();
-  cudaFuncSetAttribute(scan2d_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem_bytes(true));
-  cudaFuncSetAttribute(scan2d_tile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem_bytes(false));
-  cudaFuncSetAttribute(scan2d_bulk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bulk_smem_bytes(true));
-  cudaFuncSetAttribute(scan2d_bulk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bulk_smem_bytes(false));
-  cudaFuncSetAttribute(scan3d_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fused3d_smem_bytes(true));
-  cudaFuncSetAttribute(scan3d_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fused3d_smem_bytes(false));
   cudaFuncSetAttribute(scan2d_build_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c2_smem_bytes());
-  k2_attrs<2, 8>(); k2_attrs<3, 4>(); k2_attrs<3, 5>(); k2_attrs<3, 6>(); k2_attrs<4, 4>();
   cudaFuncSetAttribute(scan2d_build_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c2_smem_bytes());
   cudaFuncSetAttribute(scan2d_build_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)c2_smem_bytes());
+  cudaFuncSetAttribute(scan2d_keys_build_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k2_smem_bytes());
+  cudaFuncSetAttribute(scan2d_keys_build_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k2_smem_bytes());
+  cudaFuncSetAttribute(scan2d_keys_build_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k2_smem_bytes());
   cudaFuncSetAttribute(scan3d_build_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s3_smem_bytes());
   cudaFuncSetAttribute(scan3d_build_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s3_smem_bytes());
   cudaFuncSetAttribute(scan3d_build_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s3_smem_bytes());
@@ -2942,38 +2081,14 @@ void launch_scan3d_cells(const SweepParams &p, cudaStream_t s) {
 }
 
 void launch_scan(const SweepParams &p, cudaStream_t s) {
-  if (p.nd == 2 && p.fused && p.aligned16 && p.bulk == 2) {
-    const unsigned grid = (unsigned)((i64)p.nsx * p.nsy);
-    if (p.has_next) scan2d_tile_kernel<true><<<grid, (TL_CW + 1) * 32, tile_smem_bytes(true), s>>>(p);
-    else scan2d_tile_kernel<false><<<grid, (TL_CW + 1) * 32, tile_smem_bytes(false), s>>>(p);
-  } else if (p.nd == 2 && p.fused && p.aligned16 && p.bulk) {
-    const i64 warps = (i64)p.nsx * p.nsy;
-    const unsigned grid = (unsigned)((warps + FB_WARPS - 1) / FB_WARPS);
-    if (p.has_next) scan2d_bulk_kernel<true><<<grid, FB_WARPS * 32, bulk_smem_bytes(true), s>>>(p);
-    else scan2d_bulk_kernel<false><<<grid, FB_WARPS * 32, bulk_smem_bytes(false), s>>>(p);
-  } else if (p.nd == 2 && p.fused) {
-    const i64 warps = (i64)p.nsx * p.nsy;
-    const int wpb = 8;
-    const unsigned grid = (unsigned)((warps + wpb - 1) / wpb);
-    if (p.has_next) {
-      if (p.aligned16) scan2d_fused_kernel<true, true><<<grid, wpb * 32, 0, s>>>(p);
-      else scan2d_fused_kernel<true, false><<<grid, wpb * 32, 0, s>>>(p);
-    } else {
-      if (p.aligned16) scan2d_fused_kernel<false, true><<<grid, wpb * 32, 0, s>>>(p);
-      else scan2d_fused_kernel<false, false><<<grid, wpb * 32, 0, s>>>(p);
-    }
-  } else if (p.nd == 3 && p.fused) {
-    const unsigned grid = (unsigned)((i64)p.nsx * p.nsy * p.nsz);
-    if (p.has_next) scan3d_fused_kernel<true><<<grid, (F3_CW + 1) * 32, fused3d_smem_bytes(true), s>>>(p);
-    else scan3d_fused_kernel<false><<<grid, (F3_CW + 1) * 32, fused3d_smem_bytes(false), s>>>(p);
+  const unsigned grid = p.nd == 2 ? (unsigned)(((i64)p.nsx * p.nsy + 7) / 8) : (unsigned)((i64)p.nsx * p.nsy * p.nsz);
+  if (p.nd == 2 && p.fused) {     // rows that are not 16-byte aligned (aligned ones take the range-cell kernels)
+    if (p.has_next) scan2d_fused_kernel<true><<<grid, 256, 0, s>>>(p);
+    else scan2d_fused_kernel<false><<<grid, 256, 0, s>>>(p);
   } else if (p.nd == 2) {
-    const i64 warps = (i64)p.nsx * p.nsy;
-    const int wpb = 8;
-    const unsigned grid = (unsigned)((warps + wpb - 1) / wpb);
-    if (p.has_next) scan2d_kernel<true><<<grid, wpb * 32, 0, s>>>(p);
-    else scan2d_kernel<false><<<grid, wpb * 32, 0, s>>>(p);
+    if (p.has_next) scan2d_kernel<true><<<grid, 256, 0, s>>>(p);
+    else scan2d_kernel<false><<<grid, 256, 0, s>>>(p);
   } else {
-    const unsigned grid = (unsigned)((i64)p.nsx * p.nsy * p.nsz);
     const dim3 block(32, SCAN3_BY);
     if (p.has_next) scan3d_kernel<true><<<grid, block, 0, s>>>(p);
     else scan3d_kernel<false><<<grid, block, 0, s>>>(p);
@@ -3746,25 +2861,6 @@ void launch_test(const SweepParams &p, cudaStream_t s) {
   else test_kernel<3><<<grid, 128, 0, s>>>(p);
 }
 
-// Kernels of one step that ask for different shared-memory / L1 splits cannot share an SM, and an SM has to drain before its
-// split changes: the scan kernels take most of the 228 KB as shared memory, so every kernel of the step loop asks for the same
-// split -- then the test kernel's few blocks slot in next to the next scan's CTAs.  Opt-in (FTKB_CARVEOUT=1): it costs the scans L1.
-static void init_carveouts() {
-  const char *e = std::getenv("FTKB_CARVEOUT");      // off by default: measured 174 us (driver's split) against 183 us on the C2 scan
-  if (!e || std::string(e) != "1") return;
-  const int co = cudaSharedmemCarveoutMaxShared;
-#define CARVE(k) cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, co)
-  CARVE(test_kernel<2>); CARVE(test_kernel<3>);
-  CARVE((scan2d_keys_build_kernel<0, false, 3, 4>)); CARVE((scan2d_keys_build_kernel<0, true, 3, 4>)); CARVE((scan2d_keys_build_kernel<1, true, 3, 4>));
-  CARVE((scan2d_build_kernel<0, false>)); CARVE((scan2d_build_kernel<0, true>)); CARVE((scan2d_build_kernel<1, true>));
-  CARVE((scan3d_build_kernel<0, false>)); CARVE((scan3d_build_kernel<0, true>)); CARVE((scan3d_build_kernel<1, true>));
-  CARVE((vscan2d_build_kernel<0, false>)); CARVE((vscan2d_build_kernel<0, true>)); CARVE((vscan2d_build_kernel<1, true>));
-  CARVE((vscan3d_build_kernel<0, false>)); CARVE((vscan3d_build_kernel<0, true>)); CARVE((vscan3d_build_kernel<1, true>));
-  CARVE(scan2d_cells_kernel<1>); CARVE(scan2d_cells_kernel<2>); CARVE(scan3d_cells_kernel<1>); CARVE(scan3d_cells_kernel<2>);
-  CARVE(vscan2d_cells_kernel<1>); CARVE(vscan2d_cells_kernel<2>);
-#undef CARVE
-  cudaGetLastError();
-}
 
 // =============================================================================================
 // 5. field derivation + resolution

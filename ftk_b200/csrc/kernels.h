@@ -41,9 +41,7 @@ struct SweepParams {
   const double *coords;       // device: rectilinear x[W] y[H] [z[D]], or explicit (ncomp, W, H)
   // fused mode: the vector field is derived from the scalar layers on the fly (L[].V == nullptr)
   int32_t fused;
-  int32_t aligned16;          // rows of S start 16-byte aligned (W even, base aligned): vector loads allowed
   int32_t keys2d;             // 2D scalar build: high-word keys of the differences instead of fp32 ranges (scan2d_keys_build_kernel)
-  int32_t bulk;               // row staging with cp.async.bulk + mbarrier (needs aligned16): 2 = CTA-wide ring + producer warp, 1 = per-warp rings, 0 = registers
   float thrp_f;               // 2^-nbits (1 + 2^-20): approx(v) >= thrp_f  =>  |quantised v| >= 1
   float thr2_f;               // 2^(1-nbits)
   float lim_f;                // 0.999 * 4.5e18 / factor^2 (determinant magnitude bound, field units)
@@ -53,7 +51,6 @@ struct SweepParams {
   // What the slot then receives is the minimum over the values under the threshold -- equal to the layer's own minimum whenever
   // that one would lower the running minimum, which is all the tracker uses it for.
   float res_thr[3];
-  int32_t l2_hint;                   // 2D key kernel: layer rows are copied with an L2 evict-first policy (FTKB_K2_L2HINT=1; measured alternative)
   unsigned long long *poison;        // fused 3D scan: set non-zero when a scalar is NaN / Inf / >= 2^1000 (the sweep is redone unfused)
   // fused 3D scan: TMA descriptors of the two scalar layers (box = one tile plane incl. halo)
   alignas(64) CUtensorMap tmap[2];
@@ -104,7 +101,6 @@ void init_kernel_attributes();   // opt-in shared memory sizes; once per device
 // fused 3D scan geometry (host needs it for the grid decomposition and the TMA box)
 constexpr int F3_CW = 8;                       // consumer warps per CTA
 constexpr int F3_RW = 4;                       // corner rows per consumer warp
-constexpr int F3_NST = 5;                      // ring stages (scalar planes)
 constexpr int F3_STRIDE = 62;                  // corner columns per tile
 constexpr int F3_COLS = 68;                    // staged columns: C0-2 .. C0+65
 constexpr int F3_TROWS = F3_CW * F3_RW;        // corner rows per tile
@@ -123,7 +119,7 @@ enum { SUM_BUILD = 0,          // stream layer build_layer, write its cells (+ m
 void launch_scan3d_cells(const SweepParams &p, cudaStream_t s);
 size_t scan3d_cells_per_layer(const SweepParams &p);
 constexpr int SCAN2D_CELL_ROWS = 9;
-void launch_scan2d_cells(const SweepParams &p, cudaStream_t s);     // needs p.bulk == 2 geometry with p.rows a multiple of SCAN2D_CELL_ROWS
+void launch_scan2d_cells(const SweepParams &p, cudaStream_t s);     // needs 16-byte aligned rows, the CTA tiling of 7 strips and p.rows a multiple of SCAN2D_CELL_ROWS
 size_t scan2d_cells_per_layer(const SweepParams &p);
 // vector input (field GIVEN): p.fused == 0, p.L[].V set; 2D needs p.nsx = strips of 62 columns and p.rows a multiple of 8,
 // 3D the tile / chunk geometry of the fused 3D scan and W even

@@ -161,17 +161,18 @@ def test_fused_3d_scan_equals_unfused(ftk, monkeypatch):
     b.close()
 
 
-@pytest.mark.parametrize("dims,T,env,field", [([200, 150], 4, "FTKB_SCAN2D", "scalar"), ([130, 70, 44], 3, "FTKB_SCAN3D", "scalar"),
-                                              ([200, 150], 4, "FTKB_VSCAN", "vector"), ([66, 70, 24], 3, "FTKB_VSCAN", "vector"),
-                                              ([131, 37], 3, "FTKB_VSCAN", "vector")])
-def test_range_cell_scan_equals_two_layer_scan(dims, T, env, field, ftk, oracle, monkeypatch):
-    """default scan (each layer streamed once, 16-byte range cells kept per layer) against the scan that re-reads both
-    layers every step (FTKB_SCAN2D/3D=twolayer) and against the oracle: same points, same trajectories, same factor;
-    every punctured simplex's cube is in the cell scan's worklist; a repeated sweep (cells only) changes nothing"""
+@pytest.mark.parametrize("dims,T,env,value,field", [([200, 150], 4, "FTKB_SCAN2D", "f32", "scalar"), ([130, 70, 44], 3, "FTKB_SCAN3D", "plain", "scalar"),
+                                                    ([200, 150], 4, "FTKB_VSCAN", "twolayer", "vector"), ([66, 70, 24], 3, "FTKB_VSCAN", "twolayer", "vector"),
+                                                    ([131, 37], 3, "FTKB_VSCAN", "twolayer", "vector")])
+def test_range_cell_scan_equals_fallback_scan(dims, T, env, value, field, ftk, oracle, monkeypatch):
+    """default scan (each layer streamed once, 16-byte range cells kept per layer) against the fallback the same input takes
+    when the default cannot run (FTKB_SCAN2D=f32: fp32-range build kernel; FTKB_SCAN3D=plain: materialised gradient;
+    FTKB_VSCAN=twolayer: vector scan that re-reads both layers) and against the oracle: same points, same trajectories, same
+    factor; every punctured simplex's cube is in the cell scan's worklist; a repeated sweep (cells only) changes nothing"""
     rng = np.random.default_rng(4242 + len(dims))
     snaps = _rand_series(rng, dims, T, 1 if field == "scalar" else len(dims), "smooth")
     a = ftk.track(snaps, dims, field=field)
-    monkeypatch.setenv(env, "twolayer")
+    monkeypatch.setenv(env, value)
     b = ftk.track(snaps, dims, field=field)
     monkeypatch.delenv(env)
     pa, pb = a.get_discrete_critical_points(), b.get_discrete_critical_points()
@@ -203,18 +204,16 @@ def test_range_cell_scan_equals_two_layer_scan(dims, T, env, field, ftk, oracle,
     tr.close()
 
 
-def test_direct_staging_of_the_2d_cell_scan(ftk, oracle, monkeypatch):
-    """FTKB_SCAN=direct: the 2D range-cell scan without shared memory (16-byte loads, shuffles, key ranges) -- kept as a
-    measured alternative to the bulk-async tile scan; same results as the oracle on a ragged, several-strip field"""
-    monkeypatch.setenv("FTKB_SCAN", "direct")
+def test_2d_cell_scan_on_ragged_fields(ftk, oracle):
+    """the 2D range-cell scan (16-byte aligned rows) on ragged fields over several CTA tiles, strips and row chunks: same
+    results, scaling factor and resolution as the oracle"""
     rng = np.random.default_rng(9090)
     for dims, T in (([200, 150], 4), ([64, 35], 3), ([130, 17], 3)):
         snaps = _rand_series(rng, dims, T, 1, "smooth")
         c, o = _both(ftk, oracle, snaps, dims, "scalar")
-        P.assert_same_result(cuda_result(c), P.oracle_result(o), tol=TOL, what=f"direct staging {dims}")
+        P.assert_same_result(cuda_result(c), P.oracle_result(o), tol=TOL, what=f"2D cell scan {dims}")
         assert c.stats()["scaling_factor"] == o.scaling_factor and c.stats()["resolution"] == o.resolution
         c.close()
-    monkeypatch.delenv("FTKB_SCAN")
 
 
 def test_given_jacobian_and_scalar(ftk, oracle):
