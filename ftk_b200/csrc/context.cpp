@@ -646,12 +646,12 @@ static int nbits_of(double resolution) {
 }
 
 // set_coords_bounds / set_coords_rectilinear / set_coords_explicit (regular_tracker.hh:38-40): the coordinates the
-// per-simplex test interpolates (simplex_coordinates, critical_point_tracker_2d_regular.hh:494-526, ..._3d_regular.hh:343-379)
+// per-simplex test interpolates (simplex_coordinates, critical_point_tracker_2d_regular.hh:494-526, ..._3d_regular.hh:343-379).
+// A z-slab takes the whole array's coordinates (its rectilinear z array has slab_global_dim values).
 extern "C" int ftkb_set_coords(ftkb_ctx *c, int mode, const double *data, uint64_t n) {
   if (!c || mode < FTKB_COORDS_SIMPLE || mode > FTKB_COORDS_EXPLICIT || (mode != FTKB_COORDS_SIMPLE && !data)) return FTKB_ERR_INVALID;
-  if (c->slab && mode != FTKB_COORDS_SIMPLE) return fail(c, FTKB_ERR_INVALID, "set_coords: physical coordinates are not available on a spatial slab");
   CK(cudaSetDevice(c->cfg.device));
-  const uint64_t W = c->cfg.dims[0], H = c->cfg.dims[1], D = c->n == 3 ? c->cfg.dims[2] : 0;
+  const uint64_t W = c->cfg.dims[0], H = c->cfg.dims[1], D = c->n == 3 ? (c->slab ? c->cfg.slab_global_dim : c->cfg.dims[2]) : 0;
   if (mode == FTKB_COORDS_BOUNDS && n != 2u * c->n) return fail(c, FTKB_ERR_INVALID, "set_coords: bounds take 2 * nd values");
   if (mode == FTKB_COORDS_RECTILINEAR && n != W + H + D) return fail(c, FTKB_ERR_INVALID, "set_coords: rectilinear coordinates take W + H [+ D] values");
   if (mode == FTKB_COORDS_EXPLICIT && (n % (W * H) != 0 || n / (W * H) < (c->n == 3 ? 3u : 2u)))
@@ -679,6 +679,7 @@ static void fill_sweep_geometry(const ftkb_ctx *c, SweepParams &p) {
   p.nd = c->n;
   p.sm_count = c->sm_count;
   p.W = c->cfg.dims[0]; p.H = c->cfg.dims[1]; p.D = c->n == 3 ? c->cfg.dims[2] : 1;
+  p.coords_D = c->slab ? c->cfg.slab_global_dim : p.D;
   for (int j = 0; j < 3; j++) {
     const bool used = j < c->n;
     p.lb[j] = used ? c->cfg.lb[j] : 0;
@@ -893,8 +894,9 @@ static int wait_grow(ftkb_ctx *c) {
   return c->grow_failed ? FTKB_ERR_NOMEM : FTKB_OK;
 }
 
-static int grow_trajectories(ftkb_ctx *c) {
-  const uint64_t n = c->npts - c->grown;
+// one grow step over d_pts[grown .. end)
+static int grow_trajectories(ftkb_ctx *c, uint64_t end) {
+  const uint64_t n = end - c->grown;
   if (n >= 0xffffffffull) return fail(c, FTKB_ERR_OVERFLOW, "more than 2^32 punctured simplices in one step");
   { const int rc = wait_grow(c); if (rc) return rc; }
   // The device prepares the batch: element keys -> radix sort -> unique -> for every element the batch indices of its punctured
@@ -956,9 +958,17 @@ static int grow_trajectories(ftkb_ctx *c) {
   }
   catch (const std::bad_alloc &) { c->grow_failed = true; return fail(c, FTKB_ERR_NOMEM, "streaming grow step: out of memory (trajectories are incomplete)"); }
   catch (const std::exception &e) { c->grow_failed = true; return fail(c, FTKB_ERR_INVALID, std::string("streaming grow step: ") + e.what()); }
-  c->grown = c->npts;
+  c->grown = end;
   c->traced = false;
   return FTKB_OK;
+}
+
+// a streaming context that sweeps nothing itself (the merged context of a device group, include/ftkb200.h): one grow step over
+// the imported points that follow those grown so far, up to index `end` of the import order
+int ftkb::grow_imported(ftkb_ctx *c, uint64_t end) {
+  if (!c || !c->streaming || end < c->grown || end > c->npts) return FTKB_ERR_INVALID;
+  CK(cudaSetDevice(c->cfg.device));
+  return grow_trajectories(c, end);
 }
 
 extern "C" int ftkb_set_streaming_trajectories(ftkb_ctx *c, int enable) {
@@ -1474,7 +1484,7 @@ static int update_impl(ftkb_ctx *c, bool allow_defer) {
     if (npt != c->npts) { c->sorted = false; c->traced = false; }
     c->npts = npt;
     c->stats.points = npt;
-    if (c->streaming && has_next) { const int rc2 = grow_trajectories(c); if (rc2) return rc2; }
+    if (c->streaming && has_next) { const int rc2 = grow_trajectories(c, c->npts); if (rc2) return rc2; }
     return FTKB_OK;
   }
   return fail(c, FTKB_ERR_CUDA, "update_timestep: buffers kept overflowing");
@@ -1634,7 +1644,10 @@ extern "C" int ftkb_get_points(ftkb_ctx *c, ftkb_point *out, uint64_t cap) {
 
 extern "C" int ftkb_import_points(ftkb_ctx *c, const ftkb_point *pts, uint64_t n) {
   if (!c || (!pts && n)) return FTKB_ERR_INVALID;
-  if (c->streaming) return fail(c, FTKB_ERR_INVALID, "import_points: not available with streaming trajectories");
+  // a streaming context grows its trajectories from its own sweeps; one that holds no snapshot and has swept nothing takes
+  // imports instead, and grows them step by step with ftkb::grow_imported
+  if (c->streaming && (c->stats.scan_launches || !c->layers.empty()))
+    return fail(c, FTKB_ERR_INVALID, "import_points: not available on a streaming context that sweeps");
   if (!n) return FTKB_OK;
   CK(cudaSetDevice(c->cfg.device));
   { const int rc = drain(c); if (rc) return rc; }

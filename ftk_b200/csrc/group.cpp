@@ -17,6 +17,12 @@
 //   merge         ftkb_group_finalize collects the (sparse) punctured simplices of every chunk into one context on the first
 //                 device and runs the union-find + ordering there: components that cross chunk boundaries are united by
 //                 the same neighbour search that unites them inside a chunk.
+//   streaming     chunks and slabs sweep offline; the merged context then runs the reference's grow step once per swept
+//                 interval t, in time order, over its sorted points of timestep t -- the batch a single streaming context
+//                 grows at t (ordinal sweep at t + interval sweep [t, t+1]).  The last ordinal sweep's points join no
+//                 trajectory, as on one device.
+//   coordinates   physical coordinates (ftkb_group_set_coords) are kept here and handed to every chunk context as it is
+//                 created and to every slab context at once; a slab looks them up in the whole array's frame.
 #include <algorithm>
 #include <atomic>
 #include <cfloat>
@@ -34,6 +40,7 @@
 #include <cuda_runtime.h>
 
 #include "../../include/ftkb200.h"
+#include "online.h"
 
 namespace {
 
@@ -124,6 +131,10 @@ struct ftkb_group {
   std::condition_variable cv;
   double saturating = 0.0;                         // a running minimum known to saturate the factor (0: not known yet)
   int npushed = 0, nadvanced = 0;
+  int nintervals = 0;                              // intervals [t, t+1] swept so far, from start_timestep on
+  bool streaming = false;                          // grow trajectories on the merged context (ftkb_group_set_streaming_trajectories)
+  int coords_mode = FTKB_COORDS_SIMPLE;            // ftkb_group_set_coords, handed to every chunk context
+  std::vector<double> coords;
   std::atomic<int> failed{FTKB_OK};
   std::string error;
   ftkb_ctx *root = nullptr;
@@ -159,8 +170,10 @@ struct ftkb_group {
     c.device = ch->device;
     c.start_timestep = cfg.start_timestep + ch->index * B;
     c.resolution_init = res_init;
-    const int rc = ftkb_create(&c, &ch->ctx);
-    if (rc) fail(rc, std::string("chunk context: ") + ftkb_last_error(nullptr));
+    int rc = ftkb_create(&c, &ch->ctx);
+    if (rc) { fail(rc, std::string("chunk context: ") + ftkb_last_error(nullptr)); return rc; }
+    if (coords_mode != FTKB_COORDS_SIMPLE && (rc = ftkb_set_coords(ch->ctx, coords_mode, coords.data(), coords.size())))
+      fail(rc, std::string("chunk context: ") + ftkb_last_error(ch->ctx));
     return rc;
   }
   // after a sweep of a chunk: publish a saturating minimum as soon as one is known (lets the next chunk start early)
@@ -298,6 +311,29 @@ static int spatial_push(ftkb_group *g, std::function<int(Slab &)> push) {
   return rc;
 }
 
+// ---- options: set before the first push ---------------------------------------------------------------------------------------
+extern "C" int ftkb_group_set_coords(ftkb_group *g, int mode, const double *data, uint64_t n) {
+  if (!g) return FTKB_ERR_INVALID;
+  if (g->npushed) { g->error = "set_coords: call it before the first push"; return FTKB_ERR_INVALID; }
+  // the sizes of ftkb_set_coords, in the whole array's frame (a chunk context checks them again when it is created)
+  const uint64_t W = g->cfg.dims[0], H = g->cfg.dims[1], D = g->cfg.nd == 3 ? g->cfg.dims[2] : 0, nd = g->cfg.nd;
+  const bool ok = mode == FTKB_COORDS_SIMPLE ||
+                  (data && ((mode == FTKB_COORDS_BOUNDS && n == 2 * nd) || (mode == FTKB_COORDS_RECTILINEAR && n == W + H + D) ||
+                            (mode == FTKB_COORDS_EXPLICIT && n % (W * H) == 0 && n / (W * H) >= nd)));
+  if (!ok) { g->error = "set_coords: unknown mode, or a size that does not fit the array"; return FTKB_ERR_INVALID; }
+  g->coords_mode = mode;
+  g->coords.assign(data, data + (mode == FTKB_COORDS_SIMPLE ? 0 : n));
+  if (!g->spatial) return FTKB_OK;
+  return on_all_slabs(g, [g](Slab &sl) { return ftkb_set_coords(sl.ctx, g->coords_mode, g->coords.data(), g->coords.size()); }, "set_coords");
+}
+
+extern "C" int ftkb_group_set_streaming_trajectories(ftkb_group *g, int enable) {
+  if (!g) return FTKB_ERR_INVALID;
+  if (g->npushed) { g->error = "set_streaming_trajectories: call it before the first push"; return FTKB_ERR_INVALID; }
+  g->streaming = enable != 0;
+  return FTKB_OK;
+}
+
 // hand one snapshot to chunk c's context (runs on that device's worker)
 static void post_push(ftkb_group *g, int c, std::function<int(ftkb_ctx *)> push, std::shared_ptr<Done> done) {
   Chunk *ch = g->chunk(c);
@@ -413,6 +449,7 @@ static int post_sweep(ftkb_group *g, int step, bool advance) {
 extern "C" int ftkb_group_advance_timestep(ftkb_group *g) {
   if (!g) return FTKB_ERR_INVALID;
   if (g->npushed < g->nadvanced + 2) { g->error = "advance_timestep: two snapshots are needed"; return FTKB_ERR_INVALID; }
+  g->nintervals = std::max(g->nintervals, g->nadvanced + 1);
   if (g->spatial) { g->nadvanced++; return on_all_slabs(g, [](Slab &sl) { return ftkb_advance_timestep(sl.ctx); }, "sweep"); }
   return post_sweep(g, g->nadvanced++, true);
 }
@@ -420,8 +457,39 @@ extern "C" int ftkb_group_advance_timestep(ftkb_group *g) {
 extern "C" int ftkb_group_update_timestep(ftkb_group *g) {
   if (!g) return FTKB_ERR_INVALID;
   if (g->npushed < g->nadvanced + 1) { g->error = "update_timestep: no snapshot has been pushed"; return FTKB_ERR_INVALID; }
+  if (g->npushed >= g->nadvanced + 2) g->nintervals = std::max(g->nintervals, g->nadvanced + 1);     // the next snapshot is there
   if (g->spatial) return on_all_slabs(g, [](Slab &sl) { return ftkb_update_timestep(sl.ctx); }, "sweep");
   return post_sweep(g, g->nadvanced, false);
+}
+
+// The merged context on the first device: the punctured simplices of every chunk or slab, sorted and deduplicated there, then
+// traced offline -- or, with streaming trajectories, grown once per swept interval t, in time order, over the points of
+// timestep t.  The points of the last ordinal sweep are imported but never grown.
+static int build_root(ftkb_group *g, const std::vector<const std::vector<ftkb_point> *> &parts) {
+  if (g->root) { ftkb_destroy(g->root); g->root = nullptr; }
+  ftkb_config c = g->cfg;
+  c.device = g->devices[0];
+  int rc = ftkb_create(&c, &g->root);
+  if (rc) { g->error = ftkb_last_error(nullptr); return rc; }
+  if (g->streaming) {
+    std::vector<ftkb_point> all;
+    for (auto *p : parts) all.insert(all.end(), p->begin(), p->end());
+    std::stable_sort(all.begin(), all.end(), [](const ftkb_point &a, const ftkb_point &b) { return a.timestep < b.timestep; });
+    rc = ftkb_set_streaming_trajectories(g->root, 1);
+    if (!rc) rc = ftkb_import_points(g->root, all.data(), all.size());
+    for (int k = 0; !rc && k < g->nintervals; k++) {
+      const int t = g->cfg.start_timestep + k;
+      const auto end = std::upper_bound(all.begin(), all.end(), t, [](int s, const ftkb_point &p) { return s < p.timestep; });
+      rc = ftkb::grow_imported(g->root, (uint64_t)(end - all.begin()));
+    }
+  } else {
+    // (the flat simplices of a cut plane were found by both neighbouring slabs: the root's sort drops the duplicates)
+    for (auto *p : parts)
+      if (!rc && !p->empty()) rc = ftkb_import_points(g->root, p->data(), p->size());
+  }
+  if (!rc) rc = ftkb_finalize(g->root);
+  if (rc) g->error = ftkb_last_error(g->root);
+  return rc;
 }
 
 extern "C" int ftkb_group_finalize(ftkb_group *g, ftkb_ctx **root) {
@@ -436,14 +504,9 @@ extern "C" int ftkb_group_finalize(ftkb_group *g, ftkb_ctx **root) {
       return r;
     }, "collect");
     if (rc) return rc;
-    if (g->root) { ftkb_destroy(g->root); g->root = nullptr; }
-    ftkb_config c = g->cfg;
-    c.device = g->devices[0];
-    if ((rc = ftkb_create(&c, &g->root))) { g->error = ftkb_last_error(nullptr); return rc; }
-    // (the flat simplices of a cut plane were found by both neighbours: the root's sort drops the duplicates)
-    for (auto &sl : g->slabs)
-      if (!sl.points.empty() && (rc = ftkb_import_points(g->root, sl.points.data(), sl.points.size()))) { g->error = ftkb_last_error(g->root); return rc; }
-    if ((rc = ftkb_finalize(g->root))) { g->error = ftkb_last_error(g->root); return rc; }
+    std::vector<const std::vector<ftkb_point> *> parts;
+    for (auto &sl : g->slabs) parts.push_back(&sl.points);
+    if ((rc = build_root(g, parts))) return rc;
     *root = g->root;
     return FTKB_OK;
   }
@@ -460,14 +523,10 @@ extern "C" int ftkb_group_finalize(ftkb_group *g, ftkb_ctx **root) {
   for (auto &ch : g->chunks)
     if (ch->ctx && !ch->finished) g->finish_chunk(ch.get());
   if (g->failed.load()) return g->failed.load();
-  if (g->root) { ftkb_destroy(g->root); g->root = nullptr; }
-  ftkb_config c = g->cfg;
-  c.device = g->devices[0];
-  int rc = ftkb_create(&c, &g->root);
-  if (rc) { g->error = ftkb_last_error(nullptr); return rc; }
-  for (auto &ch : g->chunks)
-    if (!ch->points.empty() && (rc = ftkb_import_points(g->root, ch->points.data(), ch->points.size()))) { g->error = ftkb_last_error(g->root); return rc; }
-  if ((rc = ftkb_finalize(g->root))) { g->error = ftkb_last_error(g->root); return rc; }
+  std::vector<const std::vector<ftkb_point> *> parts;
+  for (auto &ch : g->chunks) parts.push_back(&ch->points);
+  const int rc = build_root(g, parts);
+  if (rc) return rc;
   *root = g->root;
   return FTKB_OK;
 }

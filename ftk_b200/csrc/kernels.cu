@@ -2464,19 +2464,21 @@ __device__ void jacobian3d_at(const SweepParams &p, const LayerPtrs &L, int i, i
 // physical coordinates of one vertex v = (x, y[, z], t) -> X = (x, y, z, t)
 // (ref: critical_point_tracker_2d_regular.hh:494-526, critical_point_tracker_3d_regular.hh:343-379; the array domain starts at 0).
 // The 3D explicit mode is the reference's as it stands: looked up by (x, y) only, and the time slot receives z.
+// A z-slab looks its vertices up in the whole array's frame: z + voff[2], of coords_D planes.
 template <int ND>
 __device__ __forceinline__ void simplex_coordinates(const SweepParams &p, const int *v, double X[4]) {
-  const int dims[3] = {p.W, p.H, p.D};
+  const int dims[3] = {p.W, p.H, p.coords_D};
+  const int g[3] = {v[0], v[1], ND == 3 ? v[2] + p.voff[2] : v[2]};      // (2D: g[2] is the time)
   if (p.coords_mode == 1) {
 #pragma unroll
     for (int j = 0; j < ND; j++)
-      X[j] = ((double)v[j] / (double)(dims[j] - 1)) * (p.coords_bounds[2 * j + 1] - p.coords_bounds[2 * j]) + p.coords_bounds[2 * j];
+      X[j] = ((double)g[j] / (double)(dims[j] - 1)) * (p.coords_bounds[2 * j + 1] - p.coords_bounds[2 * j]) + p.coords_bounds[2 * j];
     if (ND == 2) X[2] = 0.0;
     X[3] = (double)v[ND];
   } else if (p.coords_mode == 2) {
     int off = 0;
 #pragma unroll
-    for (int j = 0; j < ND; j++) { X[j] = __ldg(p.coords + off + v[j]); off += dims[j]; }
+    for (int j = 0; j < ND; j++) { X[j] = __ldg(p.coords + off + g[j]); off += dims[j]; }
     if (ND == 2) X[2] = 0.0;
     X[3] = (double)v[ND];
   } else {
@@ -2485,7 +2487,7 @@ __device__ __forceinline__ void simplex_coordinates(const SweepParams &p, const 
     X[1] = __ldg(p.coords + 1 + nc * k);
     if (ND == 2) X[2] = nc > 2 ? __ldg(p.coords + 2 + nc * k) : 0.0;
     else X[2] = __ldg(p.coords + 2 + nc * k);
-    X[3] = (double)v[2];
+    X[3] = (double)g[2];
   }
 }
 

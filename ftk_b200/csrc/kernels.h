@@ -37,8 +37,9 @@ struct SweepParams {
   LayerPtrs L[2];
   // physical coordinates of the vertices (regular_tracker.hh:12-17,38-40): 0 grid units, 1 bounds, 2 rectilinear, 3 explicit
   int32_t coords_mode, coords_ncomp;
+  int32_t coords_D;           // planes of the array the coordinates describe: the whole array's D on a z-slab, else D
   double coords_bounds[6];
-  const double *coords;       // device: rectilinear x[W] y[H] [z[D]], or explicit (ncomp, W, H)
+  const double *coords;       // device: rectilinear x[W] y[H] [z[coords_D]], or explicit (ncomp, W, H)
   // fused mode: the vector field is derived from the scalar layers on the fly (L[].V == nullptr)
   int32_t fused;
   int32_t keys2d;             // 2D scalar build: high-word keys of the differences instead of fp32 ranges (scan2d_keys_build_kernel)

@@ -66,4 +66,8 @@ class OnlineTracer {
   bool have_points_ = true;
 };
 
+// (context.cpp) one grow step of a streaming context over its imported points [grown so far, end): how a device group's merged
+// context replays the grow steps of the chunks or slabs that swept for it (group.cpp)
+int grow_imported(ftkb_ctx *c, uint64_t end);
+
 }  // namespace ftkb

@@ -2,15 +2,17 @@
 
 The reference hands a device list to every filter (filter.hh:47-51 set_device_ids); here one process drives the devices
 through time chunks (chunk c = `chunk` consecutive timesteps, swept by a context of its own on device_ids[c mod N], one host
-thread per device).  Results equal the one-device tracker bit for bit; ftkb_group_finalize merges everything into one
-context, which this class then exposes through the ordinary tracker getters.
+thread per device), or, with chunk=0 (3D), through z-slabs that every device sweeps at every step.  Results equal the
+one-device tracker bit for bit; ftkb_group_finalize merges everything into one context, which this class then exposes through
+the ordinary tracker getters.  streaming=True grows trajectories there as a single streaming tracker does; coords=(mode, data)
+takes make_tracker's forms, for the whole array.
 """
 import ctypes as C
 
 import numpy as np
 
 from . import _lib as L
-from .tracker import make_tracker, _RegularTracker, SOURCE_DERIVED, SOURCE_GIVEN, SOURCE_NONE
+from .tracker import coords_arg, make_tracker, _RegularTracker, SOURCE_DERIVED, SOURCE_GIVEN, SOURCE_NONE
 
 
 class _GroupRoot(_RegularTracker):
@@ -26,7 +28,7 @@ class _GroupRoot(_RegularTracker):
 
 class GroupTracker:
     def __init__(self, dims, device_ids, field="scalar", chunk=8, lb=None, ub=None, jacobian_symmetric=None, robust=True,
-                 compute_degrees=False, type_filter=None, start_timestep=0):
+                 compute_degrees=False, type_filter=None, start_timestep=0, streaming=False, coords=None):
         nd = len(dims)
         if field == "scalar":
             ss, vs, js, sym, margin = SOURCE_GIVEN, SOURCE_DERIVED, SOURCE_DERIVED, True, 2
@@ -56,6 +58,11 @@ class GroupTracker:
         self._g = g
         self._dims, self._field, self._nd = list(dims), field, nd
         self._root = None
+        if streaming:
+            self._check(L.lib().ftkb_group_set_streaming_trajectories(g, 1))
+        if coords is not None:      # copied by the library before the call returns
+            mode, data = coords_arg(coords)
+            self._check(L.lib().ftkb_group_set_coords(g, mode, data.ctypes.data, data.size))
 
     def _check(self, rc):
         if rc:

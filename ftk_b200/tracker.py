@@ -468,11 +468,16 @@ def make_tracker(dims, field="scalar", lb=None, ub=None, jacobian_symmetric=None
     tr.set_initial_resolution(resolution_init)
     tr.set_enable_streaming_trajectories(streaming)
     tr._point_capacity = int(point_capacity)      # initial size of the punctured-simplex buffer (grows on demand)
-    if coords is not None:      # ("bounds" | "rectilinear" | "explicit", flat data in the reference's order)
-        tr._coords = ({"bounds": L.COORDS_BOUNDS, "rectilinear": L.COORDS_RECTILINEAR, "explicit": L.COORDS_EXPLICIT}[coords[0]],
-                      np.ascontiguousarray(coords[1], np.float64).ravel())
+    if coords is not None:
+        tr._coords = coords_arg(coords)
     tr.initialize()
     return tr
+
+
+def coords_arg(coords):
+    """("bounds" | "rectilinear" | "explicit", flat data in the reference's order) -> (COORDS_* mode, float64 array)"""
+    return ({"bounds": L.COORDS_BOUNDS, "rectilinear": L.COORDS_RECTILINEAR, "explicit": L.COORDS_EXPLICIT}[coords[0]],
+            np.ascontiguousarray(coords[1], np.float64).ravel())
 
 
 def track(snapshots, dims, field="scalar", trace=True, **kw):

@@ -378,11 +378,11 @@ class critical_point_tracker_regular {
     cfg.use_type_filter = use_type_filter_; cfg.type_filter = type_filter_;
     cfg.start_timestep = start_timestep_; cfg.device = device_; cfg.resolution_init = resolution_init_;
     if (device_ids_.size() > 1) {
-      if (streaming_) throw std::runtime_error("ftk_b200: streaming trajectories are not available on several devices");
-      if (coords_mode_ != FTKB_COORDS_SIMPLE) throw std::runtime_error("ftk_b200: physical coordinates are not available on several devices yet");
       std::vector<int32_t> ids(device_ids_.begin(), device_ids_.end());
       const int rcg = ftkb_group_create(&cfg, ids.data(), (int32_t)ids.size(), time_chunk_, &group_);
       if (rcg != FTKB_OK) throw std::runtime_error("ftkb_group_create failed (device ids?)");
+      if (streaming_) gcheck(ftkb_group_set_streaming_trajectories(group_, 1));
+      if (coords_mode_ != FTKB_COORDS_SIMPLE) gcheck(ftkb_group_set_coords(group_, coords_mode_, coords_.data(), coords_.size()));
       return;
     }
     const int rc = ftkb_create(&cfg, &ctx_);

@@ -185,7 +185,8 @@ int ftkb_set_resolution(ftkb_ctx *, double res);   /* lower the running minimum 
  * simplicial_regular_mesh.hh:327-337), duplicates removed */
 int ftkb_num_points(ftkb_ctx *, uint64_t *n);
 int ftkb_get_points(ftkb_ctx *, ftkb_point *out, uint64_t cap);
-/* add punctured simplices found elsewhere (another time slab) before ftkb_finalize */
+/* add punctured simplices found elsewhere (another time slab) before ftkb_finalize.  A streaming context (ftkb_set_streaming_trajectories)
+ * takes imports only while it holds no snapshot and has swept nothing (the merged context of a group) */
 int ftkb_import_points(ftkb_ctx *, const ftkb_point *pts, uint64_t n);
 
 /* ---- time-slab halo through NVLink peer memory (SURVEY.md 8e) -------------------------------------------------
@@ -218,20 +219,32 @@ int ftkb_push_snapshot_remote(ftkb_ctx *, const double *scalar, const double *ve
  * starts early once the minimum known so far saturates the factor, otherwise when the predecessor has finished -- results equal
  * the one-device run bit for bit.  ftkb_group_finalize merges the punctured simplices of all chunks into one context on
  * device_ids[0] and traces there; *root stays owned by the group and serves every getter (ftkb_get_points, ftkb_get_trajectories,
- * ftkb_get_curveset ...).  cfg->device is ignored; streaming trajectories are not available on a group.
+ * ftkb_get_trajectory_complete, ftkb_get_curveset ...).  cfg->device is ignored.
  * ftkb_group_push_snapshot takes HOST memory (borrowed until return); ftkb_group_push_synthetic generates on the devices.
+ *
+ * Options, valid only before the first push (afterwards FTKB_ERR_INVALID):
+ *   ftkb_group_set_coords                   ftkb_set_coords for the whole array: same modes and sizes, host data copied before
+ *                                           the call returns; every chunk / slab context sweeps with it.
+ *   ftkb_group_set_streaming_trajectories   chunks and slabs still sweep offline; ftkb_group_finalize then runs the grow step
+ *                                           of ftkb_set_streaming_trajectories on the merged context once per swept interval t,
+ *                                           in time order, over its sorted points of timestep t -- the batch a single streaming
+ *                                           context grows at t -- and publishes trajectories, loop and complete flags as a
+ *                                           streaming context's ftkb_finalize does.
  *
  * chunk_timesteps = 0 selects the SPATIAL decomposition instead (3D only; the reference's own, regular_tracker.hh:126-149):
  * device s holds a z-slab of every snapshot -- its share of the domain's corner planes, the corner plane above (whose flat
  * simplices both neighbours find; the merge drops the duplicates) and two ghost planes beyond every vertex it uses -- and every
  * device sweeps every step, so a host snapshot travels in N pieces over N PCIe links at once.  SoS vertex ranks, interpolated
- * positions, reported corners and the device generators use the whole array's frame (ftkb_config.slab_*); until the running
+ * positions, physical coordinates, reported corners and the device generators use the whole array's frame (ftkb_config.slab_*;
+ * ftkb_set_coords on a slab context takes the whole array's coordinates); until the running
  * minimum of min non-zero |v| saturates the quantisation factor, the slabs' minima are combined before every sweep, so every
  * slab quantises exactly as the undivided run does. */
 typedef struct ftkb_group ftkb_group;
 int ftkb_group_create(const ftkb_config *cfg, const int32_t *device_ids, int32_t n_devices, int32_t chunk_timesteps, ftkb_group **out);
 void ftkb_group_destroy(ftkb_group *);
 const char *ftkb_group_last_error(const ftkb_group *);
+int ftkb_group_set_coords(ftkb_group *, int mode, const double *data, uint64_t n);
+int ftkb_group_set_streaming_trajectories(ftkb_group *, int enable);
 int ftkb_group_push_snapshot(ftkb_group *, const double *scalar, const double *vector, const double *jacobian);
 int ftkb_group_push_synthetic(ftkb_group *, int kind, const double *params, int nparams, double t);
 int ftkb_group_advance_timestep(ftkb_group *);
