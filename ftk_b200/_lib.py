@@ -80,6 +80,7 @@ EXPORTS = [
     "ftkb_online_size", "ftkb_online_get", "ftkb_set_coords", "ftkb_set_producer_stream", "ftkb_get_layer",
     "ftkb_group_create", "ftkb_group_destroy", "ftkb_group_last_error", "ftkb_group_set_coords",
     "ftkb_group_set_streaming_trajectories", "ftkb_group_push_snapshot", "ftkb_group_push_synthetic",
+    "ftkb_group_push_snapshot_device", "ftkb_group_set_producer_stream",
     "ftkb_group_advance_timestep", "ftkb_group_update_timestep", "ftkb_group_finalize", "ftkb_group_get_stats",
     "ftkb_host_alloc", "ftkb_host_free", "ftkb_push_snapshot_f32", "ftkb_bind_thread_to_device",
 ]
@@ -155,6 +156,8 @@ def lib():
     L.ftkb_group_set_coords.argtypes = [vp, C.c_int, vp, C.c_uint64]
     L.ftkb_group_set_streaming_trajectories.argtypes = [vp, C.c_int]
     L.ftkb_group_push_snapshot.argtypes = [vp, vp, vp, vp]
+    L.ftkb_group_push_snapshot_device.argtypes = [vp, vp, vp, vp]
+    L.ftkb_group_set_producer_stream.argtypes = [vp, vp, C.c_int]
     L.ftkb_group_push_synthetic.argtypes = [vp, C.c_int, C.POINTER(C.c_double), C.c_int, C.c_double]
     L.ftkb_group_advance_timestep.argtypes = [vp]
     L.ftkb_group_update_timestep.argtypes = [vp]

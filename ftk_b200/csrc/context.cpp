@@ -15,6 +15,8 @@
 #include <cstdlib>
 #include <cstring>
 #include <deque>
+#include <mutex>
+#include <set>
 #include <string>
 #include <thread>
 #include <atomic>
@@ -472,8 +474,30 @@ static int new_layer(ftkb_ctx *c, Layer &l) {
   return FTKB_OK;
 }
 
-extern "C" int ftkb_push_snapshot(ftkb_ctx *c, const double *scalar, const double *vector, const double *jacobian, int where) {
-  if (!c) return FTKB_ERR_INVALID;
+// Peer access of `device` to `peer` (device arrays of a group's push may live on any device): enabled once per (destination,
+// source) pair where the hardware allows it; without it cudaMemcpyPeerAsync still copies, staged by the driver.  Leaves `device`
+// current.
+cudaError_t ftkb::enable_peer_access(int device, int peer) {
+  static std::mutex m;
+  static std::set<std::pair<int, int>> done;
+  cudaError_t e = cudaSetDevice(device);
+  if (e != cudaSuccess || device == peer) return e;
+  std::lock_guard<std::mutex> lk(m);
+  if (done.count({device, peer})) return cudaSuccess;
+  int can = 0;
+  if ((e = cudaDeviceCanAccessPeer(&can, device, peer)) != cudaSuccess) return e;
+  if (can && (e = cudaDeviceEnablePeerAccess(peer, 0)) != cudaSuccess) {
+    if (e != cudaErrorPeerAccessAlreadyEnabled) return e;
+    cudaGetLastError();
+  }
+  done.insert({device, peer});
+  return cudaSuccess;
+}
+
+// the ingest of every push: device arrays (FTKB_MEM_DEVICE) are read on `src_device`, the context's own or any other; `after`,
+// if not null, is an event every copy waits for (it replaces the context's own producer stream)
+static int push_snapshot(ftkb_ctx *c, const double *scalar, const double *vector, const double *jacobian, int where, int src_device,
+                         cudaEvent_t after) {
   if (where < FTKB_MEM_HOST || where > FTKB_MEM_DEVICE_BORROW) return fail(c, FTKB_ERR_INVALID, "push: bad memory kind");
   if (c->cfg.scalar_source == FTKB_SOURCE_GIVEN && !scalar) return fail(c, FTKB_ERR_INVALID, "push: scalar field is GIVEN but no scalar array was passed");
   if (c->cfg.vector_source == FTKB_SOURCE_GIVEN && !vector) return fail(c, FTKB_ERR_INVALID, "push: vector field is GIVEN but no vector array was passed");
@@ -485,7 +509,9 @@ extern "C" int ftkb_push_snapshot(ftkb_ctx *c, const double *scalar, const doubl
   Layer l;
   int rc = new_layer(c, l);
   if (rc) return rc;
-  if (where != FTKB_MEM_HOST && c->has_producer) {
+  if (after) {
+    CK(cudaStreamWaitEvent(c->stream, after, 0));
+  } else if (where != FTKB_MEM_HOST && c->has_producer) {
     // device inputs are written by the caller's stream: everything this context enqueues from here on runs after the
     // work queued there so far (the context's own stream is non-blocking: the legacy default stream orders nothing)
     CK(cudaEventRecord(c->ev_input, c->producer));
@@ -498,7 +524,10 @@ extern "C" int ftkb_push_snapshot(ftkb_ctx *c, const double *scalar, const doubl
     int r = take_buffer(c, pool, count, dst);
     if (r) return r;
     *own = true;
-    CK(cudaMemcpyAsync(*dst, src, sizeof(double) * count, where == FTKB_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, c->stream));
+    if (where == FTKB_MEM_DEVICE && src_device != c->cfg.device)
+      CK(cudaMemcpyPeerAsync(*dst, c->cfg.device, src, src_device, sizeof(double) * count, c->stream));
+    else
+      CK(cudaMemcpyAsync(*dst, src, sizeof(double) * count, where == FTKB_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, c->stream));
     if (where == FTKB_MEM_HOST) c->stats.h2d_bytes += sizeof(double) * count;
     return FTKB_OK;
   };
@@ -510,6 +539,17 @@ extern "C" int ftkb_push_snapshot(ftkb_ctx *c, const double *scalar, const doubl
   if (where != FTKB_MEM_DEVICE_BORROW) CK(cudaStreamSynchronize(c->stream));
   c->layers.push_back(l);
   return FTKB_OK;
+}
+
+extern "C" int ftkb_push_snapshot(ftkb_ctx *c, const double *scalar, const double *vector, const double *jacobian, int where) {
+  if (!c) return FTKB_ERR_INVALID;
+  return push_snapshot(c, scalar, vector, jacobian, where, c->cfg.device, nullptr);
+}
+
+int ftkb::push_snapshot_from(ftkb_ctx *c, const double *scalar, const double *vector, const double *jacobian, int src_device, cudaEvent_t after) {
+  if (!c) return FTKB_ERR_INVALID;
+  CK(ftkb::enable_peer_access(c->cfg.device, src_device));
+  return push_snapshot(c, scalar, vector, jacobian, FTKB_MEM_DEVICE, src_device, after);
 }
 
 // A snapshot that exists as float32 (raw float32 file series: the reference widens them on the host, ndarray.hh read_binary_file):

@@ -135,6 +135,10 @@ struct ftkb_group {
   bool streaming = false;                          // grow trajectories on the merged context (ftkb_group_set_streaming_trajectories)
   int coords_mode = FTKB_COORDS_SIMPLE;            // ftkb_group_set_coords, handed to every chunk context
   std::vector<double> coords;
+  cudaStream_t producer = nullptr;                 // ftkb_group_set_producer_stream: device pushes wait for the work queued there
+  bool has_producer = false;
+  cudaEvent_t ev_producer = nullptr;               // recorded on `producer` by every device push (created on ev_device)
+  int ev_device = -1;
   std::atomic<int> failed{FTKB_OK};
   std::string error;
   ftkb_ctx *root = nullptr;
@@ -263,6 +267,7 @@ extern "C" void ftkb_group_destroy(ftkb_group *g) {
   for (auto &ch : g->chunks) if (ch->ctx) ftkb_destroy(ch->ctx);
   for (auto &sl : g->slabs) if (sl.ctx) ftkb_destroy(sl.ctx);
   if (g->root) ftkb_destroy(g->root);
+  if (g->ev_producer) { int cur = 0; cudaGetDevice(&cur); cudaSetDevice(g->ev_device); cudaEventDestroy(g->ev_producer); cudaSetDevice(cur); }
   delete g;
 }
 
@@ -363,48 +368,70 @@ static int push_layer(ftkb_group *g, std::function<int(ftkb_ctx *)> push, bool w
   return rc;
 }
 
+// Where a snapshot's arrays come from: host memory, or CUDA device memory on `device` (any device, in the group or not), every
+// copy ordered after `after` when it is set.  Either way the arrays are borrowed only until the push returns.
+struct Source {
+  bool on_device = false;
+  int device = -1;
+  cudaEvent_t after = nullptr;
+  int push(ftkb_ctx *c, const double *S, const double *V, const double *J) const {
+    return on_device ? ftkb::push_snapshot_from(c, S, V, J, device, after) : ftkb_push_snapshot(c, S, V, J, FTKB_MEM_HOST);
+  }
+};
+
 // The first layer of chunk c > 0 arrives while chunk c-1 may still have to finish before chunk c's context can exist (it
 // inherits the running minimum), and chunk c-1 finishes with an advance the caller only issues after this push has returned.
 // So that layer is copied to the new chunk's device right away, into buffers of the group, and handed to the context later.
 struct Staged { double *S = nullptr, *V = nullptr, *J = nullptr; };
 
-extern "C" int ftkb_group_push_snapshot(ftkb_group *g, const double *scalar, const double *vector, const double *jacobian) {
-  if (!g) return FTKB_ERR_INVALID;
-  if (g->failed.load()) return g->failed.load();
+static int push_snapshot(ftkb_group *g, const double *scalar, const double *vector, const double *jacobian, const Source src) {
   if (g->spatial) {
-    // every device copies its planes (ghost planes included) over its own PCIe link, concurrently
+    // every device copies its planes (ghost planes included) over its own link, concurrently
     const size_t plane = (size_t)g->cfg.dims[0] * (size_t)g->cfg.dims[1];
     return spatial_push(g, [=](Slab &sl) {
       const size_t o = plane * (size_t)sl.a0;
-      return ftkb_push_snapshot(sl.ctx, scalar ? scalar + o : nullptr, vector ? vector + 3 * o : nullptr, jacobian ? jacobian + 9 * o : nullptr, FTKB_MEM_HOST);
+      return src.push(sl.ctx, scalar ? scalar + o : nullptr, vector ? vector + 3 * o : nullptr, jacobian ? jacobian + 9 * o : nullptr);
     });
   }
   const int k = g->npushed;
   if (k % g->B != 0 || k == 0)
-    // host memory, borrowed until return: wait for the copy
-    return push_layer(g, [=](ftkb_ctx *c) { return ftkb_push_snapshot(c, scalar, vector, jacobian, FTKB_MEM_HOST); }, true);
+    // borrowed until return: wait for the copy
+    return push_layer(g, [=](ftkb_ctx *c) { return src.push(c, scalar, vector, jacobian); }, true);
   g->npushed++;
   const int c = k / g->B;
   size_t nvert = 1;
   for (int j = 0; j < g->cfg.nd; j++) nvert *= (size_t)g->cfg.dims[j];
   const size_t n = (size_t)g->cfg.nd;
   std::shared_ptr<Done> d_halo(new Done()), d_stage(new Done());
-  post_push(g, c - 1, [=](ftkb_ctx *x) { return ftkb_push_snapshot(x, scalar, vector, jacobian, FTKB_MEM_HOST); }, d_halo);   // halo of the chunk before
+  post_push(g, c - 1, [=](ftkb_ctx *x) { return src.push(x, scalar, vector, jacobian); }, d_halo);   // halo of the chunk before
   Chunk *ch = g->chunk(c);
   Worker *w = g->workers[ch->index % g->workers.size()].get();
   std::shared_ptr<Staged> st(new Staged());
   w->post([=] {
     int rc = g->failed.load();
-    auto up = [&](const double *src, size_t count, double **dst) {
-      if (!src || rc) return;
-      if (cudaMalloc(dst, count * sizeof(double)) != cudaSuccess || cudaMemcpy(*dst, src, count * sizeof(double), cudaMemcpyHostToDevice) != cudaSuccess) {
-        cudaGetLastError();
-        rc = FTKB_ERR_NOMEM;
-        g->fail(rc, "group: staging the first layer of a chunk failed");
-      }
+    cudaStream_t s = nullptr;      // device source: the copies run here, after the producer
+    auto ck = [&](cudaError_t e) {
+      if (e == cudaSuccess || rc) return;
+      cudaGetLastError();
+      rc = e == cudaErrorMemoryAllocation ? FTKB_ERR_NOMEM : FTKB_ERR_CUDA;
+      g->fail(rc, std::string("group: staging the first layer of a chunk failed: ") + cudaGetErrorString(e));
     };
-    if (!rc && cudaSetDevice(ch->device) != cudaSuccess) { cudaGetLastError(); rc = FTKB_ERR_CUDA; g->fail(rc, "cudaSetDevice"); }
+    auto up = [&](const double *from, size_t count, double **dst) {
+      if (!from || rc) return;
+      const size_t bytes = count * sizeof(double);
+      ck(cudaMalloc(dst, bytes));
+      if (rc) return;
+      if (!src.on_device) ck(cudaMemcpy(*dst, from, bytes, cudaMemcpyHostToDevice));
+      else if (src.device == ch->device) ck(cudaMemcpyAsync(*dst, from, bytes, cudaMemcpyDeviceToDevice, s));
+      else ck(cudaMemcpyPeerAsync(*dst, ch->device, from, src.device, bytes, s));
+    };
+    if (!rc) ck(src.on_device ? ftkb::enable_peer_access(ch->device, src.device) : cudaSetDevice(ch->device));
+    if (src.on_device) {
+      ck(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+      if (src.after) ck(cudaStreamWaitEvent(s, src.after, 0));
+    }
     up(scalar, nvert, &st->S); up(vector, nvert * n, &st->V); up(jacobian, nvert * n * n, &st->J);
+    if (s) { ck(cudaStreamSynchronize(s)); cudaStreamDestroy(s); }
     d_stage->set(rc);
   });
   w->post([=] {
@@ -419,6 +446,54 @@ extern "C" int ftkb_group_push_snapshot(ftkb_group *g, const double *scalar, con
   });
   const int r1 = d_halo->wait(), r2 = d_stage->wait();
   return r1 ? r1 : r2;
+}
+
+extern "C" int ftkb_group_push_snapshot(ftkb_group *g, const double *scalar, const double *vector, const double *jacobian) {
+  if (!g) return FTKB_ERR_INVALID;
+  if (g->failed.load()) return g->failed.load();
+  return push_snapshot(g, scalar, vector, jacobian, Source());
+}
+
+extern "C" int ftkb_group_set_producer_stream(ftkb_group *g, void *stream, int enable) {
+  if (!g) return FTKB_ERR_INVALID;
+  g->producer = reinterpret_cast<cudaStream_t>(stream);
+  g->has_producer = enable != 0;
+  return FTKB_OK;
+}
+
+extern "C" int ftkb_group_push_snapshot_device(ftkb_group *g, const double *scalar, const double *vector, const double *jacobian) {
+  if (!g) return FTKB_ERR_INVALID;
+  if (g->failed.load()) return g->failed.load();
+  // a rejected push leaves the group as it was: the caller may push a valid snapshot next
+  auto reject = [g](const std::string &msg) { std::lock_guard<std::mutex> lk(g->m); g->error = "push_snapshot_device: " + msg; return FTKB_ERR_INVALID; };
+  Source src;
+  src.on_device = true;
+  const double *arrays[3] = {scalar, vector, jacobian};
+  const char *names[3] = {"scalar", "vector", "jacobian"};
+  for (int i = 0; i < 3; i++) {
+    if (!arrays[i]) continue;
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, arrays[i]) != cudaSuccess) { cudaGetLastError(); a.type = cudaMemoryTypeUnregistered; }
+    if (a.type != cudaMemoryTypeDevice) return reject(std::string("the ") + names[i] + " array is not CUDA device memory (host, unregistered and managed memory are refused)");
+    if ((uintptr_t)arrays[i] % 8 != 0) return reject(std::string("the ") + names[i] + " array is not 8-byte aligned");
+    if (src.device >= 0 && a.device != src.device) return reject(std::string("the ") + names[i] + " array is on another device than the arrays before it");
+    src.device = a.device;
+  }
+  if (src.device < 0) return reject("no array was passed");
+  if (g->has_producer) {
+    // one event is enough: this push returns only after every copy that waits for it has completed
+    int dev = src.device, cur = 0;
+    if (g->producer && cudaStreamGetDevice(g->producer, &dev) != cudaSuccess) { cudaGetLastError(); return reject("the producer stream is not a valid CUDA stream"); }
+    cudaError_t e = cudaGetDevice(&cur);
+    if (!e) e = cudaSetDevice(dev);           // (the legacy default stream, producer = NULL, is the source device's)
+    if (!e && g->ev_producer && g->ev_device != dev) { e = cudaEventDestroy(g->ev_producer); g->ev_producer = nullptr; }
+    if (!e && !g->ev_producer && !(e = cudaEventCreateWithFlags(&g->ev_producer, cudaEventDisableTiming))) g->ev_device = dev;
+    if (!e) e = cudaEventRecord(g->ev_producer, g->producer);
+    cudaSetDevice(cur);
+    if (e) { cudaGetLastError(); std::lock_guard<std::mutex> lk(g->m); g->error = std::string("push_snapshot_device: producer event: ") + cudaGetErrorString(e); return FTKB_ERR_CUDA; }
+    src.after = g->ev_producer;
+  }
+  return push_snapshot(g, scalar, vector, jacobian, src);
 }
 
 extern "C" int ftkb_group_push_synthetic(ftkb_group *g, int kind, const double *params, int nparams, double t) {

@@ -5,6 +5,8 @@
 #include <deque>
 #include <vector>
 
+#include <cuda_runtime.h>
+
 #include "../../include/ftkb200.h"
 #include "mesh_tables.h"
 
@@ -69,5 +71,11 @@ class OnlineTracer {
 // (context.cpp) one grow step of a streaming context over its imported points [grown so far, end): how a device group's merged
 // context replays the grow steps of the chunks or slabs that swept for it (group.cpp)
 int grow_imported(ftkb_ctx *c, uint64_t end);
+
+// (context.cpp) ftkb_push_snapshot(c, .., FTKB_MEM_DEVICE) for device arrays on any device `src_device` (a peer copy when it is not
+// the context's own), every copy ordered after `after` unless it is null: how a device group pulls a device snapshot (group.cpp)
+int push_snapshot_from(ftkb_ctx *c, const double *scalar, const double *vector, const double *jacobian, int src_device, cudaEvent_t after);
+// (context.cpp) lets `device` read `peer`'s memory where the hardware allows it, once per pair; makes `device` current
+cudaError_t enable_peer_access(int device, int peer);
 
 }  // namespace ftkb

@@ -6,13 +6,17 @@ thread per device), or, with chunk=0 (3D), through z-slabs that every device swe
 one-device tracker bit for bit; ftkb_group_finalize merges everything into one context, which this class then exposes through
 the ordinary tracker getters.  streaming=True grows trajectories there as a single streaming tracker does; coords=(mode, data)
 takes make_tracker's forms, for the whole array.
+
+Snapshots are numpy arrays (host memory) or device arrays -- torch CUDA tensors, or anything with __cuda_array_interface__ --
+on any visible device, one of the group's or not: every device then copies what it needs from the source device (peer copies
+over NVLink), ordered after torch's current stream on the tensor's device.  Either kind is consumed before the push returns.
 """
 import ctypes as C
 
 import numpy as np
 
 from . import _lib as L
-from .tracker import coords_arg, make_tracker, _RegularTracker, SOURCE_DERIVED, SOURCE_GIVEN, SOURCE_NONE
+from .tracker import coords_arg, make_tracker, _dev_ptr, _RegularTracker, SOURCE_DERIVED, SOURCE_GIVEN, SOURCE_NONE
 
 
 class _GroupRoot(_RegularTracker):
@@ -28,7 +32,8 @@ class _GroupRoot(_RegularTracker):
 
 class GroupTracker:
     def __init__(self, dims, device_ids, field="scalar", chunk=8, lb=None, ub=None, jacobian_symmetric=None, robust=True,
-                 compute_degrees=False, type_filter=None, start_timestep=0, streaming=False, coords=None):
+                 compute_degrees=False, type_filter=None, start_timestep=0, streaming=False, coords=None,
+                 scalar_source=None, vector_source=None, jacobian_source=None):
         nd = len(dims)
         if field == "scalar":
             ss, vs, js, sym, margin = SOURCE_GIVEN, SOURCE_DERIVED, SOURCE_DERIVED, True, 2
@@ -43,7 +48,9 @@ class GroupTracker:
             cfg.dims[i] = dims[i] if i < nd else 1
             cfg.lb[i] = lo[i] if i < nd else 0
             cfg.ub[i] = hi[i] if i < nd else 0
-        cfg.scalar_source, cfg.vector_source, cfg.jacobian_source = ss, vs, js
+        cfg.scalar_source = ss if scalar_source is None else int(scalar_source)
+        cfg.vector_source = vs if vector_source is None else int(vector_source)
+        cfg.jacobian_source = js if jacobian_source is None else int(jacobian_source)
         cfg.jacobian_symmetric = int(sym if jacobian_symmetric is None else jacobian_symmetric)
         cfg.robust_detection = int(robust)
         cfg.compute_degrees = int(compute_degrees)
@@ -69,12 +76,54 @@ class GroupTracker:
             raise L.FTKBError(rc, L.lib().ftkb_group_last_error(self._g).decode())
 
     def push_scalar_field_snapshot(self, a):
-        h = np.ascontiguousarray(a, dtype=np.float64)
-        self._check(L.lib().ftkb_group_push_snapshot(self._g, h.ctypes.data, None, None))
+        self.push_field_data_snapshot(scalar=a)
 
     def push_vector_field_snapshot(self, a):
-        h = np.ascontiguousarray(a, dtype=np.float64)
-        self._check(L.lib().ftkb_group_push_snapshot(self._g, None, h.ctypes.data, None))
+        self.push_field_data_snapshot(vector=a)
+
+    def push_field_data_snapshot(self, scalar=None, vector=None, jacobian=None):
+        """ref: critical_point_tracker.hh:202-213.  Host arrays, or float64 device arrays on one device (any visible one):
+        copied to every device of the group before the call returns."""
+        n = self._nd
+        shape = tuple(reversed(self._dims))
+        ptrs, hold, on_device = [], [], None
+        for a, trailing in ((scalar, ()), (vector, (n,)), (jacobian, (n, n))):
+            if a is None:
+                ptrs.append(None)
+                continue
+            dp = _dev_ptr(a)
+            count = int(np.prod(shape + trailing))
+            if dp is not None:
+                if int(np.prod(tuple(a.shape))) != count or (hasattr(a, "is_contiguous") and not a.is_contiguous()):
+                    raise ValueError("device array has the wrong size or is not contiguous")
+                if str(getattr(a, "dtype", "")) != "torch.float64" and getattr(a, "__cuda_array_interface__", {}).get("typestr") != "<f8":
+                    raise ValueError("device arrays must be float64")
+                ptrs.append(dp)
+            else:
+                h = np.ascontiguousarray(a, dtype=np.float64)
+                if h.size != count:
+                    raise ValueError(f"array has {h.size} elements, expected {count}")
+                ptrs.append(h.ctypes.data)
+                a = h
+            hold.append(a)
+            if on_device is not None and on_device != (dp is not None):
+                raise ValueError("scalar/vector/jacobian must all be host arrays or all be device arrays")
+            on_device = dp is not None
+        if on_device:
+            self._order_after_producer(hold)
+            self._check(L.lib().ftkb_group_push_snapshot_device(self._g, ptrs[0], ptrs[1], ptrs[2]))
+        else:
+            self._check(L.lib().ftkb_group_push_snapshot(self._g, ptrs[0], ptrs[1], ptrs[2]))
+
+    def _order_after_producer(self, arrays):
+        """device inputs: every copy waits for torch's current stream on the tensor's device (ftkb_group_set_producer_stream);
+        other producers synchronise before pushing"""
+        for a in arrays:
+            if getattr(a, "is_cuda", False) and hasattr(a, "data_ptr"):
+                import torch
+                stream = int(torch.cuda.current_stream(a.device).cuda_stream)
+                self._check(L.lib().ftkb_group_set_producer_stream(self._g, C.c_void_p(stream), 1))
+                return
 
     def push_synthetic_snapshot(self, kind, params, t):
         p = (C.c_double * max(len(params), 1))(*[float(v) for v in params])

@@ -92,7 +92,8 @@ class ndarray {
     dims_ = shape;
     if (!borrowed_) own_.assign(nelem(), T());
   }
-  // borrow caller memory (no copy); device = the pointer is CUDA device memory on the tracker's device
+  // borrow caller memory (no copy); device = the pointer is CUDA device memory: on the tracker's device for one device, on any
+  // visible device for a tracker on several devices (set_device_ids), whose devices copy it from there
   static ndarray wrap(const T *p, const std::vector<size_t> &shape, bool device = false) {
     ndarray a;
     a.dims_ = shape; a.ext_ = p; a.borrowed_ = true; a.device_ = device;
@@ -410,10 +411,9 @@ class critical_point_tracker_regular {
     };
     const double *s = ptr(scalar, nvert, "scalar"), *v = ptr(vector, nvert * nd_, "vector"), *j = ptr(jacobian, nvert * nd_ * nd_, "jacobian");
     const bool dev = scalar.on_device() || vector.on_device() || jacobian.on_device();
-    if (group_) {
-      if (dev) throw std::runtime_error("ftk_b200: a tracker on several devices takes host snapshots");
-      gcheck(ftkb_group_push_snapshot(group_, s, v, j));
-    } else
+    if (group_)
+      gcheck(dev ? ftkb_group_push_snapshot_device(group_, s, v, j) : ftkb_group_push_snapshot(group_, s, v, j));
+    else
     check(ftkb_push_snapshot(ctx_, s, v, j, dev ? FTKB_MEM_DEVICE : FTKB_MEM_HOST));
     points_valid_ = false;
   }

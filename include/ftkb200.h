@@ -221,6 +221,15 @@ int ftkb_push_snapshot_remote(ftkb_ctx *, const double *scalar, const double *ve
  * device_ids[0] and traces there; *root stays owned by the group and serves every getter (ftkb_get_points, ftkb_get_trajectories,
  * ftkb_get_trajectory_complete, ftkb_get_curveset ...).  cfg->device is ignored.
  * ftkb_group_push_snapshot takes HOST memory (borrowed until return); ftkb_group_push_synthetic generates on the devices.
+ * ftkb_group_push_snapshot_device takes CUDA DEVICE memory on any visible device, one of the group's or not (a producer on
+ * GPU 0 feeding a group of eight): every context that needs the snapshot -- a chunk's own and, for the first layer of a chunk,
+ * the one-layer halo of the chunk before; or every z-slab, for its planes -- copies it from the source device on its own
+ * stream, all at once: a device-to-device copy on the same device, cudaMemcpyPeerAsync (NVLink copy engines, no kernel)
+ * otherwise.  Peer access is enabled once per (destination, source) pair where the hardware allows it.  Host and device pushes
+ * may alternate in one series.
+ * ftkb_group_set_producer_stream names the stream (on its own device; NULL: the legacy default stream of the source device)
+ * that writes those arrays: every later device push records an event there and every copy waits for it.  Without it the caller
+ * synchronises the producer before pushing.
  *
  * Options, valid only before the first push (afterwards FTKB_ERR_INVALID):
  *   ftkb_group_set_coords                   ftkb_set_coords for the whole array: same modes and sizes, host data copied before
@@ -246,6 +255,14 @@ const char *ftkb_group_last_error(const ftkb_group *);
 int ftkb_group_set_coords(ftkb_group *, int mode, const double *data, uint64_t n);
 int ftkb_group_set_streaming_trajectories(ftkb_group *, int enable);
 int ftkb_group_push_snapshot(ftkb_group *, const double *scalar, const double *vector, const double *jacobian);
+/* a snapshot in CUDA device memory on any visible device (not necessarily one of the group's): same arrays, sizes and NULL
+ * rules as ftkb_group_push_snapshot; all non-NULL pointers on the same device, 8-byte aligned.  Copied: the call returns when
+ * every device of the group holds its copy, so the caller may overwrite the arrays right away.  Host, unregistered and managed
+ * memory, arrays on two devices and misaligned arrays are refused with FTKB_ERR_INVALID and leave the group as it was. */
+int ftkb_group_push_snapshot_device(ftkb_group *, const double *scalar, const double *vector, const double *jacobian);
+/* the group's counterpart of ftkb_set_producer_stream: every copy of a later device push waits for the work queued on
+ * `stream` (on its own device) when the push is called; enable = 0 turns it off */
+int ftkb_group_set_producer_stream(ftkb_group *, void *cuda_stream, int enable);
 int ftkb_group_push_synthetic(ftkb_group *, int kind, const double *params, int nparams, double t);
 int ftkb_group_advance_timestep(ftkb_group *);
 int ftkb_group_update_timestep(ftkb_group *);
