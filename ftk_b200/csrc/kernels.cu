@@ -1139,7 +1139,7 @@ void launch_scan2d_cells(const SweepParams &p, cudaStream_t s) {
 // Determinant guard, exponent form: with e_c the biased exponent of max |d_c| (at least that of 2^-nbits),
 // |quantised v_c| < 2^(e_c - 1023 + nbits) and M_c := |quantised| + 1 <= 2^(e_c - 1022 + nbits).  Every determinant of
 // the cascade is at most 48 Mx My Mz (cube_excluded3 with R <= 2 M) < 2^(6 + sum(e_c) - 3066 + 3 nbits), which stays
-// below 2^62 for sum(e_c) <= 3119 - 3 nbits.
+// below 2^59 for sum(e_c) <= 3119 - 3 nbits: three binades under 2^62, four under the int64 range.
 constexpr int F3_LAYER_BYTES = ((F3_ROWS * F3_COLS * 8 + 127) / 128) * 128;   // one staged plane of one layer
 constexpr uint32_t F3_BOX_BYTES = F3_ROWS * F3_COLS * 8;
 
@@ -1257,9 +1257,10 @@ __device__ __noinline__ bool s3_union_excluded_precise(const float mn0, const fl
                                                        const float mn2, const float mx2, const int nbits20) {
   const auto lo = [](float f) { const int k = __float_as_int(f); return k < 0 ? (k | 0xFFFF) : k; };
   const auto hi = [](float f) { const int k = __float_as_int(f); return k < 0 ? k : (k | 0xFFFF); };
-  const KeyRange x{vertex_range(lo(mn0), nbits20).mn, vertex_range(hi(mx0), nbits20).mx};
-  const KeyRange y{vertex_range(lo(mn1), nbits20).mn, vertex_range(hi(mx1), nbits20).mx};
-  const KeyRange z{vertex_range(lo(mn2), nbits20).mn, vertex_range(hi(mx2), nbits20).mx};
+  // merged, not {lo.mn, hi.mx}: a poisoned upper end (|p| >= 2^63) must poison the range's mn, which the guards test
+  const KeyRange x = merge(vertex_range(lo(mn0), nbits20), vertex_range(hi(mx0), nbits20));
+  const KeyRange y = merge(vertex_range(lo(mn1), nbits20), vertex_range(hi(mx1), nbits20));
+  const KeyRange z = merge(vertex_range(lo(mn2), nbits20), vertex_range(hi(mx2), nbits20));
   return cube_excluded3(x, y, z);
 }
 
@@ -1758,8 +1759,10 @@ __device__ __forceinline__ void vcells2d_decide(const SweepParams &p, const floa
   const int nbits20 = p.nbits << 20;
   bool excl = false;
   if (!(xmn != xmn) && !(ymn != ymn)) {       // a NaN union (no vertex) goes to the cold path, which is exact
-    const KeyRange x{vertex_range(__float_as_int(xmn), nbits20).mn, vertex_range(__float_as_int(xmx), nbits20).mx};
-    const KeyRange y{vertex_range(__float_as_int(ymn), nbits20).mn, vertex_range(__float_as_int(ymx), nbits20).mx};
+    // merged, not {min.mn, max.mx}: a positive value with |p| >= 2^63 (INT64_MIN in the reference) at the upper end must poison
+    // the range's mn, which cube_excluded2 tests
+    const KeyRange x = merge(vertex_range(__float_as_int(xmn), nbits20), vertex_range(__float_as_int(xmx), nbits20));
+    const KeyRange y = merge(vertex_range(__float_as_int(ymn), nbits20), vertex_range(__float_as_int(ymx), nbits20));
     excl = cube_excluded2(x, y);
   }
   const unsigned fm = __ballot_sync(0xffffffffu, own && !excl);
