@@ -65,6 +65,12 @@ CURVE_INFO_DTYPE = np.dtype([
 ], align=True)
 assert CURVE_INFO_DTYPE.itemsize == 136
 
+class Piece(C.Structure):
+    """ftkb_piece: planes [first, first + count) of a snapshot's slowest axis, in device memory"""
+    _fields_ = [("scalar", C.c_void_p), ("vector", C.c_void_p), ("jacobian", C.c_void_p), ("first", C.c_int32), ("count", C.c_int32),
+                ("stream", C.c_void_p), ("has_stream", C.c_int32), ("reserved", C.c_int32)]
+
+
 # every symbol include/ftkb200.h declares
 EXPORTS = [
     "ftkb_abi_version", "ftkb_device_count", "ftkb_create", "ftkb_destroy", "ftkb_last_error", "ftkb_push_snapshot",
@@ -80,7 +86,7 @@ EXPORTS = [
     "ftkb_online_size", "ftkb_online_get", "ftkb_set_coords", "ftkb_set_producer_stream", "ftkb_get_layer",
     "ftkb_group_create", "ftkb_group_destroy", "ftkb_group_last_error", "ftkb_group_set_coords",
     "ftkb_group_set_streaming_trajectories", "ftkb_group_push_snapshot", "ftkb_group_push_synthetic",
-    "ftkb_group_push_snapshot_device", "ftkb_group_set_producer_stream",
+    "ftkb_group_push_snapshot_device", "ftkb_group_set_producer_stream", "ftkb_group_push_pieces_device", "ftkb_group_get_slab",
     "ftkb_group_advance_timestep", "ftkb_group_update_timestep", "ftkb_group_finalize", "ftkb_group_get_stats",
     "ftkb_host_alloc", "ftkb_host_free", "ftkb_push_snapshot_f32", "ftkb_bind_thread_to_device",
 ]
@@ -158,6 +164,8 @@ def lib():
     L.ftkb_group_push_snapshot.argtypes = [vp, vp, vp, vp]
     L.ftkb_group_push_snapshot_device.argtypes = [vp, vp, vp, vp]
     L.ftkb_group_set_producer_stream.argtypes = [vp, vp, C.c_int]
+    L.ftkb_group_push_pieces_device.argtypes = [vp, C.POINTER(Piece), C.c_int32]
+    L.ftkb_group_get_slab.argtypes = [vp, C.c_int32, C.POINTER(C.c_int32)]
     L.ftkb_group_push_synthetic.argtypes = [vp, C.c_int, C.POINTER(C.c_double), C.c_int, C.c_double]
     L.ftkb_group_advance_timestep.argtypes = [vp]
     L.ftkb_group_update_timestep.argtypes = [vp]

@@ -494,46 +494,61 @@ cudaError_t ftkb::enable_peer_access(int device, int peer) {
   return cudaSuccess;
 }
 
-// the ingest of every push: device arrays (FTKB_MEM_DEVICE) are read on `src_device`, the context's own or any other; `after`,
-// if not null, is an event every copy waits for (it replaces the context's own producer stream)
-static int push_snapshot(ftkb_ctx *c, const double *scalar, const double *vector, const double *jacobian, int where, int src_device,
-                         cudaEvent_t after) {
+// the ingest of every push: the layer is copied from `segs`, which tile the array in plane order (one segment covering it all
+// for host input and for borrowed arrays); device arrays (FTKB_MEM_DEVICE) are read on each segment's device, the context's own
+// or any other.  A segment's `after`, if not null, is an event its copies wait for (it replaces the context's own producer stream).
+static int push_snapshot(ftkb_ctx *c, const ftkb::Segment *segs, int nsegs, int where) {
+  const double *scalar = segs[0].scalar, *vector = segs[0].vector, *jacobian = segs[0].jacobian;
   if (where < FTKB_MEM_HOST || where > FTKB_MEM_DEVICE_BORROW) return fail(c, FTKB_ERR_INVALID, "push: bad memory kind");
   if (c->cfg.scalar_source == FTKB_SOURCE_GIVEN && !scalar) return fail(c, FTKB_ERR_INVALID, "push: scalar field is GIVEN but no scalar array was passed");
   if (c->cfg.vector_source == FTKB_SOURCE_GIVEN && !vector) return fail(c, FTKB_ERR_INVALID, "push: vector field is GIVEN but no vector array was passed");
   if (c->cfg.vector_source == FTKB_SOURCE_DERIVED && !vector && !scalar) return fail(c, FTKB_ERR_INVALID, "push: vector field is DERIVED but no scalar array was passed");
   if (c->cfg.jacobian_source == FTKB_SOURCE_GIVEN && !jacobian) return fail(c, FTKB_ERR_INVALID, "push: jacobian is GIVEN but no jacobian array was passed");
   CK(cudaSetDevice(c->cfg.device));
-  for (const double *q : {scalar, vector, jacobian})
-    if ((uintptr_t)q % 8 != 0) return fail(c, FTKB_ERR_INVALID, "push: arrays must be 8-byte aligned");
+  const int extent = c->n == 3 ? c->cfg.dims[2] : c->cfg.dims[1];
+  for (int i = 0, next = 0; i < nsegs; next += segs[i++].count) {
+    const ftkb::Segment &s = segs[i];
+    if (s.first != next || s.count < 1 || (i == nsegs - 1 && s.first + s.count != extent) || (where == FTKB_MEM_DEVICE_BORROW && nsegs != 1) ||
+        !s.scalar != !scalar || !s.vector != !vector || !s.jacobian != !jacobian)
+      return fail(c, FTKB_ERR_INVALID, "push: segments do not tile the array with the same arrays");
+    for (const double *q : {s.scalar, s.vector, s.jacobian})
+      if ((uintptr_t)q % 8 != 0) return fail(c, FTKB_ERR_INVALID, "push: arrays must be 8-byte aligned");
+  }
   Layer l;
   int rc = new_layer(c, l);
   if (rc) return rc;
-  if (after) {
-    CK(cudaStreamWaitEvent(c->stream, after, 0));
-  } else if (where != FTKB_MEM_HOST && c->has_producer) {
+  bool ordered = false;
+  for (int i = 0; i < nsegs; i++)
+    if (segs[i].after) { CK(cudaStreamWaitEvent(c->stream, segs[i].after, 0)); ordered = true; }
+  if (!ordered && where != FTKB_MEM_HOST && c->has_producer) {
     // device inputs are written by the caller's stream: everything this context enqueues from here on runs after the
     // work queued there so far (the context's own stream is non-blocking: the legacy default stream orders nothing)
     CK(cudaEventRecord(c->ev_input, c->producer));
     CK(cudaStreamWaitEvent(c->stream, c->ev_input, 0));
   }
-  const size_t nS = c->nvert, nV = c->nvert * c->n, nJ = c->nvert * c->n * c->n;
-  auto ingest = [&](const double *src, size_t count, std::vector<double *> &pool, double **dst, bool *own) -> int {
-    if (!src) return FTKB_OK;
-    if (where == FTKB_MEM_DEVICE_BORROW) { *dst = const_cast<double *>(src); *own = false; return FTKB_OK; }
-    int r = take_buffer(c, pool, count, dst);
+  const size_t plane = c->nvert / (size_t)extent;
+  // one copy per segment of array `a`, whose vertices hold `per` doubles each
+  auto ingest = [&](const double *ftkb::Segment::*a, size_t per, std::vector<double *> &pool, double **dst, bool *own) -> int {
+    if (!(segs[0].*a)) return FTKB_OK;
+    if (where == FTKB_MEM_DEVICE_BORROW) { *dst = const_cast<double *>(segs[0].*a); *own = false; return FTKB_OK; }
+    int r = take_buffer(c, pool, c->nvert * per, dst);
     if (r) return r;
     *own = true;
-    if (where == FTKB_MEM_DEVICE && src_device != c->cfg.device)
-      CK(cudaMemcpyPeerAsync(*dst, c->cfg.device, src, src_device, sizeof(double) * count, c->stream));
-    else
-      CK(cudaMemcpyAsync(*dst, src, sizeof(double) * count, where == FTKB_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, c->stream));
-    if (where == FTKB_MEM_HOST) c->stats.h2d_bytes += sizeof(double) * count;
+    for (int i = 0; i < nsegs; i++) {
+      const ftkb::Segment &s = segs[i];
+      double *to = *dst + (size_t)s.first * plane * per;
+      const size_t bytes = sizeof(double) * (size_t)s.count * plane * per;
+      if (where == FTKB_MEM_DEVICE && s.device != c->cfg.device)
+        CK(cudaMemcpyPeerAsync(to, c->cfg.device, s.*a, s.device, bytes, c->stream));
+      else
+        CK(cudaMemcpyAsync(to, s.*a, bytes, where == FTKB_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice, c->stream));
+      if (where == FTKB_MEM_HOST) c->stats.h2d_bytes += bytes;
+    }
     return FTKB_OK;
   };
-  if ((rc = ingest(scalar, nS, c->freeS, &l.S, &l.ownS))) { release_layer(c, l); return rc; }
-  if ((rc = ingest(vector, nV, c->freeV, &l.V, &l.ownV))) { release_layer(c, l); return rc; }
-  if ((rc = ingest(jacobian, nJ, c->freeJ, &l.J, &l.ownJ))) { release_layer(c, l); return rc; }
+  if ((rc = ingest(&ftkb::Segment::scalar, 1, c->freeS, &l.S, &l.ownS))) { release_layer(c, l); return rc; }
+  if ((rc = ingest(&ftkb::Segment::vector, c->n, c->freeV, &l.V, &l.ownV))) { release_layer(c, l); return rc; }
+  if ((rc = ingest(&ftkb::Segment::jacobian, c->n * c->n, c->freeJ, &l.J, &l.ownJ))) { release_layer(c, l); return rc; }
   if ((rc = derive_layer(c, l))) { release_layer(c, l); return rc; }
   // copied inputs (host or device) are borrowed only until return: the caller may free or overwrite them right away
   if (where != FTKB_MEM_DEVICE_BORROW) CK(cudaStreamSynchronize(c->stream));
@@ -543,13 +558,17 @@ static int push_snapshot(ftkb_ctx *c, const double *scalar, const double *vector
 
 extern "C" int ftkb_push_snapshot(ftkb_ctx *c, const double *scalar, const double *vector, const double *jacobian, int where) {
   if (!c) return FTKB_ERR_INVALID;
-  return push_snapshot(c, scalar, vector, jacobian, where, c->cfg.device, nullptr);
+  ftkb::Segment s;           // the whole array as one segment
+  s.count = c->n == 3 ? c->cfg.dims[2] : c->cfg.dims[1];
+  s.scalar = scalar; s.vector = vector; s.jacobian = jacobian;
+  s.device = c->cfg.device;
+  return push_snapshot(c, &s, 1, where);
 }
 
-int ftkb::push_snapshot_from(ftkb_ctx *c, const double *scalar, const double *vector, const double *jacobian, int src_device, cudaEvent_t after) {
-  if (!c) return FTKB_ERR_INVALID;
-  CK(ftkb::enable_peer_access(c->cfg.device, src_device));
-  return push_snapshot(c, scalar, vector, jacobian, FTKB_MEM_DEVICE, src_device, after);
+int ftkb::push_segments(ftkb_ctx *c, const Segment *segs, int n) {
+  if (!c || !segs || n < 1) return FTKB_ERR_INVALID;
+  for (int i = 0; i < n; i++) CK(ftkb::enable_peer_access(c->cfg.device, segs[i].device));
+  return push_snapshot(c, segs, n, FTKB_MEM_DEVICE);
 }
 
 // A snapshot that exists as float32 (raw float32 file series: the reference widens them on the host, ndarray.hh read_binary_file):

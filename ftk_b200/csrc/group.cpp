@@ -112,10 +112,18 @@ int nbits_of(double res) {
 // spatial mode (chunk_timesteps == 0, 3D): device s holds planes [a0, a1] of every snapshot -- its corner planes plus the ghost
 // planes its stencils reach (the reference's spatial decomposition, regular_tracker.hh:126-149)
 struct Slab {
-  int device = 0, a0 = 0, a1 = 0;
+  int device = 0, c0 = 0, c1 = 0, a0 = 0, a1 = 0;
   ftkb_ctx *ctx = nullptr;
   std::vector<ftkb_point> points;
   ftkb_stats stats{};
+};
+
+// an event a device push records on a producer's stream, kept by the group for the next push
+struct ProducerEvent {
+  cudaEvent_t ev = nullptr;
+  int device = -1;
+  cudaError_t record(cudaStream_t stream, int dev);
+  void destroy();
 };
 
 struct ftkb_group {
@@ -127,7 +135,7 @@ struct ftkb_group {
   double running = DBL_MAX;                        // spatial mode: running minimum of min non-zero |v| over the whole array
   std::vector<std::unique_ptr<Worker>> workers;
   std::deque<std::unique_ptr<Chunk>> chunks;       // by index
-  std::mutex m;                                    // protects chunk state shared between workers
+  mutable std::mutex m;                            // protects chunk state shared between workers
   std::condition_variable cv;
   double saturating = 0.0;                         // a running minimum known to saturate the factor (0: not known yet)
   int npushed = 0, nadvanced = 0;
@@ -137,10 +145,10 @@ struct ftkb_group {
   std::vector<double> coords;
   cudaStream_t producer = nullptr;                 // ftkb_group_set_producer_stream: device pushes wait for the work queued there
   bool has_producer = false;
-  cudaEvent_t ev_producer = nullptr;               // recorded on `producer` by every device push (created on ev_device)
-  int ev_device = -1;
+  ProducerEvent ev_producer;                       // recorded on `producer` by every device push
+  std::vector<ProducerEvent> ev_pieces;            // piece pushes: one per producer stream the pieces name
   std::atomic<int> failed{FTKB_OK};
-  std::string error;
+  mutable std::string error;                       // (set by refusals of const queries too)
   ftkb_ctx *root = nullptr;
 
   Chunk *chunk(int c) {
@@ -232,6 +240,8 @@ extern "C" int ftkb_group_create(const ftkb_config *cfg, const int32_t *device_i
       sl.device = device_ids[s];
       const int c0 = glb + (int)((long long)nplanes * s / n_devices), c1 = glb + (int)((long long)nplanes * (s + 1) / n_devices) - 1;
       const int vtop = std::min(c1 + 1, gub);
+      sl.c0 = c0;
+      sl.c1 = c1;
       sl.a0 = s == 0 ? 0 : std::max(0, c0 - 2);
       sl.a1 = s == n_devices - 1 ? D - 1 : std::min(D - 1, vtop + 2);
       ftkb_config c = *cfg;
@@ -267,7 +277,8 @@ extern "C" void ftkb_group_destroy(ftkb_group *g) {
   for (auto &ch : g->chunks) if (ch->ctx) ftkb_destroy(ch->ctx);
   for (auto &sl : g->slabs) if (sl.ctx) ftkb_destroy(sl.ctx);
   if (g->root) ftkb_destroy(g->root);
-  if (g->ev_producer) { int cur = 0; cudaGetDevice(&cur); cudaSetDevice(g->ev_device); cudaEventDestroy(g->ev_producer); cudaSetDevice(cur); }
+  g->ev_producer.destroy();
+  for (auto &e : g->ev_pieces) e.destroy();
   delete g;
 }
 
@@ -368,14 +379,39 @@ static int push_layer(ftkb_group *g, std::function<int(ftkb_ctx *)> push, bool w
   return rc;
 }
 
-// Where a snapshot's arrays come from: host memory, or CUDA device memory on `device` (any device, in the group or not), every
-// copy ordered after `after` when it is set.  Either way the arrays are borrowed only until the push returns.
+// Where a snapshot's arrays come from: pieces that tile the whole array in plane order along its slowest axis (z in 3D, y in 2D),
+// in the whole array's frame.  Host memory comes as one piece; CUDA device memory as one piece or several, each on any device
+// (in the group or not), every copy from a piece ordered after its `after` when that is set.  Either way the arrays are borrowed
+// only until the push returns.
 struct Source {
   bool on_device = false;
-  int device = -1;
-  cudaEvent_t after = nullptr;
-  int push(ftkb_ctx *c, const double *S, const double *V, const double *J) const {
-    return on_device ? ftkb::push_snapshot_from(c, S, V, J, device, after) : ftkb_push_snapshot(c, S, V, J, FTKB_MEM_HOST);
+  std::vector<ftkb::Segment> pieces;
+  size_t plane = 0, n = 0;                     // doubles per plane of a scalar array; components per vertex of a vector
+  Source(const ftkb_config &cfg, bool device) : on_device(device), n((size_t)cfg.nd) {
+    plane = (size_t)cfg.dims[0] * (cfg.nd == 3 ? (size_t)cfg.dims[1] : 1);
+  }
+  int extent() const { return pieces.back().first + pieces.back().count; }
+  // the plan for a destination that holds planes [a0, a1]: one segment per intersecting piece, in the destination's frame
+  std::vector<ftkb::Segment> cut(int a0, int a1) const {
+    std::vector<ftkb::Segment> out;
+    for (const ftkb::Segment &p : pieces) {
+      const int lo = std::max(a0, p.first), hi = std::min(a1 + 1, p.first + p.count);
+      if (lo >= hi) continue;
+      const size_t o = plane * (size_t)(lo - p.first);
+      ftkb::Segment s = p;
+      s.first = lo - a0;
+      s.count = hi - lo;
+      s.scalar = p.scalar ? p.scalar + o : nullptr;
+      s.vector = p.vector ? p.vector + n * o : nullptr;
+      s.jacobian = p.jacobian ? p.jacobian + n * n * o : nullptr;
+      out.push_back(s);
+    }
+    return out;
+  }
+  int push(ftkb_ctx *c, int a0, int a1) const {
+    const std::vector<ftkb::Segment> segs = cut(a0, a1);
+    if (!on_device) return ftkb_push_snapshot(c, segs[0].scalar, segs[0].vector, segs[0].jacobian, FTKB_MEM_HOST);
+    return ftkb::push_segments(c, segs.data(), (int)segs.size());
   }
 };
 
@@ -384,53 +420,51 @@ struct Source {
 // So that layer is copied to the new chunk's device right away, into buffers of the group, and handed to the context later.
 struct Staged { double *S = nullptr, *V = nullptr, *J = nullptr; };
 
-static int push_snapshot(ftkb_group *g, const double *scalar, const double *vector, const double *jacobian, const Source src) {
-  if (g->spatial) {
+static int push_snapshot(ftkb_group *g, const Source src) {
+  const int last = src.extent() - 1;
+  if (g->spatial)
     // every device copies its planes (ghost planes included) over its own link, concurrently
-    const size_t plane = (size_t)g->cfg.dims[0] * (size_t)g->cfg.dims[1];
-    return spatial_push(g, [=](Slab &sl) {
-      const size_t o = plane * (size_t)sl.a0;
-      return src.push(sl.ctx, scalar ? scalar + o : nullptr, vector ? vector + 3 * o : nullptr, jacobian ? jacobian + 9 * o : nullptr);
-    });
-  }
+    return spatial_push(g, [=](Slab &sl) { return src.push(sl.ctx, sl.a0, sl.a1); });
   const int k = g->npushed;
   if (k % g->B != 0 || k == 0)
     // borrowed until return: wait for the copy
-    return push_layer(g, [=](ftkb_ctx *c) { return src.push(c, scalar, vector, jacobian); }, true);
+    return push_layer(g, [=](ftkb_ctx *c) { return src.push(c, 0, last); }, true);
   g->npushed++;
   const int c = k / g->B;
-  size_t nvert = 1;
-  for (int j = 0; j < g->cfg.nd; j++) nvert *= (size_t)g->cfg.dims[j];
-  const size_t n = (size_t)g->cfg.nd;
   std::shared_ptr<Done> d_halo(new Done()), d_stage(new Done());
-  post_push(g, c - 1, [=](ftkb_ctx *x) { return src.push(x, scalar, vector, jacobian); }, d_halo);   // halo of the chunk before
+  post_push(g, c - 1, [=](ftkb_ctx *x) { return src.push(x, 0, last); }, d_halo);   // halo of the chunk before
   Chunk *ch = g->chunk(c);
   Worker *w = g->workers[ch->index % g->workers.size()].get();
   std::shared_ptr<Staged> st(new Staged());
   w->post([=] {
     int rc = g->failed.load();
-    cudaStream_t s = nullptr;      // device source: the copies run here, after the producer
+    cudaStream_t s = nullptr;      // device source: the copies run here, after the producers
     auto ck = [&](cudaError_t e) {
       if (e == cudaSuccess || rc) return;
       cudaGetLastError();
       rc = e == cudaErrorMemoryAllocation ? FTKB_ERR_NOMEM : FTKB_ERR_CUDA;
       g->fail(rc, std::string("group: staging the first layer of a chunk failed: ") + cudaGetErrorString(e));
     };
-    auto up = [&](const double *from, size_t count, double **dst) {
-      if (!from || rc) return;
-      const size_t bytes = count * sizeof(double);
-      ck(cudaMalloc(dst, bytes));
-      if (rc) return;
-      if (!src.on_device) ck(cudaMemcpy(*dst, from, bytes, cudaMemcpyHostToDevice));
-      else if (src.device == ch->device) ck(cudaMemcpyAsync(*dst, from, bytes, cudaMemcpyDeviceToDevice, s));
-      else ck(cudaMemcpyPeerAsync(*dst, ch->device, from, src.device, bytes, s));
+    auto up = [&](const double *ftkb::Segment::*a, size_t per, double **dst) {
+      if (!(src.pieces[0].*a) || rc) return;
+      ck(cudaMalloc(dst, src.plane * per * (last + 1) * sizeof(double)));
+      for (const ftkb::Segment &p : src.pieces) {
+        if (rc) return;
+        double *to = *dst + src.plane * per * (size_t)p.first;
+        const size_t bytes = src.plane * per * (size_t)p.count * sizeof(double);
+        if (!src.on_device) ck(cudaMemcpy(to, p.*a, bytes, cudaMemcpyHostToDevice));
+        else if (p.device == ch->device) ck(cudaMemcpyAsync(to, p.*a, bytes, cudaMemcpyDeviceToDevice, s));
+        else ck(cudaMemcpyPeerAsync(to, ch->device, p.*a, p.device, bytes, s));
+      }
     };
-    if (!rc) ck(src.on_device ? ftkb::enable_peer_access(ch->device, src.device) : cudaSetDevice(ch->device));
+    if (!rc) ck(cudaSetDevice(ch->device));
     if (src.on_device) {
+      for (const ftkb::Segment &p : src.pieces) ck(ftkb::enable_peer_access(ch->device, p.device));
       ck(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
-      if (src.after) ck(cudaStreamWaitEvent(s, src.after, 0));
+      for (const ftkb::Segment &p : src.pieces)
+        if (p.after) ck(cudaStreamWaitEvent(s, p.after, 0));
     }
-    up(scalar, nvert, &st->S); up(vector, nvert * n, &st->V); up(jacobian, nvert * n * n, &st->J);
+    up(&ftkb::Segment::scalar, 1, &st->S); up(&ftkb::Segment::vector, src.n, &st->V); up(&ftkb::Segment::jacobian, src.n * src.n, &st->J);
     if (s) { ck(cudaStreamSynchronize(s)); cudaStreamDestroy(s); }
     d_stage->set(rc);
   });
@@ -448,10 +482,23 @@ static int push_snapshot(ftkb_group *g, const double *scalar, const double *vect
   return r1 ? r1 : r2;
 }
 
+// the whole array as one piece
+static Source whole(const ftkb_group *g, const double *scalar, const double *vector, const double *jacobian, bool on_device, int device,
+                    cudaEvent_t after) {
+  Source src(g->cfg, on_device);
+  ftkb::Segment p;
+  p.count = g->cfg.dims[g->cfg.nd - 1];
+  p.scalar = scalar; p.vector = vector; p.jacobian = jacobian;
+  p.device = device;
+  p.after = after;
+  src.pieces.push_back(p);
+  return src;
+}
+
 extern "C" int ftkb_group_push_snapshot(ftkb_group *g, const double *scalar, const double *vector, const double *jacobian) {
   if (!g) return FTKB_ERR_INVALID;
   if (g->failed.load()) return g->failed.load();
-  return push_snapshot(g, scalar, vector, jacobian, Source());
+  return push_snapshot(g, whole(g, scalar, vector, jacobian, false, -1, nullptr));
 }
 
 extern "C" int ftkb_group_set_producer_stream(ftkb_group *g, void *stream, int enable) {
@@ -461,39 +508,148 @@ extern "C" int ftkb_group_set_producer_stream(ftkb_group *g, void *stream, int e
   return FTKB_OK;
 }
 
+// The checks a device push makes of its arrays (the whole snapshot, or one piece of it): every non-null array is CUDA device
+// memory, 8-byte aligned, and on the same device as the others, which goes to *device.  Returns what is wrong, or "".
+static std::string device_of(const double *const arrays[3], int *device) {
+  static const char *const names[3] = {"scalar", "vector", "jacobian"};
+  *device = -1;
+  for (int i = 0; i < 3; i++) {
+    if (!arrays[i]) continue;
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, arrays[i]) != cudaSuccess) { cudaGetLastError(); a.type = cudaMemoryTypeUnregistered; }
+    if (a.type != cudaMemoryTypeDevice) return std::string("the ") + names[i] + " array is not CUDA device memory (host, unregistered and managed memory are refused)";
+    if ((uintptr_t)arrays[i] % 8 != 0) return std::string("the ") + names[i] + " array is not 8-byte aligned";
+    if (*device >= 0 && a.device != *device) return std::string("the ") + names[i] + " array is on another device than the arrays before it";
+    *device = a.device;
+  }
+  return *device < 0 ? "no array was passed" : "";
+}
+
+// Records `ev` on `stream`, which lives on `dev` (NULL: the legacy default stream of `dev`), creating it there, or again when
+// the event it kept from an earlier push is on another device.
+cudaError_t ProducerEvent::record(cudaStream_t stream, int dev) {
+  int cur = 0;
+  cudaError_t e = cudaGetDevice(&cur);
+  if (!e) e = cudaSetDevice(dev);
+  if (!e && ev && device != dev) { e = cudaEventDestroy(ev); ev = nullptr; }
+  if (!e && !ev && !(e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming))) device = dev;
+  if (!e) e = cudaEventRecord(ev, stream);
+  cudaSetDevice(cur);
+  if (e) cudaGetLastError();
+  return e;
+}
+
+void ProducerEvent::destroy() {
+  if (!ev) return;
+  int cur = 0;
+  cudaGetDevice(&cur);
+  cudaSetDevice(device);
+  cudaEventDestroy(ev);
+  cudaSetDevice(cur);
+  ev = nullptr;
+}
+
 extern "C" int ftkb_group_push_snapshot_device(ftkb_group *g, const double *scalar, const double *vector, const double *jacobian) {
   if (!g) return FTKB_ERR_INVALID;
   if (g->failed.load()) return g->failed.load();
   // a rejected push leaves the group as it was: the caller may push a valid snapshot next
   auto reject = [g](const std::string &msg) { std::lock_guard<std::mutex> lk(g->m); g->error = "push_snapshot_device: " + msg; return FTKB_ERR_INVALID; };
-  Source src;
-  src.on_device = true;
   const double *arrays[3] = {scalar, vector, jacobian};
-  const char *names[3] = {"scalar", "vector", "jacobian"};
-  for (int i = 0; i < 3; i++) {
-    if (!arrays[i]) continue;
-    cudaPointerAttributes a{};
-    if (cudaPointerGetAttributes(&a, arrays[i]) != cudaSuccess) { cudaGetLastError(); a.type = cudaMemoryTypeUnregistered; }
-    if (a.type != cudaMemoryTypeDevice) return reject(std::string("the ") + names[i] + " array is not CUDA device memory (host, unregistered and managed memory are refused)");
-    if ((uintptr_t)arrays[i] % 8 != 0) return reject(std::string("the ") + names[i] + " array is not 8-byte aligned");
-    if (src.device >= 0 && a.device != src.device) return reject(std::string("the ") + names[i] + " array is on another device than the arrays before it");
-    src.device = a.device;
-  }
-  if (src.device < 0) return reject("no array was passed");
+  int device = -1;
+  const std::string why = device_of(arrays, &device);
+  if (!why.empty()) return reject(why);
+  cudaEvent_t after = nullptr;
   if (g->has_producer) {
-    // one event is enough: this push returns only after every copy that waits for it has completed
-    int dev = src.device, cur = 0;
-    if (g->producer && cudaStreamGetDevice(g->producer, &dev) != cudaSuccess) { cudaGetLastError(); return reject("the producer stream is not a valid CUDA stream"); }
-    cudaError_t e = cudaGetDevice(&cur);
-    if (!e) e = cudaSetDevice(dev);           // (the legacy default stream, producer = NULL, is the source device's)
-    if (!e && g->ev_producer && g->ev_device != dev) { e = cudaEventDestroy(g->ev_producer); g->ev_producer = nullptr; }
-    if (!e && !g->ev_producer && !(e = cudaEventCreateWithFlags(&g->ev_producer, cudaEventDisableTiming))) g->ev_device = dev;
-    if (!e) e = cudaEventRecord(g->ev_producer, g->producer);
-    cudaSetDevice(cur);
-    if (e) { cudaGetLastError(); std::lock_guard<std::mutex> lk(g->m); g->error = std::string("push_snapshot_device: producer event: ") + cudaGetErrorString(e); return FTKB_ERR_CUDA; }
-    src.after = g->ev_producer;
+    // one event is enough: this push returns only after every copy that waits for it has completed.  The stream may live on
+    // another device than the arrays: `device` stays the arrays' own, the source of every copy.
+    int stream_device = device;
+    if (g->producer && cudaStreamGetDevice(g->producer, &stream_device) != cudaSuccess) { cudaGetLastError(); return reject("the producer stream is not a valid CUDA stream"); }
+    const cudaError_t e = g->ev_producer.record(g->producer, stream_device);
+    if (e) { std::lock_guard<std::mutex> lk(g->m); g->error = std::string("push_snapshot_device: producer event: ") + cudaGetErrorString(e); return FTKB_ERR_CUDA; }
+    after = g->ev_producer.ev;
   }
-  return push_snapshot(g, scalar, vector, jacobian, src);
+  return push_snapshot(g, whole(g, scalar, vector, jacobian, true, device, after));
+}
+
+extern "C" int ftkb_group_push_pieces_device(ftkb_group *g, const ftkb_piece *pieces, int32_t n) {
+  if (!g) return FTKB_ERR_INVALID;
+  if (g->failed.load()) return g->failed.load();
+  // everything is checked before anything is enqueued: a rejected push leaves the group as it was
+  auto reject = [g](const std::string &msg) { std::lock_guard<std::mutex> lk(g->m); g->error = "push_pieces_device: " + msg; return FTKB_ERR_INVALID; };
+  if (!pieces || n < 1) return reject("no pieces were passed (n = " + std::to_string(n) + ")");
+  const ftkb_config &cfg = g->cfg;
+  const long long extent = cfg.dims[cfg.nd - 1];
+  const char *axis = cfg.nd == 3 ? "z plane" : "y row";
+  Source src(cfg, true);
+  std::vector<int> stream_devices;         // the device of every piece's stream (NULL: the legacy stream of the piece's device)
+  long long next = 0;
+  for (int i = 0; i < n; i++) {
+    const ftkb_piece &p = pieces[i];
+    const std::string who = "piece " + std::to_string(i) + ": ";
+    if (p.count < 1) return reject(who + "count is " + std::to_string(p.count) + " (a piece holds at least one " + axis + ")");
+    if (p.first != next)
+      return reject(who + "starts at " + axis + " " + std::to_string(p.first) + " where " + std::to_string(next) + " was expected (" +
+                    (p.first > next ? "a gap" : "an overlap, or pieces out of order") + "; pieces tile the array in order)");
+    if (next + p.count > extent)
+      return reject(who + "ends at " + axis + " " + std::to_string(next + p.count) + ", past the array's " + std::to_string(extent));
+    next += p.count;
+    const double *arrays[3] = {p.scalar, p.vector, p.jacobian}, *first[3] = {pieces[0].scalar, pieces[0].vector, pieces[0].jacobian};
+    static const char *const names[3] = {"scalar", "vector", "jacobian"};
+    for (int a = 0; a < 3; a++)
+      if (!arrays[a] != !first[a])
+        return reject(who + (arrays[a] ? "passes a " : "lacks the ") + names[a] + " array" + (arrays[a] ? " that piece 0 lacks" : " that piece 0 passes") +
+                      " (every piece passes the same arrays)");
+    int device = -1;
+    const std::string why = device_of(arrays, &device);
+    if (!why.empty()) return reject(who + why);
+    int stream_device = device;
+    if (p.has_stream && p.stream && cudaStreamGetDevice(reinterpret_cast<cudaStream_t>(p.stream), &stream_device) != cudaSuccess) {
+      cudaGetLastError();
+      return reject(who + "its stream is not a valid CUDA stream");
+    }
+    ftkb::Segment s;
+    s.first = p.first; s.count = p.count;
+    s.scalar = p.scalar; s.vector = p.vector; s.jacobian = p.jacobian;
+    s.device = device;
+    src.pieces.push_back(s);
+    stream_devices.push_back(stream_device);
+  }
+  if (next != extent)
+    return reject("piece " + std::to_string(n - 1) + ": the pieces end at " + axis + " " + std::to_string(next) + ", the array has " + std::to_string(extent));
+  const ftkb_piece &p0 = pieces[0];
+  if ((cfg.scalar_source == FTKB_SOURCE_GIVEN && !p0.scalar) || (cfg.vector_source == FTKB_SOURCE_DERIVED && !p0.vector && !p0.scalar))
+    return reject("piece 0: lacks the scalar array, which the configuration's sources need");
+  if (cfg.vector_source == FTKB_SOURCE_GIVEN && !p0.vector) return reject("piece 0: lacks the vector array, which the configuration's sources need");
+  if (cfg.jacobian_source == FTKB_SOURCE_GIVEN && !p0.jacobian) return reject("piece 0: lacks the jacobian array, which the configuration's sources need");
+  // one event per producer stream named by the pieces (pieces written by the same stream share it), kept for the next push:
+  // enough for the same reason as ftkb_group_set_producer_stream's single event
+  std::vector<std::pair<cudaStream_t, int>> streams;
+  for (int i = 0; i < n; i++) {
+    if (!pieces[i].has_stream) continue;
+    const std::pair<cudaStream_t, int> key(reinterpret_cast<cudaStream_t>(pieces[i].stream), stream_devices[i]);
+    size_t e = std::find(streams.begin(), streams.end(), key) - streams.begin();
+    if (e == streams.size()) {
+      streams.push_back(key);
+      if (g->ev_pieces.size() < streams.size()) g->ev_pieces.emplace_back();
+      const cudaError_t r = g->ev_pieces[e].record(key.first, key.second);
+      if (r) { std::lock_guard<std::mutex> lk(g->m); g->error = "push_pieces_device: piece " + std::to_string(i) + ": producer event: " + cudaGetErrorString(r); return FTKB_ERR_CUDA; }
+    }
+    src.pieces[i].after = g->ev_pieces[e].ev;
+  }
+  return push_snapshot(g, src);
+}
+
+extern "C" int ftkb_group_get_slab(const ftkb_group *g, int32_t s, int32_t planes[4]) {
+  if (!g || !planes) return FTKB_ERR_INVALID;
+  if (!g->spatial || s < 0 || s >= (int32_t)g->slabs.size()) {
+    std::lock_guard<std::mutex> lk(g->m);
+    g->error = !g->spatial ? "get_slab: the group runs time chunks, not z-slabs"
+                           : "get_slab: slab " + std::to_string(s) + " does not exist (the group has " + std::to_string(g->slabs.size()) + ")";
+    return FTKB_ERR_INVALID;
+  }
+  const Slab &sl = g->slabs[s];
+  planes[0] = sl.c0; planes[1] = sl.c1; planes[2] = sl.a0; planes[3] = sl.a1;
+  return FTKB_OK;
 }
 
 extern "C" int ftkb_group_push_synthetic(ftkb_group *g, int kind, const double *params, int nparams, double t) {

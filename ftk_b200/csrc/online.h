@@ -72,9 +72,19 @@ class OnlineTracer {
 // context replays the grow steps of the chunks or slabs that swept for it (group.cpp)
 int grow_imported(ftkb_ctx *c, uint64_t end);
 
-// (context.cpp) ftkb_push_snapshot(c, .., FTKB_MEM_DEVICE) for device arrays on any device `src_device` (a peer copy when it is not
-// the context's own), every copy ordered after `after` unless it is null: how a device group pulls a device snapshot (group.cpp)
-int push_snapshot_from(ftkb_ctx *c, const double *scalar, const double *vector, const double *jacobian, int src_device, cudaEvent_t after);
+// One source of a layer's planes [first, first + count) along the slowest axis (z in 3D, y in 2D) of the context's array: the
+// arrays start at plane `first` and live on `device`; every copy from them waits for `after` unless it is null.
+struct Segment {
+  int first = 0, count = 0;
+  const double *scalar = nullptr, *vector = nullptr, *jacobian = nullptr;
+  int device = 0;
+  cudaEvent_t after = nullptr;
+};
+// (context.cpp) ftkb_push_snapshot(c, .., FTKB_MEM_DEVICE) for a layer assembled from device segments on any devices, which tile
+// the context's array in plane order and all pass the same arrays: one copy per (segment, array), a peer copy when the segment
+// is on another device than the context's.  How a device group feeds its contexts from a device snapshot (one segment) or from
+// snapshot pieces (group.cpp); ftkb_push_snapshot is the one-segment case for its own memory kinds.
+int push_segments(ftkb_ctx *c, const Segment *segs, int n);
 // (context.cpp) lets `device` read `peer`'s memory where the hardware allows it, once per pair; makes `device` current
 cudaError_t enable_peer_access(int device, int peer);
 

@@ -10,6 +10,8 @@ takes make_tracker's forms, for the whole array.
 Snapshots are numpy arrays (host memory) or device arrays -- torch CUDA tensors, or anything with __cuda_array_interface__ --
 on any visible device, one of the group's or not: every device then copies what it needs from the source device (peer copies
 over NVLink), ordered after torch's current stream on the tensor's device.  Either kind is consumed before the push returns.
+A producer decomposed over several GPUs pushes its pieces as they are (push_field_data_snapshot_pieces): every device then
+copies only the planes it needs, from whichever pieces hold them; slab(s) tells where z-slab s needs planes.
 """
 import ctypes as C
 
@@ -114,6 +116,56 @@ class GroupTracker:
             self._check(L.lib().ftkb_group_push_snapshot_device(self._g, ptrs[0], ptrs[1], ptrs[2]))
         else:
             self._check(L.lib().ftkb_group_push_snapshot(self._g, ptrs[0], ptrs[1], ptrs[2]))
+
+    def push_field_data_snapshot_pieces(self, scalar=None, vector=None, jacobian=None):
+        """A snapshot in pieces along the slowest axis (z in 3D, y in 2D), the way a decomposed producer holds it: each argument
+        is a list of float64 device arrays (torch CUDA tensors or __cuda_array_interface__ objects), one per piece, in plane
+        order, each piece's arrays on one device (any visible one).  A piece's leading dimension is its plane count: shapes
+        (count, H, W) for a 3D scalar, (count, W) for a 2D one, with trailing (n,) or (n, n) for vector and Jacobian.  Every copy
+        from a torch tensor waits for torch's current stream on its device; other producers synchronise before pushing.  Copied
+        to every device that needs the planes before the call returns (ftkb_group_push_pieces_device)."""
+        n = self._nd
+        lists = [list(a) if a is not None else None for a in (scalar, vector, jacobian)]
+        given = [a for a in lists if a is not None]
+        if not given or any(len(a) != len(given[0]) for a in given):
+            raise ValueError("pass one array per piece for every array, the same number of pieces for each")
+        plane = tuple(reversed(self._dims))[1:]
+        pieces = (L.Piece * len(given[0]))()
+        first = 0
+        for i, p in enumerate(pieces):
+            count = None
+            for a, trailing, field in zip(lists, ((), (n,), (n, n)), ("scalar", "vector", "jacobian")):
+                if a is None:
+                    continue
+                x = a[i]
+                if x is None:       # (refused by the library: every piece passes the same arrays)
+                    continue
+                dp = _dev_ptr(x)
+                if dp is None:
+                    raise ValueError(f"piece {i}: the {field} array is not a device array")
+                shape = tuple(x.shape)
+                if len(shape) != 1 + len(plane) + len(trailing) or shape[1:] != plane + trailing or \
+                        (hasattr(x, "is_contiguous") and not x.is_contiguous()):
+                    raise ValueError(f"piece {i}: the {field} array has shape {shape}, expected (count,) + {plane + trailing}, contiguous")
+                if str(getattr(x, "dtype", "")) != "torch.float64" and getattr(x, "__cuda_array_interface__", {}).get("typestr") != "<f8":
+                    raise ValueError(f"piece {i}: device arrays must be float64")
+                if count is not None and shape[0] != count:
+                    raise ValueError(f"piece {i}: its arrays hold different numbers of planes")
+                count = shape[0]
+                setattr(p, field, dp)
+                if getattr(x, "is_cuda", False) and hasattr(x, "data_ptr"):
+                    import torch
+                    p.stream = int(torch.cuda.current_stream(x.device).cuda_stream)
+                    p.has_stream = 1
+            p.first, p.count = first, count or 0
+            first += count or 0
+        self._check(L.lib().ftkb_group_push_pieces_device(self._g, pieces, len(pieces)))
+
+    def slab(self, s):
+        """z-slab mode: (c0, c1, a0, a1), the corner planes slab s owns and the array planes it holds (ftkb_group_get_slab)"""
+        planes = (C.c_int32 * 4)()
+        self._check(L.lib().ftkb_group_get_slab(self._g, int(s), planes))
+        return tuple(planes)
 
     def _order_after_producer(self, arrays):
         """device inputs: every copy waits for torch's current stream on the tensor's device (ftkb_group_set_producer_stream);

@@ -417,6 +417,33 @@ class critical_point_tracker_regular {
     check(ftkb_push_snapshot(ctx_, s, v, j, dev ? FTKB_MEM_DEVICE : FTKB_MEM_HOST));
     points_valid_ = false;
   }
+  // A snapshot in pieces along the slowest axis (z in 3D, y in 2D), as a producer decomposed over several GPUs holds it: piece i
+  // is a device ndarray view (ndarray::wrap(p, shape, true), on any visible device) of planes [first[i], first[i] + its last
+  // dimension); an array not passed is an empty list.  Only on several devices (set_device_ids): every device copies the planes
+  // it needs from the pieces that hold them (ftkb_group_push_pieces_device).  The caller synchronises its producer first.
+  void push_field_data_snapshot_pieces(const std::vector<int> &first, const std::vector<ndarray<double>> &scalar,
+                                       const std::vector<ndarray<double>> &vector = {}, const std::vector<ndarray<double>> &jacobian = {}) {
+    need();
+    if (!group_) throw std::runtime_error("ftk_b200: snapshot pieces need a tracker on several devices (set_device_ids)");
+    std::vector<ftkb_piece> pieces(first.size(), ftkb_piece{});
+    for (auto *a : {&scalar, &vector, &jacobian})
+      if (!a->empty() && a->size() != first.size()) throw std::runtime_error("ftk_b200: pass one array per piece");
+    for (size_t i = 0; i < first.size(); i++) {
+      ftkb_piece &p = pieces[i];
+      p.first = first[i];
+      const ndarray<double> *arrays[3] = {scalar.empty() ? nullptr : &scalar[i], vector.empty() ? nullptr : &vector[i], jacobian.empty() ? nullptr : &jacobian[i]};
+      const double **ptrs[3] = {&p.scalar, &p.vector, &p.jacobian};
+      for (int k = 0; k < 3; k++) {
+        const ndarray<double> *a = arrays[k];
+        if (!a || a->empty()) continue;
+        if (!a->on_device()) throw std::runtime_error("ftk_b200: snapshot pieces are device arrays");
+        *ptrs[k] = a->data();
+        p.count = (int32_t)a->dim(a->nd() - 1);
+      }
+    }
+    gcheck(ftkb_group_push_pieces_device(group_, pieces.data(), (int32_t)pieces.size()));
+    points_valid_ = false;
+  }
   void push_scalar_field_snapshot(const ndarray<double> &scalar) { push_field_data_snapshot(scalar, ndarray<double>(), ndarray<double>()); }
   void push_vector_field_snapshot(const ndarray<double> &vector) { push_field_data_snapshot(ndarray<double>(), vector, ndarray<double>()); }
   // float32 host snapshots (raw float32 series; the reference's streams widen them on the host): they travel as float32 and are

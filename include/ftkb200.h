@@ -230,6 +230,12 @@ int ftkb_push_snapshot_remote(ftkb_ctx *, const double *scalar, const double *ve
  * ftkb_group_set_producer_stream names the stream (on its own device; NULL: the legacy default stream of the source device)
  * that writes those arrays: every later device push records an event there and every copy waits for it.  Without it the caller
  * synchronises the producer before pushing.
+ * ftkb_group_push_pieces_device takes a snapshot that lives in PIECES, the way a simulation decomposed over several GPUs holds
+ * it: each piece is a contiguous range of planes along the slowest axis (z planes in 3D, y rows in 2D) in CUDA device memory
+ * on any visible device.  Every context assembles its layer from the pieces that intersect the planes it needs -- a z-slab its
+ * planes [a0, a1], ghost planes included; a chunk's context, the halo of the chunk before and the staged first layer of a new
+ * chunk the whole array -- with one copy per (context, intersecting piece, array), on the context's stream.  A producer that
+ * cuts its pieces at the slabs' array planes (ftkb_group_get_slab) sends only ghost planes from one device to another.
  *
  * Options, valid only before the first push (afterwards FTKB_ERR_INVALID):
  *   ftkb_group_set_coords                   ftkb_set_coords for the whole array: same modes and sizes, host data copied before
@@ -263,6 +269,27 @@ int ftkb_group_push_snapshot_device(ftkb_group *, const double *scalar, const do
 /* the group's counterpart of ftkb_set_producer_stream: every copy of a later device push waits for the work queued on
  * `stream` (on its own device) when the push is called; enable = 0 turns it off */
 int ftkb_group_set_producer_stream(ftkb_group *, void *cuda_stream, int enable);
+/* one piece of a snapshot: planes [first, first + count) of the slowest axis (z in 3D, y in 2D), each array holding exactly
+ * those planes (count * H * W scalars in 3D, count * W in 2D; times n or n*n for the vector and Jacobian arrays) */
+typedef struct ftkb_piece {
+  const double *scalar, *vector, *jacobian; /* device memory, all on one device; NULL rules as ftkb_group_push_snapshot */
+  int32_t first, count;                     /* planes [first, first + count) of the slowest axis (z in 3D, y in 2D) */
+  void *stream;                             /* stream on the piece's device that writes it (NULL: that device's legacy stream) */
+  int32_t has_stream;                       /* 1: every copy from this piece waits for the work queued on `stream` at the push */
+  int32_t reserved;
+} ftkb_piece;
+/* a snapshot as n >= 1 pieces that tile the array in order: piece 0 starts at plane 0, each piece starts where the one before
+ * ends, every count >= 1, and the counts add up to the extent (D in 3D, H in 2D).  Every piece passes the same arrays, which
+ * meet the configuration's sources; every array is CUDA device memory, 8-byte aligned, and one piece's arrays are on one device
+ * (several pieces may share a device).  Otherwise FTKB_ERR_INVALID, with a message that names the piece and the array, before
+ * anything is enqueued: the group stays as it was.  Ordering is per piece: the push records one event of the group's on every
+ * stream the pieces name (has_stream = 1) and every copy from those pieces waits for it; ftkb_group_set_producer_stream does
+ * not apply to piece pushes.  Copied: the call returns when every device holds its copy, so the caller may overwrite or free
+ * the pieces right away.  Piece, whole-device and host pushes may alternate in one series. */
+int ftkb_group_push_pieces_device(ftkb_group *, const ftkb_piece *pieces, int32_t n);
+/* z-slab mode: corner planes [c0, c1] slab s owns and array planes [a0, a1] it holds, so that a producer can cut its pieces
+ * where only ghost planes cross devices; FTKB_ERR_INVALID in time-chunk mode */
+int ftkb_group_get_slab(const ftkb_group *, int32_t s, int32_t planes[4]);
 int ftkb_group_push_synthetic(ftkb_group *, int kind, const double *params, int nparams, double t);
 int ftkb_group_advance_timestep(ftkb_group *);
 int ftkb_group_update_timestep(ftkb_group *);
