@@ -43,6 +43,17 @@ struct Layer {
   bool cells_foreign = false;    // the cells belong to a peer process (remote snapshot) or were exported: never recycled
 };
 
+// The scans a context's input can still use.  Each input has a fast scan and a slower one that takes every input; a context
+// starts at the fastest its configuration and the environment switches allow and only ever moves down (fall_back).
+enum class Scans : uint8_t {
+  keys2d,       // 2D scalar input: high-word key build kernel
+  f32_2d,       //   fp32-range build kernel: NaN / Inf / >= 2^1000 scalars, FTKB_SCAN2D=f32
+  fused3d,      // 3D scalar input: gradient fused into the TMA-staged range-cell scan
+  gradient3d,   //   gradient materialised: odd W, robust detection off, NaN / Inf / >= 2^1000, no TMA descriptor, FTKB_SCAN3D=plain
+  vcells,       // vector input: range-cell scan, each layer streamed once
+  twolayer,     //   both layers re-read every step + resolution pass: |v| >= 2^1000 / Inf, 3D odd W or robust detection off, FTKB_VSCAN=twolayer
+};
+
 }  // namespace
 
 // host arrays that are filled completely right after they are sized (by a device-to-host copy or a loop): no value-initialisation
@@ -79,14 +90,10 @@ struct ftkb_ctx {
   int nbits = 0;
   int next_slot = 0;
   int sm_count = 148;
-  bool cellsV = true;            // vector input (field GIVEN): each layer is streamed once and keeps its range cells;
-                                 // FTKB_VSCAN=twolayer re-reads both layers every step and runs the resolution pass
-  bool keys2d = true;            // 2D scalar build kernel keeps high-word keys of the differences (no fp64->fp32 conversions);
-                                 // FTKB_SCAN2D=f32 (or a poisoned layer: NaN / Inf / >= 2^1000) selects the fp32-range build kernel
+  Scans scans = Scans::keys2d;
   std::vector<uint4 *> freeCells;
   std::vector<uint4 *> exportedCells;   // handed to a peer process (ftkb_export_layer_cells): freed at destroy only
   size_t ncells = 0;             // cells per layer (fixed by the dims)
-  bool fused3d = false;          // 3D scalar input: gradient fused into the scan (TMA-staged); FTKB_SCAN3D=plain materialises the gradient instead
 
   // device scalars: [0..7] per-layer resolution bits, [8] worklist count, [9] point count, [10] unique count, [11] poison,
   // [12] the second worklist counter (deferred steps alternate), [13] ticket of the test kernel's blocks, [14] second poison flag
@@ -339,15 +346,15 @@ extern "C" int ftkb_create(const ftkb_config *cfg, ftkb_ctx **out) {
   c->slab = cfg->slab_global_dim != 0;
   c->sm_count = prop.multiProcessorCount > 0 ? prop.multiProcessorCount : 148;
   {
-    // the fused 3D scan needs TMA-compatible rows (W even) and the exact early-out (robust detection on)
-    const char *e = std::getenv("FTKB_SCAN3D");
-    c->fused3d = n == 3 && cfg->vector_source == FTKB_SOURCE_DERIVED && cfg->robust_detection && cfg->dims[0] % 2 == 0 &&
-                 !(e && std::string(e) == "plain");
-    const char *ev = std::getenv("FTKB_VSCAN");
-    c->cellsV = cfg->vector_source == FTKB_SOURCE_GIVEN && !(n == 3 && !cfg->robust_detection) && (n == 2 || cfg->dims[0] % 2 == 0) &&
-                !(ev && std::string(ev) == "twolayer");
-    const char *e2 = std::getenv("FTKB_SCAN2D");
-    c->keys2d = !(e2 && std::string(e2) == "f32");
+    // the 3D range-cell scans need TMA-compatible rows (W even) and the exact early-out (robust detection on)
+    auto env_is = [](const char *name, const char *value) { const char *e = std::getenv(name); return e && std::string(e) == value; };
+    if (cfg->vector_source == FTKB_SOURCE_GIVEN)
+      c->scans = (n == 2 || (cfg->robust_detection && cfg->dims[0] % 2 == 0)) && !env_is("FTKB_VSCAN", "twolayer") ? Scans::vcells : Scans::twolayer;
+    else if (n == 3)
+      c->scans = cfg->vector_source == FTKB_SOURCE_DERIVED && cfg->robust_detection && cfg->dims[0] % 2 == 0 && !env_is("FTKB_SCAN3D", "plain")
+                     ? Scans::fused3d : Scans::gradient3d;
+    else
+      c->scans = env_is("FTKB_SCAN2D", "f32") ? Scans::f32_2d : Scans::keys2d;
   }
   c->n = n;
   c->nvert = (size_t)cfg->dims[0] * cfg->dims[1] * (n == 3 ? cfg->dims[2] : 1);
@@ -429,21 +436,27 @@ static int queue_resolution(ftkb_ctx *c, Layer &l, bool fused_in_gradient) {
   return check_launch(c, "resolution");
 }
 
+static bool aligned16(const void *a) { return (uintptr_t)a % 16 == 0; }
+
+// the sweep derives the vector field from layer l0's scalars on the fly (SweepParams::fused)
+static bool derives_vectors(const ftkb_ctx *c, const Layer &l0) {
+  return !l0.V && l0.S && c->cfg.vector_source == FTKB_SOURCE_DERIVED && (c->n == 2 || c->scans == Scans::fused3d);
+}
+
+// the scan derives the layer's gradient on the fly, or streams its vectors into range cells, and folds the layer's min
+// non-zero |v| into that pass
+static bool scan_resolves(const ftkb_ctx *c, const Layer &l) {
+  return l.V ? c->scans == Scans::vcells && aligned16(l.V) : derives_vectors(c, l) && (c->n == 2 || aligned16(l.S));
+}
+
 static int derive_layer(ftkb_ctx *c, Layer &l) {
   // slot <- all ones: above the bit pattern of every finite double, so the kernels' atomicMin on the
   // bit patterns of |v| works unchanged and "nothing found" reads back as DBL_MAX (slot_value).
   // Layers whose resolution the scan produces (res_pending) only mark the host mirror: the sweep's one
   // host-to-device copy of the counter block resets the device slot (no separate memset per push).
   bool fused = false;
-  if (!l.V && c->cfg.vector_source == FTKB_SOURCE_DERIVED && l.S && (c->n == 2 || (c->fused3d && (uintptr_t)l.S % 16 == 0))) {
-    // the gradient is never materialised; the fused scan derives it on the fly and computes this
-    // layer's resolution during the first sweep that reads it
-    l.res_pending = true;
-    c->h_scalars[l.slot] = ~0ull;
-    return FTKB_OK;
-  }
-  if (l.V && c->cellsV && c->cfg.vector_source == FTKB_SOURCE_GIVEN && (uintptr_t)l.V % 16 == 0) {
-    // the range-cell scan streams this layer once and folds min non-zero |v| into that pass
+  if (scan_resolves(c, l)) {
+    // the first sweep that reads this layer computes its resolution
     l.res_pending = true;
     c->h_scalars[l.slot] = ~0ull;
     return FTKB_OK;
@@ -747,15 +760,27 @@ static void fill_sweep_geometry(const ftkb_ctx *c, SweepParams &p) {
     p.vmax[j] = p.ub[j];   // vertices outside the domain belong to no valid simplex: keep them out of the cube ranges
     p.voff[j] = 0; p.rank_lb[j] = p.lb[j]; p.rank_nc[j] = p.nc[j];
   }
-  // scalar build kernels: key filter of the layer's min non-zero |v| against the running minimum known now (kernels.h);
-  // gradient2D scales the differences by W - 1 / H - 1 (grad.hh:24-27), gradient3D halves them (grad.hh:140-144)
-  for (int j = 0; j < 3; j++)
-    p.res_thr[j] = res_threshold_key(c->resolution, c->n == 2 ? (double)(c->cfg.dims[j < 2 ? j : 0] - 1) : 0.5);
   if (c->slab) {           // a z-slab of a larger array: ranks / positions / corners in the whole lattice's frame
     p.voff[2] = c->cfg.slab_offset;
     p.rank_lb[2] = c->cfg.slab_global_lb;
     p.rank_nc[2] = c->cfg.slab_global_ub - c->cfg.slab_global_lb + 1;
   }
+}
+
+// scalar build kernels: key filter of the layer's min non-zero |v| against the running minimum known now (kernels.h);
+// gradient2D scales the differences by W - 1 / H - 1 (grad.hh:24-27), gradient3D halves them (grad.hh:140-144)
+static void set_key_filter(const ftkb_ctx *c, SweepParams &p) {
+  for (int j = 0; j < 3; j++)
+    p.res_thr[j] = res_threshold_key(c->resolution, c->n == 2 ? (double)(c->cfg.dims[j < 2 ? j : 0] - 1) : 0.5);
+}
+
+// quantisation factor 2^nbits and the fp32 thresholds of the scans' exclusion test
+static void set_factor(SweepParams &p, int nbits) {
+  p.nbits = nbits;
+  p.factor = (double)(uint64_t)(1 << nbits);
+  p.thrp_f = (float)((1.0 / p.factor) * (1.0 + 1.0 / 1048576.0));
+  p.thr2_f = (float)(2.0 / p.factor);
+  p.lim_f = (float)(0.999 * 4.5e18 / (p.factor * p.factor));
 }
 
 // strips x row chunks of the fused 2D scan.  aligned: 16-byte aligned rows, range-cell kernels on CTA tiles of 7 x 62 corner
@@ -833,8 +858,20 @@ static int materialise_gradient(ftkb_ctx *c, Layer &l) {
   return check_launch(c, "gradient");
 }
 
-static int abandon_fused3d(ftkb_ctx *c) {
-  c->fused3d = false;
+// The context's input moves down to its slower scan for good (Scans): values the float keys cannot order (NaN, Inf,
+// |v| >= 2^1000), no TMA descriptor, or 3D layers of both forms.  Every layer's range cells are dropped, those that came from a
+// peer included; in 3D the resident layers get their gradient materialised instead.
+static int fall_back(ftkb_ctx *c) {
+  switch (c->scans) {
+    case Scans::keys2d: c->scans = Scans::f32_2d; break;
+    case Scans::fused3d: c->scans = Scans::gradient3d; break;
+    case Scans::vcells: c->scans = Scans::twolayer; break;
+    default: break;
+  }
+  if (c->scans != Scans::gradient3d) {
+    for (Layer &l : c->layers) l.cells_valid = false;
+    return FTKB_OK;
+  }
   for (Layer &l : c->layers) {
     const int rc = materialise_gradient(c, l);
     if (rc) return rc;
@@ -844,106 +881,130 @@ static int abandon_fused3d(ftkb_ctx *c) {
 }
 
 static bool rows_aligned16(const ftkb_ctx *c, const double *a, const double *b) {
-  return (c->cfg.dims[0] % 2 == 0) && ((uintptr_t)a % 16 == 0) && (!b || (uintptr_t)b % 16 == 0);
+  return (c->cfg.dims[0] % 2 == 0) && aligned16(a) && (!b || aligned16(b));
 }
 
-// resolution of a layer whose vector field is derived on the fly, outside a sweep (time-slab exchange)
+// The scan of a sweep over layers l0, l1 (l1 == l0 without a next layer).  launch is the kernel family's launcher; cells: a
+// range-cell scan, whose layers keep their cells from one step to the next.
+struct Scan {
+  void (*launch)(const SweepParams &, cudaStream_t);
+  bool cells;
+};
+
+// Chooses the scan from the context's Scans and the two layers, and sets p.fused, p.keys2d, the TMA descriptors and the grid
+// decomposition.  Choices that depend on the layers hold for this sweep only: misaligned 2D rows take the register kernel,
+// a misaligned vector layer the two-layer scan.  launch == nullptr: the fused 3D scan has no TMA descriptor (driver entry
+// point or alignment) for a layer, and the context has to fall back before it sweeps.
+static Scan choose_scan(const ftkb_ctx *c, const Layer &l0, const Layer &l1, SweepParams &p) {
+  p.fused = derives_vectors(c, l0);
+  if (p.fused && c->n == 3) {
+    if (!encode_scalar_tmap3d(l0.S, p.W, p.H, p.D, &p.tmap[0]) || !encode_scalar_tmap3d(l1.S, p.W, p.H, p.D, &p.tmap[1])) return {nullptr, false};
+    fused3d_decomposition(c, p);
+    return {launch_scan3d_cells, true};
+  }
+  if (p.fused) {
+    const bool aligned = rows_aligned16(c, l0.S, l1.S);    // the range-cell kernels need 16-byte aligned rows
+    fused2d_decomposition(c, p, aligned);
+    p.keys2d = c->scans == Scans::keys2d;
+    return {aligned ? launch_scan2d_cells : launch_scan, aligned};
+  }
+  if (l0.V && l1.V && scan_resolves(c, l0) && scan_resolves(c, l1)) {
+    vcells_decomposition(c, p);
+    return {launch_vscan_cells, true};
+  }
+  // two-layer scans of vector layers: strips of 31 corners x 64 rows (2D) / x 15 rows x 32 planes (3D)
+  p.nsx = (p.nc[0] + 30) / 31;
+  if (c->n == 2) {
+    p.rows = 64;
+    p.nsy = (p.nc[1] + p.rows - 1) / p.rows;
+    p.nsz = 1;
+  } else {
+    p.rows = 32;
+    p.nsy = (p.nc[1] + 14) / 15;
+    p.nsz = (p.nc[2] + p.rows - 1) / p.rows;
+  }
+  return {launch_scan, false};
+}
+
+// what every sweep over l0, l1 shares (the quantisation factor, the key filter and the buffers aside), and its scan
+static Scan sweep_setup(const ftkb_ctx *c, const Layer &l0, const Layer &l1, bool has_next, SweepParams &p) {
+  fill_sweep_geometry(c, p);
+  p.t = c->current_timestep;
+  p.has_next = has_next;
+  p.no_filter = (c->n == 3 && !c->cfg.robust_detection);
+  p.scalar_source = l0.S ? c->cfg.scalar_source : FTKB_SOURCE_NONE;
+  p.jacobian_source = c->cfg.jacobian_source;
+  p.jacobian_symmetric = c->cfg.jacobian_symmetric;
+  // 2D: jacobian2D<double,true> on the scalar path, <double,false> when the vector field was pushed
+  p.derived_symmetric = c->cfg.vector_source == FTKB_SOURCE_DERIVED;
+  p.robust = c->cfg.robust_detection;
+  p.compute_degrees = c->cfg.compute_degrees;
+  p.use_type_filter = c->cfg.use_type_filter;
+  p.type_filter = c->cfg.type_filter;
+  p.L[0] = {l0.S, l0.V, l0.J};
+  p.L[1] = {l1.S, l1.V, l1.J};
+  p.poison = c->d_scalars + ftkb_ctx::SLOT_POISON;
+  p.wl_count = c->d_scalars + ftkb_ctx::SLOT_WL;
+  p.pt_count = c->d_scalars + ftkb_ctx::SLOT_PT;
+  p.ticket = c->d_scalars + ftkb_ctx::SLOT_TICKET;
+  return choose_scan(c, l0, l1, p);
+}
+
+// min non-zero |v| of a layer that no sweep has streamed yet, outside a sweep (time-slab halos, z-slab groups, vector layers
+// pushed further ahead than the sweep reads): the layer's own scan streams it once -- its range cells and min |v| -- and tests
+// no cube
 static int resolve_pending(ftkb_ctx *c, Layer &l) {
+  const bool vector_input = l.V != nullptr;
   c->primed = false;
   CK(cudaMemsetAsync(c->d_scalars + l.slot, 0xff, sizeof(unsigned long long), c->stream));   // (a pending layer's device slot is reset lazily)
-  if (l.V) {
-    if (c->cellsV && c->cfg.vector_source == FTKB_SOURCE_GIVEN && (uintptr_t)l.V % 16 == 0 && !l.cells_valid) {
-      // vector input: stream the layer once -- its range cells and min |v|; no cube is tested (the sweeps then read the cells)
-      SweepParams p{};
-      fill_sweep_geometry(c, p);
-      p.fused = 0;
-      p.has_next = 0;
-      p.nbits = c->nbits ? c->nbits : 8;
-      p.L[0].V = l.V; p.L[1].V = l.V;
-      p.res_slot[0] = c->d_scalars + l.slot;
-      p.poison = c->d_scalars + ftkb_ctx::SLOT_POISON;
-      p.wl_count = c->d_scalars + ftkb_ctx::SLOT_WL;
-      p.wl = c->d_wl; p.wl_cap = 0;
-      vcells_decomposition(c, p);
-      const int rc = ensure_cells(c, l, p);
-      if (rc) return rc;
-      CK(cudaMemsetAsync(p.poison, 0, sizeof(unsigned long long), c->stream));
-      p.sum_mode = SUM_BUILD; p.build_layer = 0; p.sum_out = l.cells;
-      launch_vscan_cells(p, c->stream);
-      c->stats.kernel_launches++;
-      CK(cudaMemcpyAsync(c->h_scalars + l.slot, c->d_scalars + l.slot, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
-      CK(cudaMemcpyAsync(c->h_scalars + ftkb_ctx::SLOT_POISON, p.poison, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
-      c->stats.d2h_bytes += 16;
-      const int rl = check_launch(c, "resolution (vector cells)");
-      if (rl) return rl;
-      CK(cudaStreamSynchronize(c->stream));
-      if (!c->h_scalars[ftkb_ctx::SLOT_POISON]) {
-        l.cells_valid = true;
-        l.res_pending = false;
-        return FTKB_OK;
-      }
-      // magnitudes the float keys cannot order: fall back to the plain pass (and the two-layer scans)
-      c->cellsV = false;
-      for (Layer &x : c->layers) x.cells_valid = false;
-      CK(cudaMemsetAsync(c->d_scalars + l.slot, 0xff, sizeof(unsigned long long), c->stream));
-    }
+  SweepParams p{};
+  const Scan s = sweep_setup(c, l, l, false, p);
+  if (!s.launch) return fall_back(c);        // the materialised gradient brings the layer's min |v|
+  if (vector_input && (!s.cells || l.cells_valid)) {
     l.res_pending = false;
     return queue_resolution(c, l, false);
   }
-  SweepParams p{};
-  fill_sweep_geometry(c, p);
-  p.lb[1] = 1; p.ub[1] = 0;           // empty domain: gradient + resolution only, no cube is tested
-  p.fused = 1;
-  p.has_next = 0;
-  p.thrp_f = 1.f; p.thr2_f = 1.f; p.lim_f = 0.f;
-  p.L[0].S = l.S; p.L[1].S = l.S;
+  set_key_filter(c, p);
+  p.keys2d = 0;                              // 2D: the fp32-range build, which orders every value (no poison flag to read back)
+  p.nbits = vector_input ? (c->nbits ? c->nbits : 8) : (c->n == 3 ? 8 : 0);
+  if (!vector_input) { p.thrp_f = 1.f; p.thr2_f = 1.f; p.lim_f = 0.f; }
   p.res_slot[0] = c->d_scalars + l.slot;
-  p.wl_count = c->d_scalars + ftkb_ctx::SLOT_WL;
   p.wl = c->d_wl; p.wl_cap = 0;
-  if (c->n == 3) {
-    p.nbits = 8;
-    p.poison = c->d_scalars + ftkb_ctx::SLOT_POISON;
-    if (!encode_scalar_tmap3d(l.S, p.W, p.H, p.D, &p.tmap[0])) { c->fused3d = false; return materialise_gradient(c, l); }
-    p.tmap[1] = p.tmap[0];
-    CK(cudaMemsetAsync(p.poison, 0, sizeof(unsigned long long), c->stream));
-    fused3d_decomposition(c, p);
-    // stream the layer once: its range cells (with the real domain masks) and min |v|; no cube is tested
-    fill_sweep_geometry(c, p);
-    int rc = ensure_cells(c, l, p);
+  if (s.cells) {
+    // the build keeps the real domain: the cells need its masks
+    const int rc = ensure_cells(c, l, p);
     if (rc) return rc;
     p.sum_mode = SUM_BUILD; p.build_layer = 0; p.sum_out = l.cells;
-    launch_scan3d_cells(p, c->stream);
-    l.cells_valid = true;
-    c->stats.kernel_launches++;
-    CK(cudaMemcpyAsync(c->h_scalars + l.slot, c->d_scalars + l.slot, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaMemcpyAsync(c->h_scalars + ftkb_ctx::SLOT_POISON, p.poison, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
-    c->stats.d2h_bytes += 16;
-    rc = check_launch(c, "resolution (fused 3D)");
-    if (rc) return rc;
-    CK(cudaStreamSynchronize(c->stream));
-    l.res_pending = false;
-    if (c->h_scalars[ftkb_ctx::SLOT_POISON]) return abandon_fused3d(c);
-    return FTKB_OK;
-  }
-  const bool aligned = rows_aligned16(c, l.S, nullptr);
-  fused2d_decomposition(c, p, aligned);
-  if (aligned) {
-    // stream the layer once: its range cells and min |v|; no cube is tested
-    fill_sweep_geometry(c, p);
-    int rc = ensure_cells(c, l, p);
-    if (rc) return rc;
-    p.sum_mode = SUM_BUILD; p.build_layer = 0; p.sum_out = l.cells;
-    launch_scan2d_cells(p, c->stream);
-    l.cells_valid = true;
   } else {
-    launch_scan(p, c->stream);
+    p.lb[1] = 1; p.ub[1] = 0;                // the register kernel over an empty domain: gradient and min |v| only
   }
+  const bool keyed = vector_input || c->n == 3;   // the key scans raise the poison flag
+  if (keyed) CK(cudaMemsetAsync(p.poison, 0, sizeof(unsigned long long), c->stream));
+  s.launch(p, c->stream);
   c->stats.kernel_launches++;
   CK(cudaMemcpyAsync(c->h_scalars + l.slot, c->d_scalars + l.slot, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
-  c->stats.d2h_bytes += 8;
+  if (keyed) CK(cudaMemcpyAsync(c->h_scalars + ftkb_ctx::SLOT_POISON, p.poison, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+  c->stats.d2h_bytes += keyed ? 16 : 8;
+  int rc = check_launch(c, "resolution (scan)");
+  if (rc) return rc;
+  if (!keyed) {
+    l.cells_valid = l.cells_valid || s.cells;
+    l.res_pending = false;
+    c->push_d2h_outstanding = true;
+    return FTKB_OK;
+  }
+  CK(cudaStreamSynchronize(c->stream));
+  if (!c->h_scalars[ftkb_ctx::SLOT_POISON]) {
+    l.cells_valid = true;
+    l.res_pending = false;
+    return FTKB_OK;
+  }
+  // values the float keys cannot order: a 3D scalar layer gets its gradient (and with it its min |v|), a vector layer the
+  // plain resolution pass
+  if ((rc = fall_back(c)) || !vector_input) return rc;
+  CK(cudaMemsetAsync(c->d_scalars + l.slot, 0xff, sizeof(unsigned long long), c->stream));
   l.res_pending = false;
-  c->push_d2h_outstanding = true;
-  return check_launch(c, "resolution (fused)");
+  return queue_resolution(c, l, false);
 }
 
 // ref: critical_point_tracker_{2d,3d}_regular::update_timestep (xl == NONE branch)
@@ -966,7 +1027,6 @@ static int grow_trajectories(ftkb_ctx *c, uint64_t end) {
   const size_t per = 8 + 4 * 9 + 1;
   if (n && c->grow_stage_cap < per * n) {
     if (c->grow_stage) cudaFreeHost(c->grow_stage);
-  for (ftkb_point *q : c->retired_pts) cudaFree(q);
     c->grow_stage = nullptr; c->grow_stage_cap = 0;
     const size_t want = per * (n + n / 2 + 1024);
     if (cudaMallocHost(&c->grow_stage, want) != cudaSuccess) { cudaGetLastError(); return fail(c, FTKB_ERR_NOMEM, "streaming grow step: out of page-locked memory"); }
@@ -1043,7 +1103,6 @@ extern "C" int ftkb_set_streaming_trajectories(ftkb_ctx *c, int enable) {
 
 // ---- deferred steps: confirmation, replay ------------------------------------------------------------------------
 static int update_impl(ftkb_ctx *c, bool allow_defer);
-static int abandon_fused3d(ftkb_ctx *c);
 
 static void absorb_resolutions(ftkb_ctx *c, const ftkb_ctx::Pending &pd) {
   const volatile unsigned long long *r = c->h_ring + 8 * pd.ring;
@@ -1076,16 +1135,8 @@ static int replay(ftkb_ctx *c, bool poison) {
   c->sorted = false;
   c->traced = false;
   if (poison) {
-    if (c->cfg.vector_source == FTKB_SOURCE_GIVEN) {
-      c->cellsV = false;
-      for (Layer &l : c->layers) l.cells_valid = false;
-    } else if (c->n == 3) {
-      const int rc = abandon_fused3d(c);
-      if (rc) return rc;
-    } else {
-      c->keys2d = false;
-      for (Layer &l : c->layers) l.cells_valid = false;
-    }
+    const int rc = fall_back(c);
+    if (rc) return rc;
   }
   c->stats.sweeps_repeated += pops.size();
   for (size_t i = 0; i < pops.size(); i++) {
@@ -1201,273 +1252,141 @@ extern "C" int ftkb_update_timestep(ftkb_ctx *c) {
   return update_impl(c, c->defer);
 }
 
-static int update_impl(ftkb_ctx *c, bool allow_defer) {
-  if (c->layers.empty()) return fail(c, FTKB_ERR_INVALID, "update_timestep: no snapshot has been pushed");
-  CK(cudaSetDevice(c->cfg.device));
-  bool may_defer = allow_defer && !c->streaming && !c->push_d2h_outstanding;
-  if (!may_defer) { const int rc = drain(c); if (rc) return rc; }
-  if (c->n == 3 && c->fused3d && c->cfg.vector_source == FTKB_SOURCE_DERIVED) {
-    // a layer whose pointer TMA cannot take was materialised at push time: the sweep cannot mix the two forms
-    bool anyV = false, anyS = false;
-    for (const Layer &l : c->layers) { anyV = anyV || l.V; anyS = anyS || (!l.V && l.S); }
-    if (anyV && anyS) c->fused3d = false;
-  }
-  if (c->n == 3 && !c->fused3d) {
-    // layers pushed while the fused 3D path was still on (it was abandoned since): materialise their gradient
-    bool any = false;
-    for (Layer &l : c->layers)
-      if (!l.V && l.S && c->cfg.vector_source == FTKB_SOURCE_DERIVED) {
-        int rc = drain(c);
-        if (!rc) rc = materialise_gradient(c, l);
-        if (rc) return rc;
-        any = true;
-      }
-    if (any) { CK(cudaStreamSynchronize(c->stream)); may_defer = false; }
-  }
-  const bool fused = !c->layers[0].V && c->layers[0].S && c->cfg.vector_source == FTKB_SOURCE_DERIVED && (c->n == 2 || c->fused3d);
-  if (!c->layers[0].V && !fused) return fail(c, FTKB_ERR_INVALID, "update_timestep: the snapshot has no vector field");
-  if (c->current_timestep + 1 >= (1 << KEY_TIME_BITS)) return fail(c, FTKB_ERR_OVERFLOW, "update_timestep: timestep exceeds the element id range");
-  if (c->push_d2h_outstanding) {
-    CK(cudaStreamSynchronize(c->stream));   // resolutions of layers derived at push time are on the host now
-    c->push_d2h_outstanding = false;
-  }
-  // derive timing of the most recent gradient launch
-  if (c->derive_timed) {
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]) == cudaSuccess) { c->stats.ms_derive += ms; c->stats.last_ms_derive = ms; }
-    else cudaGetLastError();
-    c->derive_timed = false;
-  }
-  const bool has_next = c->layers.size() >= 2;
-  if (has_next && !c->layers[1].V && !(fused && c->layers[1].S)) return fail(c, FTKB_ERR_INVALID, "update_timestep: the next snapshot has no vector field");
-  // vector input: the range-cell scan streams each layer once and produces its min |v|; layers it cannot take now
-  // (pushed further ahead than this sweep reads) get the plain resolution pass
-  bool vcells = !fused && c->cellsV && c->layers[0].V && c->cfg.vector_source == FTKB_SOURCE_GIVEN;
-  for (size_t k = 0; vcells && k < (has_next ? 2u : 1u); k++)
-    if (!c->layers[k].V || (uintptr_t)c->layers[k].V % 16 != 0) vcells = false;
-  {
-    bool any = false;
-    for (size_t k = 0; k < c->layers.size(); k++) {
-      Layer &l = c->layers[k];
-      if (l.V && l.res_pending && !(vcells && k < 2)) {
-        int rc = drain(c);
-        if (!rc) rc = resolve_pending(c, l);
-        if (rc) return rc;
-        any = true;
-      }
-    }
-    if (any) { CK(cudaStreamSynchronize(c->stream)); c->push_d2h_outstanding = false; may_defer = false; }
-  }
-  if (has_next && fused && c->layers[1].V) return fail(c, FTKB_ERR_INVALID, "update_timestep: resident snapshots mix derived and given vector fields");
-  // ref: critical_point_tracker.hh:850-864 (running minimum over every resident snapshot, every sweep).
-  // Layers whose resolution the fused scan still has to produce are left out here: the sweep runs with
-  // the factor known so far and is repeated if the completed minimum changes nbits (nbits only ever
-  // grows and is clamped to [8, 21], so at most 13 sweeps of a whole run are repeated).
-  for (const Layer &l : c->layers)
-    if ((l.V || l.S) && !l.res_pending) c->resolution = std::min(c->resolution, slot_value(c, l.slot));
-  int nbits = nbits_of(c->resolution);
+// arm the device counters from the host mirror; the same copy resets the resolution slots whose mirror is all ones
+static int arm_counters(ftkb_ctx *c) {
+  for (int k : {ftkb_ctx::SLOT_WL, ftkb_ctx::SLOT_WL2, ftkb_ctx::SLOT_UQ, ftkb_ctx::SLOT_POISON, ftkb_ctx::SLOT_POISON2, ftkb_ctx::SLOT_TICKET})
+    c->h_scalars[k] = 0;
+  c->h_scalars[ftkb_ctx::SLOT_PT] = c->npts;
+  CK(cudaMemcpyAsync(c->d_scalars, c->h_scalars, 15 * sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
+  return FTKB_OK;
+}
 
-  SweepParams p{};
-  fill_sweep_geometry(c, p);
-  p.t = c->current_timestep;
-  p.has_next = has_next;
-  p.no_filter = (c->n == 3 && !c->cfg.robust_detection);
-  p.scalar_source = c->layers[0].S ? c->cfg.scalar_source : FTKB_SOURCE_NONE;
-  p.jacobian_source = c->cfg.jacobian_source;
-  p.jacobian_symmetric = c->cfg.jacobian_symmetric;
-  // 2D: jacobian2D<double,true> on the scalar path, <double,false> when the vector field was pushed
-  p.derived_symmetric = c->cfg.vector_source == FTKB_SOURCE_DERIVED;
-  p.robust = c->cfg.robust_detection;
-  p.compute_degrees = c->cfg.compute_degrees;
-  p.use_type_filter = c->cfg.use_type_filter;
-  p.type_filter = c->cfg.type_filter;
-  Layer *lay[2] = {&c->layers[0], &c->layers[has_next ? 1 : 0]};
-  for (int k = 0; k < 2; k++) { p.L[k].S = lay[k]->S; p.L[k].V = lay[k]->V; p.L[k].J = lay[k]->J; }
-  if (has_next && p.scalar_source != FTKB_SOURCE_NONE && !c->layers[1].S) return fail(c, FTKB_ERR_INVALID, "update_timestep: the next snapshot has no scalar field");
-  p.fused = fused;
-  p.poison = c->d_scalars + ftkb_ctx::SLOT_POISON;
-  const bool aligned = rows_aligned16(c, lay[0]->S, lay[1]->S);    // 2D scalar input: the range-cell kernels need 16-byte aligned rows
-  if (fused && c->n == 3) {
-    if (!encode_scalar_tmap3d(lay[0]->S, p.W, p.H, p.D, &p.tmap[0]) || !encode_scalar_tmap3d(lay[1]->S, p.W, p.H, p.D, &p.tmap[1])) {
-      int rc = drain(c);
-      if (!rc) rc = abandon_fused3d(c);      // no TMA descriptor (driver entry point or alignment): unfused path
-      return rc ? rc : update_impl(c, allow_defer);
+// One sweep: the scan between ev[0] and ev[1] on the context's stream, then the exact test up to ev[2] on stream ts, behind
+// test_after as well if that is given.  A range-cell scan streams each layer once (the step that first sees it) and reads
+// its cells after that; the very first step streams both layers.
+static int launch_sweep(ftkb_ctx *c, const Scan &s, SweepParams &p, Layer &l0, Layer &l1, cudaEvent_t *ev, cudaStream_t ts,
+                        cudaEvent_t test_after) {
+  CK(cudaEventRecord(ev[0], c->stream));
+  if (!s.cells) {
+    s.launch(p, c->stream);
+  } else if (!l0.cells_valid) {
+    p.sum_in[0] = l0.cells; p.sum_in[1] = l1.cells;
+    p.sum_mode = p.has_next ? SUM_BUILD : SUM_BUILD_TEST1; p.build_layer = 0; p.sum_out = l0.cells;
+    s.launch(p, c->stream);
+    l0.cells_valid = true;
+    if (p.has_next) {
+      c->stats.kernel_launches++;
+      p.sum_mode = l1.cells_valid ? SUM_TEST2 : SUM_BUILD_TEST2; p.build_layer = 1; p.sum_out = l1.cells;
+      s.launch(p, c->stream);
+      l1.cells_valid = true;
     }
-    fused3d_decomposition(c, p);
-  } else if (fused) {
-    fused2d_decomposition(c, p, aligned);
-  } else if (vcells) {
-    vcells_decomposition(c, p);
   } else {
-    p.nsx = (p.nc[0] + 30) / 31;
-    if (c->n == 2) {
-      p.rows = 64;
-      p.nsy = (p.nc[1] + p.rows - 1) / p.rows;
-      p.nsz = 1;
+    p.sum_in[0] = l0.cells; p.sum_in[1] = l1.cells;
+    if (p.has_next && !l1.cells_valid) {
+      p.sum_mode = SUM_BUILD_TEST2; p.build_layer = 1; p.sum_out = l1.cells;
+      l1.cells_valid = true;
     } else {
-      p.rows = 32;
-      p.nsy = (p.nc[1] + 14) / 15;
-      p.nsz = (p.nc[2] + p.rows - 1) / p.rows;
+      p.sum_mode = p.has_next ? SUM_TEST2 : SUM_TEST1;
     }
+    s.launch(p, c->stream);
   }
-  p.keys2d = c->keys2d;
-  p.pt_count = c->d_scalars + ftkb_ctx::SLOT_PT;
-  p.ticket = c->d_scalars + ftkb_ctx::SLOT_TICKET;
-  p.test_blocks = test_grid(c);
-  const bool cells_path = vcells || (fused && (c->n == 3 || aligned));
-  void (*launch_cells)(const SweepParams &, cudaStream_t) = vcells ? launch_vscan_cells : (c->n == 3 ? launch_scan3d_cells : launch_scan2d_cells);
+  CK(cudaEventRecord(ev[1], c->stream));
+  if (test_after) CK(cudaStreamWaitEvent(c->stream, test_after, 0));
+  if (ts != c->stream) CK(cudaStreamWaitEvent(ts, ev[1], 0));
+  launch_test(p, ts);
+  CK(cudaEventRecord(ev[2], ts));
+  c->stats.kernel_launches += 2;
+  return check_launch(c, "sweep");
+}
 
-  // ---- deferred step: enqueue and return; the previous one is confirmed behind it ------------------------------------
-  if (may_defer && cells_path && lay[0]->cells_valid && !p.no_filter) {
-    if (has_next && !lay[1]->cells) {
-      // (an empty pool means one more buffer: with a step in flight four layers hold cells -- the one in limbo, the two being
-      // swept and the one being built; confirming the step in flight first would serialise the steps again)
-      const int rc0 = ensure_cells(c, *lay[1], p);
-      if (rc0) return rc0;
-    }
-    p.nbits = nbits;
-    p.factor = (double)(uint64_t)(1 << nbits);
-    p.thrp_f = (float)((1.0 / p.factor) * (1.0 + 1.0 / 1048576.0));
-    p.thr2_f = (float)(2.0 / p.factor);
-    p.lim_f = (float)(0.999 * 4.5e18 / (p.factor * p.factor));
-    const auto te0 = std::chrono::steady_clock::now();
-    ftkb_ctx::Pending pd;
-    pd.seq = ++c->step_seq;
-    pd.ring = (int)(pd.seq % ftkb_ctx::RING);
-    pd.evset = (int)(pd.seq & 1);
-    pd.has_next = has_next;
-    pd.nbits = nbits;
-    pd.npts_before = c->npts;                 // exact for the oldest enqueued step (set again when it becomes the oldest)
-    p.res_slot[0] = p.res_slot[1] = nullptr;
-    for (int k = 0; k < (has_next ? 2 : 1); k++)
-      if (lay[k]->res_pending) {
-        p.res_slot[k] = c->d_scalars + lay[k]->slot;
-        pd.res_slots[k] = lay[k]->slot;
-        lay[k]->res_pending = false;          // this scan produces it; the value reaches the host at confirmation
-      }
-    pd.wl_sel = c->wl_sel;
-    p.wl = c->wl_sel ? c->d_wl2 : c->d_wl; p.wl_cap = c->wl_cap;
-    { const int rcg = grow_points_ahead(c); if (rcg) return rcg; }
-    p.pts = c->d_pts; p.pt_cap = c->pt_cap;
-    pd.pt_cap = c->pt_cap;
-    // worklist, its counter and the poison flag alternate between two sets: the test kernel of this step may still run
-    // (on stream2) while the scan of the next step fills the other set; each test kernel re-arms its own set when done
-    p.wl_count = c->d_scalars + (c->wl_sel ? ftkb_ctx::SLOT_WL2 : ftkb_ctx::SLOT_WL);
-    p.poison = c->d_scalars + (c->wl_sel ? ftkb_ctx::SLOT_POISON2 : ftkb_ctx::SLOT_POISON);
-    p.step_out = c->h_ring + 8 * pd.ring;     // pinned + mapped, unified addressing: the device writes it in place
-    p.step_seq = pd.seq;
-    // resolution slots are handed out in push order: the layer the scan of step k+1 / k+2 resolves sits 2 / 3 places
-    // behind the current front, resident already or still to be pushed.  This step's test kernel re-arms the slot for
-    // step k+2 (step k+1's scan may already be running by then; its slot was re-armed by the previous test kernel).
-    auto slot_at = [&](size_t idx) { return idx < c->layers.size() ? c->layers[idx].slot : (int)((c->next_slot + (idx - c->layers.size())) % 8); };
-    p.res_reset = c->d_scalars + slot_at(3);
-    if (!c->primed) {
-      // first deferred step after a synchronous one: arm the device counters once from the host mirror
-      c->h_scalars[ftkb_ctx::SLOT_WL] = 0;
-      c->h_scalars[ftkb_ctx::SLOT_WL2] = 0;
-      c->h_scalars[ftkb_ctx::SLOT_PT] = c->npts;
-      c->h_scalars[ftkb_ctx::SLOT_UQ] = 0;
-      c->h_scalars[ftkb_ctx::SLOT_POISON] = 0;
-      c->h_scalars[ftkb_ctx::SLOT_POISON2] = 0;
-      c->h_scalars[ftkb_ctx::SLOT_TICKET] = 0;
-      if (c->layers.size() < 3) c->h_scalars[slot_at(2)] = ~0ull;      // the layer the next step's scan resolves (not pushed yet)
-      CK(cudaMemcpyAsync(c->d_scalars, c->h_scalars, 15 * sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
-    }
-    CK(cudaEventRecord(c->dev[pd.evset][0], c->stream));
-    p.sum_in[0] = lay[0]->cells; p.sum_in[1] = lay[1]->cells;
-    if (has_next && !lay[1]->cells_valid) {
-      p.sum_mode = SUM_BUILD_TEST2; p.build_layer = 1; p.sum_out = lay[1]->cells;
-      lay[1]->cells_valid = true;
-    } else {
-      p.sum_mode = has_next ? SUM_TEST2 : SUM_TEST1;
-    }
-    launch_cells(p, c->stream);
-    CK(cudaEventRecord(c->dev[pd.evset][1], c->stream));
-    // a test kernel with a GPU's worth of work (feature-dense fields: 1e5 .. 1e6 surviving cubes) gains nothing next to the
-    // following scan -- the two take turns on the SMs, measured 0.90 .. 1.64 ms per step against 0.95 in a row -- so only
-    // the small, latency-bound ones go to the second stream
-    const bool overlap = c->wl_hint < 100000;
-    if (!overlap && c->last_test_overlapped && !c->pend.empty())
-      CK(cudaStreamWaitEvent(c->stream, c->dev[c->pend.back().evset][2], 0));     // test kernels share one ticket counter: never two at once
-    c->last_test_overlapped = overlap;
-    cudaStream_t ts = overlap ? c->stream2 : c->stream;
-    if (overlap) CK(cudaStreamWaitEvent(c->stream2, c->dev[pd.evset][1], 0));
-    launch_test(p, ts);
-    CK(cudaEventRecord(c->dev[pd.evset][2], ts));
-    c->stats.kernel_launches += 2;
-    const int rc = check_launch(c, "sweep");
-    if (rc) return rc;
-    c->pend.push_back(pd);
-    c->primed = true;
-    c->wl_sel ^= 1;
-    if (c->debug_timing) { c->host_enq_us += std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - te0).count(); c->host_enq_n++; }
-    while (c->pend.size() > 1) {
-      const int rc2 = confirm_front(c);
-      if (rc2) return rc2;
-    }
-    return FTKB_OK;
+// ---- deferred step: enqueue and return; the previous one is confirmed behind it ------------------------------------
+static int enqueue_step(ftkb_ctx *c, const Scan &s, SweepParams &p, Layer &l0, Layer &l1, int nbits) {
+  const bool has_next = p.has_next;
+  if (has_next && !l1.cells) {
+    // (an empty pool means one more buffer: with a step in flight four layers hold cells -- the one in limbo, the two being
+    // swept and the one being built; confirming the step in flight first would serialise the steps again)
+    const int rc0 = ensure_cells(c, l1, p);
+    if (rc0) return rc0;
   }
+  set_factor(p, nbits);
+  p.test_blocks = test_grid(c);
+  const auto te0 = std::chrono::steady_clock::now();
+  ftkb_ctx::Pending pd;
+  pd.seq = ++c->step_seq;
+  pd.ring = (int)(pd.seq % ftkb_ctx::RING);
+  pd.evset = (int)(pd.seq & 1);
+  pd.has_next = has_next;
+  pd.nbits = nbits;
+  pd.npts_before = c->npts;                 // exact for the oldest enqueued step (set again when it becomes the oldest)
+  Layer *lay[2] = {&l0, &l1};
+  for (int k = 0; k < (has_next ? 2 : 1); k++)
+    if (lay[k]->res_pending) {
+      p.res_slot[k] = c->d_scalars + lay[k]->slot;
+      pd.res_slots[k] = lay[k]->slot;
+      lay[k]->res_pending = false;          // this scan produces it; the value reaches the host at confirmation
+    }
+  pd.wl_sel = c->wl_sel;
+  p.wl = c->wl_sel ? c->d_wl2 : c->d_wl; p.wl_cap = c->wl_cap;
+  { const int rcg = grow_points_ahead(c); if (rcg) return rcg; }
+  p.pts = c->d_pts; p.pt_cap = c->pt_cap;
+  pd.pt_cap = c->pt_cap;
+  // worklist, its counter and the poison flag alternate between two sets: the test kernel of this step may still run
+  // (on stream2) while the scan of the next step fills the other set; each test kernel re-arms its own set when done
+  p.wl_count = c->d_scalars + (c->wl_sel ? ftkb_ctx::SLOT_WL2 : ftkb_ctx::SLOT_WL);
+  p.poison = c->d_scalars + (c->wl_sel ? ftkb_ctx::SLOT_POISON2 : ftkb_ctx::SLOT_POISON);
+  p.step_out = c->h_ring + 8 * pd.ring;     // pinned + mapped, unified addressing: the device writes it in place
+  p.step_seq = pd.seq;
+  // resolution slots are handed out in push order: the layer the scan of step k+1 / k+2 resolves sits 2 / 3 places
+  // behind the current front, resident already or still to be pushed.  This step's test kernel re-arms the slot for
+  // step k+2 (step k+1's scan may already be running by then; its slot was re-armed by the previous test kernel).
+  auto slot_at = [&](size_t idx) { return idx < c->layers.size() ? c->layers[idx].slot : (int)((c->next_slot + (idx - c->layers.size())) % 8); };
+  p.res_reset = c->d_scalars + slot_at(3);
+  if (!c->primed) {
+    // first deferred step after a synchronous one: arm the device counters once
+    if (c->layers.size() < 3) c->h_scalars[slot_at(2)] = ~0ull;      // the layer the next step's scan resolves (not pushed yet)
+    const int rc = arm_counters(c);
+    if (rc) return rc;
+  }
+  // a test kernel with a GPU's worth of work (feature-dense fields: 1e5 .. 1e6 surviving cubes) gains nothing next to the
+  // following scan -- the two take turns on the SMs, measured 0.90 .. 1.64 ms per step against 0.95 in a row -- so only
+  // the small, latency-bound ones go to the second stream
+  const bool overlap = c->wl_hint < 100000;
+  // test kernels share one ticket counter: never two at once
+  const cudaEvent_t test_after = !overlap && c->last_test_overlapped && !c->pend.empty() ? c->dev[c->pend.back().evset][2] : nullptr;
+  c->last_test_overlapped = overlap;
+  const int rc = launch_sweep(c, s, p, l0, l1, c->dev[pd.evset], overlap ? c->stream2 : c->stream, test_after);
+  if (rc) return rc;
+  c->pend.push_back(pd);
+  c->primed = true;
+  c->wl_sel ^= 1;
+  if (c->debug_timing) { c->host_enq_us += std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - te0).count(); c->host_enq_n++; }
+  while (c->pend.size() > 1) {
+    const int rc2 = confirm_front(c);
+    if (rc2) return rc2;
+  }
+  return FTKB_OK;
+}
+
+// ---- synchronous step: confirmed before it returns; redone until the factor is right and the buffers were big enough --
+static int sync_step(ftkb_ctx *c, const Scan &s, SweepParams &p, Layer &l0, Layer &l1, int nbits) {
   { const int rc = drain(c); if (rc) return rc; }
   c->primed = false;
-  p.wl_count = c->d_scalars + ftkb_ctx::SLOT_WL;
-  p.step_out = nullptr;
-
+  const bool has_next = p.has_next;
+  Layer *lay[2] = {&l0, &l1};
   for (int attempt = 0; attempt < 12; attempt++) {
-    p.nbits = nbits;
-    p.factor = (double)(uint64_t)(1 << nbits);
-    p.thrp_f = (float)((1.0 / p.factor) * (1.0 + 1.0 / 1048576.0));
-    p.thr2_f = (float)(2.0 / p.factor);
-    p.lim_f = (float)(0.999 * 4.5e18 / (p.factor * p.factor));
+    set_factor(p, nbits);
     p.res_slot[0] = p.res_slot[1] = nullptr;
     bool pending = false;
-    if (fused || vcells)
+    if (p.fused || s.cells)
       for (int k = 0; k < (has_next ? 2 : 1); k++)
         if (lay[k]->res_pending) { p.res_slot[k] = c->d_scalars + lay[k]->slot; pending = true; }
     p.wl = c->d_wl; p.wl_cap = c->wl_cap;
     p.pts = c->d_pts; p.pt_cap = c->pt_cap;
     p.test_blocks = test_grid(c);
-    c->h_scalars[ftkb_ctx::SLOT_WL] = 0;
-    c->h_scalars[ftkb_ctx::SLOT_PT] = c->npts;
-    c->h_scalars[ftkb_ctx::SLOT_UQ] = 0;
-    c->h_scalars[ftkb_ctx::SLOT_POISON] = 0;
-    c->h_scalars[ftkb_ctx::SLOT_WL2] = 0;
-    c->h_scalars[ftkb_ctx::SLOT_TICKET] = 0;
-    // one copy resets the counters AND the resolution slots of the layers this sweep resolves (host mirror = all ones)
-    c->h_scalars[ftkb_ctx::SLOT_POISON2] = 0;
-    CK(cudaMemcpyAsync(c->d_scalars, c->h_scalars, 15 * sizeof(unsigned long long), cudaMemcpyHostToDevice, c->stream));
-    CK(cudaEventRecord(c->ev[0], c->stream));
-    if (cells_path) {
-      // each layer is streamed once (the step that first sees it); everything else reads its 16-byte range cells
-      int rc0 = ensure_cells(c, *lay[0], p);
-      if (!rc0 && has_next) rc0 = ensure_cells(c, *lay[1], p);
-      if (rc0) return rc0;
-      p.sum_in[0] = lay[0]->cells; p.sum_in[1] = lay[1]->cells;
-      if (!lay[0]->cells_valid) {
-        p.sum_mode = has_next ? SUM_BUILD : SUM_BUILD_TEST1; p.build_layer = 0; p.sum_out = lay[0]->cells;
-        launch_cells(p, c->stream);
-        lay[0]->cells_valid = true;
-        if (has_next) {
-          c->stats.kernel_launches++;       // the very first step streams two layers
-          p.sum_mode = lay[1]->cells_valid ? SUM_TEST2 : SUM_BUILD_TEST2; p.build_layer = 1; p.sum_out = lay[1]->cells;
-          launch_cells(p, c->stream);
-          lay[1]->cells_valid = true;
-        }
-      } else if (has_next && !lay[1]->cells_valid) {
-        p.sum_mode = SUM_BUILD_TEST2; p.build_layer = 1; p.sum_out = lay[1]->cells;
-        launch_cells(p, c->stream);
-        lay[1]->cells_valid = true;
-      } else {
-        p.sum_mode = has_next ? SUM_TEST2 : SUM_TEST1;
-        launch_cells(p, c->stream);
-      }
-    } else {
-      launch_scan(p, c->stream);
-    }
-    CK(cudaEventRecord(c->ev[1], c->stream));
-    launch_test(p, c->stream);
-    CK(cudaEventRecord(c->ev[2], c->stream));
-    c->stats.kernel_launches += 2;
-    int rc = check_launch(c, "sweep");
+    int rc = arm_counters(c);
+    if (!rc && s.cells) rc = ensure_cells(c, l0, p);
+    if (!rc && s.cells && has_next) rc = ensure_cells(c, l1, p);
+    if (!rc) rc = launch_sweep(c, s, p, l0, l1, c->ev, c->stream, nullptr);
     if (rc) return rc;
     if (pending) {   // slots 0..7 hold the per-layer resolutions, 8..11 the counters: one copy
       CK(cudaMemcpyAsync(c->h_scalars, c->d_scalars, 12 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
@@ -1477,25 +1396,11 @@ static int update_impl(ftkb_ctx *c, bool allow_defer) {
     }
     CK(cudaStreamSynchronize(c->stream));
     c->stats.d2h_bytes += 32;
-    if (vcells && c->h_scalars[ftkb_ctx::SLOT_POISON]) {
-      // a component was NaN-ordered by the float keys (|v| >= 2^1000, Inf): redo the step with the two-layer scan
+    if ((p.fused || s.cells) && c->h_scalars[ftkb_ctx::SLOT_POISON]) {
+      // a value the scan's float keys cannot order (NaN / Inf / >= 2^1000): redo the step with the slower scan
       c->stats.sweeps_repeated++;
-      c->cellsV = false;
-      for (Layer &l : c->layers) l.cells_valid = false;
-      return update_impl(c, false);
-    }
-    if (fused && c->n == 3 && c->h_scalars[ftkb_ctx::SLOT_POISON]) {
-      // a scalar was NaN / Inf / >= 2^1000: the fused scan's keys cannot bracket such values; redo the step unfused
-      c->stats.sweeps_repeated++;
-      const int rc2 = abandon_fused3d(c);
+      const int rc2 = fall_back(c);
       return rc2 ? rc2 : update_impl(c, false);
-    }
-    if (fused && c->n == 2 && c->h_scalars[ftkb_ctx::SLOT_POISON]) {
-      // 2D key scan: a scalar was NaN / Inf / >= 2^1000; the fp32-range build kernel handles those (slower)
-      c->stats.sweeps_repeated++;
-      c->keys2d = false;
-      for (Layer &l : c->layers) l.cells_valid = false;
-      return update_impl(c, false);
     }
     float ms_scan = 0, ms_test = 0;
     CK(cudaEventElapsedTime(&ms_scan, c->ev[0], c->ev[1]));
@@ -1547,6 +1452,86 @@ static int update_impl(ftkb_ctx *c, bool allow_defer) {
     return FTKB_OK;
   }
   return fail(c, FTKB_ERR_CUDA, "update_timestep: buffers kept overflowing");
+}
+
+static int update_impl(ftkb_ctx *c, bool allow_defer) {
+  if (c->layers.empty()) return fail(c, FTKB_ERR_INVALID, "update_timestep: no snapshot has been pushed");
+  CK(cudaSetDevice(c->cfg.device));
+  bool may_defer = allow_defer && !c->streaming && !c->push_d2h_outstanding;
+  if (!may_defer) { const int rc = drain(c); if (rc) return rc; }
+  if (c->n == 3 && c->scans == Scans::fused3d && c->cfg.vector_source == FTKB_SOURCE_DERIVED) {
+    // a layer whose pointer TMA cannot take was materialised at push time: the sweep cannot mix the two forms
+    bool anyV = false, anyS = false;
+    for (const Layer &l : c->layers) { anyV = anyV || l.V; anyS = anyS || (!l.V && l.S); }
+    if (anyV && anyS) {
+      int rc = drain(c);
+      if (!rc) rc = fall_back(c);
+      if (rc) return rc;
+      may_defer = false;
+    }
+  }
+  if (c->n == 3 && c->scans != Scans::fused3d) {
+    // scalar layers that reached the context without their gradient (remote snapshots): materialise it
+    bool any = false;
+    for (Layer &l : c->layers)
+      if (!l.V && l.S && c->cfg.vector_source == FTKB_SOURCE_DERIVED) {
+        int rc = drain(c);
+        if (!rc) rc = materialise_gradient(c, l);
+        if (rc) return rc;
+        any = true;
+      }
+    if (any) { CK(cudaStreamSynchronize(c->stream)); may_defer = false; }
+  }
+  const bool has_next = c->layers.size() >= 2;
+  Layer &l0 = c->layers[0], &l1 = c->layers[has_next ? 1 : 0];
+  SweepParams p{};
+  const Scan s = sweep_setup(c, l0, l1, has_next, p);
+  if (!s.launch) {
+    int rc = drain(c);
+    if (!rc) rc = fall_back(c);
+    return rc ? rc : update_impl(c, allow_defer);
+  }
+  if (!l0.V && !p.fused) return fail(c, FTKB_ERR_INVALID, "update_timestep: the snapshot has no vector field");
+  if (c->current_timestep + 1 >= (1 << KEY_TIME_BITS)) return fail(c, FTKB_ERR_OVERFLOW, "update_timestep: timestep exceeds the element id range");
+  if (c->push_d2h_outstanding) {
+    CK(cudaStreamSynchronize(c->stream));   // resolutions of layers derived at push time are on the host now
+    c->push_d2h_outstanding = false;
+  }
+  // derive timing of the most recent gradient launch
+  if (c->derive_timed) {
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, c->ev[4], c->ev[5]) == cudaSuccess) { c->stats.ms_derive += ms; c->stats.last_ms_derive = ms; }
+    else cudaGetLastError();
+    c->derive_timed = false;
+  }
+  if (has_next && !l1.V && !(p.fused && l1.S)) return fail(c, FTKB_ERR_INVALID, "update_timestep: the next snapshot has no vector field");
+  {
+    // vector input: the range-cell scan streams each layer once and produces its min |v|; layers it cannot take now
+    // (pushed further ahead than this sweep reads) get the plain resolution pass
+    bool any = false;
+    for (size_t k = 0; k < c->layers.size(); k++) {
+      Layer &l = c->layers[k];
+      if (l.V && l.res_pending && !(s.cells && !p.fused && k < 2)) {
+        int rc = drain(c);
+        if (!rc) rc = resolve_pending(c, l);
+        if (rc) return rc;
+        any = true;
+      }
+    }
+    if (any) { CK(cudaStreamSynchronize(c->stream)); c->push_d2h_outstanding = false; may_defer = false; }
+  }
+  if (has_next && p.fused && l1.V) return fail(c, FTKB_ERR_INVALID, "update_timestep: resident snapshots mix derived and given vector fields");
+  // ref: critical_point_tracker.hh:850-864 (running minimum over every resident snapshot, every sweep).
+  // Layers whose resolution the fused scan still has to produce are left out here: the sweep runs with
+  // the factor known so far and is repeated if the completed minimum changes nbits (nbits only ever
+  // grows and is clamped to [8, 21], so at most 13 sweeps of a whole run are repeated).
+  for (const Layer &l : c->layers)
+    if ((l.V || l.S) && !l.res_pending) c->resolution = std::min(c->resolution, slot_value(c, l.slot));
+  set_key_filter(c, p);
+  if (has_next && p.scalar_source != FTKB_SOURCE_NONE && !l1.S) return fail(c, FTKB_ERR_INVALID, "update_timestep: the next snapshot has no scalar field");
+  const int nbits = nbits_of(c->resolution);
+  if (may_defer && s.cells && l0.cells_valid && !p.no_filter) return enqueue_step(c, s, p, l0, l1, nbits);
+  return sync_step(c, s, p, l0, l1, nbits);
 }
 
 extern "C" int ftkb_advance_timestep(ftkb_ctx *c) {
