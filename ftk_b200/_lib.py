@@ -80,7 +80,7 @@ EXPORTS = [
     "ftkb_reset_stats", "ftkb_synchronize", "ftkb_timer_start", "ftkb_timer_stop", "ftkb_mesh_ntypes", "ftkb_mesh_unit_simplex", "ftkb_mesh_scope_type",
     "ftkb_mesh_sides", "ftkb_mesh_side_of",
     "ftkb_curveset_create", "ftkb_get_curveset", "ftkb_curveset_destroy", "ftkb_curveset_post_process", "ftkb_curveset_size",
-    "ftkb_curveset_get", "ftkb_curveset_last_error", "ftkb_curveset_slice",
+    "ftkb_curveset_get", "ftkb_curveset_last_error", "ftkb_curveset_slice", "ftkb_get_live_curveset", "ftkb_group_get_live_curveset",
     "ftkb_ipc_export", "ftkb_ipc_import", "ftkb_ipc_close", "ftkb_export_layer_cells", "ftkb_push_snapshot_remote",
     "ftkb_set_streaming_trajectories", "ftkb_get_trajectory_complete", "ftkb_online_create", "ftkb_online_destroy", "ftkb_online_grow", "ftkb_online_grow_prepared",
     "ftkb_online_size", "ftkb_online_get", "ftkb_set_coords", "ftkb_set_producer_stream", "ftkb_get_layer",
@@ -138,6 +138,8 @@ def lib():
     L.ftkb_mesh_side_of.argtypes = [C.c_int, C.c_int, C.c_int, vp]
     L.ftkb_curveset_create.argtypes = [vp, C.c_uint64, vp, vp, vp, C.c_uint64, C.POINTER(vp)]
     L.ftkb_get_curveset.argtypes = [vp, C.POINTER(vp)]
+    L.ftkb_get_live_curveset.argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(vp)]
+    L.ftkb_group_get_live_curveset.argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(vp)]
     L.ftkb_curveset_destroy.argtypes = [vp]
     L.ftkb_curveset_destroy.restype = None
     L.ftkb_curveset_post_process.argtypes = [vp, C.c_char_p]

@@ -108,7 +108,7 @@ struct ftkb_ctx {
   // run with a stale quantisation factor, or whose buffers overflowed, is replayed synchronously together with
   // whatever was enqueued behind it.  Layers popped in between wait in `limbo`.
   struct Pending {
-    int ring = 0, evset = 0, pops = 0, nbits = 0, wl_sel = 0;
+    int ring = 0, evset = 0, pops = 0, nbits = 0, wl_sel = 0, timestep = 0;
     uint64_t seq = 0, npts_before = 0, pt_cap = 0;     // pt_cap: the point buffer's capacity this step ran with
     bool has_next = false;
     int res_slots[2] = {-1, -1};     // resolution slots this step's scan fills
@@ -173,7 +173,13 @@ struct ftkb_ctx {
   bool streaming = false;
   std::unique_ptr<ftkb::OnlineTracer> online;
   uint64_t grown = 0;            // d_pts[0 .. grown) have been through a grow step
+  int grown_through = 0;         // the last timestep whose grow step has run (start_timestep - 1: none)
   bool grow_failed = false;      // a grow step threw: every later call that depends on the trajectories reports it
+
+  // d_pts[begin, end) = the points of the confirmed sweep of timestep start_timestep + k (steps[k]); a replay only redoes steps
+  // that were not confirmed, from the point count they started at, so a confirmed step's points stay where they are
+  struct StepRange { uint64_t begin = 0, end = 0; bool interval = false; };
+  std::vector<StepRange> steps;
 
   ftkb_stats stats{};
 };
@@ -371,7 +377,8 @@ extern "C" int ftkb_create(const ftkb_config *cfg, ftkb_ctx **out) {
   c->n_ord = (int)mt.ordinal_types[n].size();
   c->n_int = (int)mt.interval_types[n].size();
   c->current_timestep = cfg->start_timestep;
-  c->resolution = cfg->resolution_init > 0 ? cfg->resolution_init : DBL_MAX;
+  c->grown_through = cfg->start_timestep - 1;
+  c->resolution =cfg->resolution_init > 0 ? cfg->resolution_init : DBL_MAX;
 
   auto bail = [&](const std::string &m, int code) { g_create_error = m; ftkb_destroy(c); return code; };
   cudaError_t e;
@@ -1014,8 +1021,8 @@ static int wait_grow(ftkb_ctx *c) {
   return c->grow_failed ? FTKB_ERR_NOMEM : FTKB_OK;
 }
 
-// one grow step over d_pts[grown .. end)
-static int grow_trajectories(ftkb_ctx *c, uint64_t end) {
+// one grow step over d_pts[grown .. end), the batch of timestep t
+static int grow_trajectories(ftkb_ctx *c, uint64_t end, int t) {
   const uint64_t n = end - c->grown;
   if (n >= 0xffffffffull) return fail(c, FTKB_ERR_OVERFLOW, "more than 2^32 punctured simplices in one step");
   { const int rc = wait_grow(c); if (rc) return rc; }
@@ -1078,16 +1085,68 @@ static int grow_trajectories(ftkb_ctx *c, uint64_t end) {
   catch (const std::bad_alloc &) { c->grow_failed = true; return fail(c, FTKB_ERR_NOMEM, "streaming grow step: out of memory (trajectories are incomplete)"); }
   catch (const std::exception &e) { c->grow_failed = true; return fail(c, FTKB_ERR_INVALID, std::string("streaming grow step: ") + e.what()); }
   c->grown = end;
+  c->grown_through = t;
   c->traced = false;
   return FTKB_OK;
 }
 
 // a streaming context that sweeps nothing itself (the merged context of a device group, include/ftkb200.h): one grow step over
-// the imported points that follow those grown so far, up to index `end` of the import order
-int ftkb::grow_imported(ftkb_ctx *c, uint64_t end) {
-  if (!c || !c->streaming || end < c->grown || end > c->npts) return FTKB_ERR_INVALID;
+// the imported points that follow those grown so far, the batch of timestep t
+int ftkb::grow_imported(ftkb_ctx *c, int t) {
+  if (!c || !c->streaming) return FTKB_ERR_INVALID;
   CK(cudaSetDevice(c->cfg.device));
-  return grow_trajectories(c, end);
+  return grow_trajectories(c, c->npts, t);
+}
+
+// the sweep of timestep t has been confirmed with d_pts[begin, end) as its points (a second sweep of the same timestep appends)
+static void record_step(ftkb_ctx *c, int t, uint64_t begin, uint64_t end, bool interval) {
+  const size_t k = (size_t)(t - c->cfg.start_timestep);
+  if (k >= c->steps.size()) {
+    c->steps.resize(k + 1);
+    c->steps[k].begin = begin;
+  }
+  c->steps[k].end = end;
+  c->steps[k].interval = c->steps[k].interval || interval;
+}
+
+int ftkb::confirmed_through(const ftkb_ctx *c) { return c->cfg.start_timestep + (int)c->steps.size() - 1; }
+
+int ftkb::import_step(ftkb_ctx *dst, ftkb_ctx *src, int t, bool *interval) {
+  const size_t k = (size_t)(t - src->cfg.start_timestep);
+  if (!dst->streaming || t < src->cfg.start_timestep || k >= src->steps.size())
+    return fail(dst, FTKB_ERR_INVALID, "import_step: timestep " + std::to_string(t) + " has no confirmed sweep");
+  ftkb_ctx *c = dst;        // (CK reports to c)
+  const ftkb_ctx::StepRange r = src->steps[k];
+  *interval = r.interval;
+  const uint64_t n = r.end - r.begin;
+  if (!n) return FTKB_OK;
+  const int dd = dst->cfg.device, sd = src->cfg.device;
+  if (!src->retired_pts.empty()) {
+    // the source's point buffer was replaced while steps were in flight: its confirmed points reach the new buffer by a copy
+    // queued on its stream
+    CK(cudaSetDevice(sd));
+    CK(cudaEventRecord(src->ev[3], src->stream));
+    CK(cudaSetDevice(dd));
+    CK(cudaStreamWaitEvent(dst->stream, src->ev[3], 0));
+  }
+  CK(cudaSetDevice(dd));
+  if (dst->npts + n > dst->pt_cap) {
+    const int rc = grow_points(dst, dst->npts + n);
+    if (rc) return rc;
+  }
+  if (dd == sd) {
+    CK(cudaMemcpyAsync(dst->d_pts + dst->npts, src->d_pts + r.begin, sizeof(ftkb_point) * n, cudaMemcpyDeviceToDevice, dst->stream));
+  } else {
+    CK(enable_peer_access(dd, sd));
+    CK(cudaMemcpyPeerAsync(dst->d_pts + dst->npts, dd, src->d_pts + r.begin, sd, sizeof(ftkb_point) * n, dst->stream));
+  }
+  // complete before the source's owner may move its buffer again
+  CK(cudaStreamSynchronize(dst->stream));
+  dst->npts += n;
+  dst->stats.points = dst->npts;
+  dst->sorted = false;
+  dst->traced = false;
+  return FTKB_OK;
 }
 
 extern "C" int ftkb_set_streaming_trajectories(ftkb_ctx *c, int enable) {
@@ -1098,6 +1157,7 @@ extern "C" int ftkb_set_streaming_trajectories(ftkb_ctx *c, int enable) {
   c->grow_failed = false;
   c->online.reset(c->streaming ? new ftkb::OnlineTracer(c->n, c->cfg.lb, c->cfg.ub) : nullptr);
   c->grown = 0;
+  c->grown_through = c->cfg.start_timestep - 1;
   return FTKB_OK;
 }
 
@@ -1195,6 +1255,7 @@ static int confirm_front(ftkb_ctx *c) {
   c->stats.simplices_tested += c->ncore * (uint64_t)(c->n_ord + (pd.has_next ? c->n_int : 0));
   if (npt != c->npts) { c->sorted = false; c->traced = false; }
   if (npt > c->npts) c->max_step_points = std::max(c->max_step_points, npt - c->npts);
+  record_step(c, pd.timestep, pd.npts_before, npt, pd.has_next);
   c->npts = npt;
   c->stats.points = npt;
   for (int j = 0; j < pd.pops && !c->limbo.empty(); j++) {
@@ -1318,6 +1379,7 @@ static int enqueue_step(ftkb_ctx *c, const Scan &s, SweepParams &p, Layer &l0, L
   pd.has_next = has_next;
   pd.nbits = nbits;
   pd.npts_before = c->npts;                 // exact for the oldest enqueued step (set again when it becomes the oldest)
+  pd.timestep = c->current_timestep;
   Layer *lay[2] = {&l0, &l1};
   for (int k = 0; k < (has_next ? 2 : 1); k++)
     if (lay[k]->res_pending) {
@@ -1446,9 +1508,10 @@ static int sync_step(ftkb_ctx *c, const Scan &s, SweepParams &p, Layer &l0, Laye
     c->last_wl_sel = 0;
     c->stats.simplices_tested += c->ncore * (uint64_t)(c->n_ord + (has_next ? c->n_int : 0));
     if (npt != c->npts) { c->sorted = false; c->traced = false; }
+    record_step(c, c->current_timestep, c->npts, npt, has_next);
     c->npts = npt;
     c->stats.points = npt;
-    if (c->streaming && has_next) { const int rc2 = grow_trajectories(c, c->npts); if (rc2) return rc2; }
+    if (c->streaming && has_next) { const int rc2 = grow_trajectories(c, c->npts, c->current_timestep); if (rc2) return rc2; }
     return FTKB_OK;
   }
   return fail(c, FTKB_ERR_CUDA, "update_timestep: buffers kept overflowing");
@@ -1710,6 +1773,40 @@ extern "C" int ftkb_import_points(ftkb_ctx *c, const ftkb_point *pts, uint64_t n
   return FTKB_OK;
 }
 
+// A streaming context's trajectories grown so far, in id order, as CSR over its sorted points (traj_*): what ftkb_finalize
+// publishes, and what ftkb_get_live_curveset reads at any time.  Points that no grow step has seen yet are among the sorted
+// points but on no trajectory.
+static int publish_grown(ftkb_ctx *c) {
+  { const int rc = wait_grow(c); if (rc) return rc; }
+  { const int rc = ensure_sorted(c); if (rc) return rc; }
+  const uint64_t n = c->nsorted;
+  const auto t0 = std::chrono::steady_clock::now();
+  c->traj_off.assign(1, 0);
+  c->traj_idx.clear();
+  c->traj_loop.clear();
+  c->traj_complete.clear();
+  std::vector<uint64_t> keys(n);
+  if (n) {      // the sorted points' element keys (the device sorted by them)
+    CK(cudaMemcpyAsync(keys.data(), c->d_keys_sorted, 8 * n, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    c->stats.d2h_bytes += 8 * n;
+  }
+  const std::vector<uint64_t> &streamed = c->online->keys();
+  for (const ftkb::OnlineCurve &cv : c->online->curves()) {
+    for (const uint32_t g : cv.idx) {
+      const uint64_t key = streamed[g];
+      const auto it = std::lower_bound(keys.begin(), keys.end(), key);
+      if (it == keys.end() || *it != key) return fail(c, FTKB_ERR_INVALID, "a streamed point is missing from the sorted points");
+      c->traj_idx.push_back((uint64_t)(it - keys.begin()));
+    }
+    c->traj_loop.push_back(cv.loop);
+    c->traj_complete.push_back(cv.complete);
+    c->traj_off.push_back(c->traj_idx.size());
+  }
+  c->stats.ms_finalize_host += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  return FTKB_OK;
+}
+
 // ref: critical_point_tracker.hh:668-817 trace_critical_points_offline; cc2curves.hh:10-122
 extern "C" int ftkb_finalize(ftkb_ctx *c) {
   if (!c) return FTKB_ERR_INVALID;
@@ -1728,29 +1825,9 @@ extern "C" int ftkb_finalize(ftkb_ctx *c) {
   c->traj_loop.clear();
   c->traj_complete.clear();
   if (c->streaming) {
-    { const int rc2 = wait_grow(c); if (rc2) return rc2; }
-    // "done" (critical_point_tracker_2d_regular.hh:150-151): publish the grown trajectories, in id order, as CSR over
-    // the sorted points; the component labels / degrees of the offline trace are not computed
-    const auto t0 = std::chrono::steady_clock::now();
-    std::vector<uint64_t> keys(n);
-    if (n) {      // the sorted points' element keys (the device sorted by them)
-      CK(cudaMemcpyAsync(keys.data(), c->d_keys_sorted, 8 * n, cudaMemcpyDeviceToHost, c->stream));
-      CK(cudaStreamSynchronize(c->stream));
-      c->stats.d2h_bytes += 8 * n;
-    }
-    const std::vector<uint64_t> &streamed = c->online->keys();
-    for (const ftkb::OnlineCurve &cv : c->online->curves()) {
-      for (const uint32_t g : cv.idx) {
-        const uint64_t key = streamed[g];
-        const auto it = std::lower_bound(keys.begin(), keys.end(), key);
-        if (it == keys.end() || *it != key) return fail(c, FTKB_ERR_INVALID, "finalize: a streamed point is missing from the sorted points");
-        c->traj_idx.push_back((uint64_t)(it - keys.begin()));
-      }
-      c->traj_loop.push_back(cv.loop);
-      c->traj_complete.push_back(cv.complete);
-      c->traj_off.push_back(c->traj_idx.size());
-    }
-    c->stats.ms_finalize_host += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    // "done" (critical_point_tracker_2d_regular.hh:150-151): the grown trajectories as they stand; the component labels /
+    // degrees of the offline trace are not computed
+    { const int rc2 = publish_grown(c); if (rc2) return rc2; }
     c->traced = true;
     return FTKB_OK;
   }
@@ -1986,9 +2063,8 @@ extern "C" int ftkb_push_snapshot_remote(ftkb_ctx *c, const double *scalar, cons
   return FTKB_OK;
 }
 
-extern "C" int ftkb_get_curveset(ftkb_ctx *c, ftkb_curveset **out) {
-  if (!c || !out) return FTKB_ERR_INVALID;
-  if (!c->traced) return fail(c, FTKB_ERR_INVALID, "get_curveset: call finalize first");
+// the curve set of the trajectories in traj_* over the sorted points
+static int build_curveset(ftkb_ctx *c, ftkb_curveset **out) {
   const uint64_t ntraj = c->traj_off.empty() ? 0 : c->traj_off.size() - 1;
   static const uint64_t zero = 0;
   { const int rch = host_points(c); if (rch) return rch; }
@@ -1996,6 +2072,26 @@ extern "C" int ftkb_get_curveset(ftkb_ctx *c, ftkb_curveset **out) {
                                       c->traj_loop.data(), ntraj, out);
   if (rc == FTKB_OK)   // streaming: feature_curve_t::complete as the grow steps left it (curves are in id order)
     for (size_t k = 0; k < c->traj_complete.size() && k < (*out)->curves.size(); k++) (*out)->curves[k].complete = c->traj_complete[k] != 0;
+  return rc;
+}
+
+extern "C" int ftkb_get_curveset(ftkb_ctx *c, ftkb_curveset **out) {
+  if (!c || !out) return FTKB_ERR_INVALID;
+  if (!c->traced) return fail(c, FTKB_ERR_INVALID, "get_curveset: call finalize first");
+  return build_curveset(c, out);
+}
+
+extern "C" int ftkb_get_live_curveset(ftkb_ctx *c, int32_t *grown_through, ftkb_curveset **out) {
+  if (!c || !grown_through || !out) return fail(c, FTKB_ERR_INVALID, "get_live_curveset: null argument");
+  *out = nullptr;
+  if (!c->streaming) return fail(c, FTKB_ERR_INVALID, "get_live_curveset: streaming trajectories are off (ftkb_set_streaming_trajectories)");
+  CK(cudaSetDevice(c->cfg.device));
+  { const int rc = drain(c); if (rc) return rc; }
+  // after finalize traj_* hold what it published; before, they are rebuilt from the tracer (traced stays false, so the
+  // finalize-only getters still refuse, and any later sweep, grow or import makes the next query rebuild them)
+  if (!c->traced) { const int rc = publish_grown(c); if (rc) return rc; }
+  const int rc = build_curveset(c, out);
+  if (rc == FTKB_OK) *grown_through = c->grown_through;
   return rc;
 }
 

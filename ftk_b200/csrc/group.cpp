@@ -17,15 +17,20 @@
 //   merge         ftkb_group_finalize collects the (sparse) punctured simplices of every chunk into one context on the first
 //                 device and runs the union-find + ordering there: components that cross chunk boundaries are united by
 //                 the same neighbour search that unites them inside a chunk.
-//   streaming     chunks and slabs sweep offline; the merged context then runs the reference's grow step once per swept
-//                 interval t, in time order, over its sorted points of timestep t -- the batch a single streaming context
-//                 grows at t (ordinal sweep at t + interval sweep [t, t+1]).  The last ordinal sweep's points join no
-//                 trajectory, as on one device.
+//   streaming     the merged context exists from the first push and grows during the run.  Chunks and slabs keep sweeping
+//                 deferred; once the sweep of timestep t is confirmed (by every slab, or by the chunk that owns t) and t-1 has
+//                 been grown, the points of that sweep are copied to the merged context's device (peer copies, no host) and the
+//                 reference's grow step runs over them -- the batch a single streaming context grows at t (ordinal sweep at t +
+//                 interval sweep [t, t+1]).  Slabs are grown by the caller's thread after every sweep, chunks by a thread of the
+//                 merged context's own.  The last ordinal sweep's points join no trajectory, as on one device.
+//                 Locks: a chunk's `m` (its context) may be taken before the group's `m`, never after; `root_m` (the merged
+//                 context) before a chunk's `m`.
 //   coordinates   physical coordinates (ftkb_group_set_coords) are kept here and handed to every chunk context as it is
 //                 created and to every slab context at once; a slab looks them up in the whole array's frame.
 #include <algorithm>
 #include <atomic>
 #include <cfloat>
+#include <climits>
 #include <cmath>
 #include <condition_variable>
 #include <cstring>
@@ -94,7 +99,9 @@ struct Done {
 
 struct Chunk {
   int index = 0, device = 0;
+  std::mutex m;                          // ctx: held by the worker around every call into it, and by the grower while it copies
   ftkb_ctx *ctx = nullptr;               // created by the device's worker when the chunk may start
+  int confirmed = INT_MIN;               // streaming: the last timestep whose sweep ctx has confirmed (under the group's m)
   bool finished = false;                 // every sweep of the chunk has been confirmed
   double resolution_out = DBL_MAX;       // running minimum after the chunk (valid once finished)
   std::vector<ftkb_point> points;
@@ -150,6 +157,11 @@ struct ftkb_group {
   std::atomic<int> failed{FTKB_OK};
   mutable std::string error;                       // (set by refusals of const queries too)
   ftkb_ctx *root = nullptr;
+  // streaming: the merged context grows during the run
+  std::mutex root_m;                               // root, while the grower may use it
+  int imported = 0;                                // sweeps of timesteps start .. start + imported - 1 are in root (grown if intervals)
+  std::thread grower;                              // time chunks: imports and grows in time order (grow_in_time_order)
+  bool grower_stop = false;                        // (under m) finalize: every chunk has been imported
 
   Chunk *chunk(int c) {
     std::lock_guard<std::mutex> lk(m);
@@ -182,11 +194,19 @@ struct ftkb_group {
     c.device = ch->device;
     c.start_timestep = cfg.start_timestep + ch->index * B;
     c.resolution_init = res_init;
-    int rc = ftkb_create(&c, &ch->ctx);
+    ftkb_ctx *ctx = nullptr;
+    int rc = ftkb_create(&c, &ctx);
     if (rc) { fail(rc, std::string("chunk context: ") + ftkb_last_error(nullptr)); return rc; }
-    if (coords_mode != FTKB_COORDS_SIMPLE && (rc = ftkb_set_coords(ch->ctx, coords_mode, coords.data(), coords.size())))
-      fail(rc, std::string("chunk context: ") + ftkb_last_error(ch->ctx));
+    if (coords_mode != FTKB_COORDS_SIMPLE && (rc = ftkb_set_coords(ctx, coords_mode, coords.data(), coords.size())))
+      fail(rc, std::string("chunk context: ") + ftkb_last_error(ctx));
+    std::lock_guard<std::mutex> lk(ch->m);
+    ch->ctx = ctx;
     return rc;
+  }
+  // streaming: tell the grower how far the chunk's context has confirmed its sweeps (ct from ftkb::confirmed_through)
+  void note_confirmed(Chunk *ch, int ct) {
+    { std::lock_guard<std::mutex> lk(m); ch->confirmed = ct; }
+    cv.notify_all();
   }
   // after a sweep of a chunk: publish a saturating minimum as soon as one is known (lets the next chunk start early)
   void publish_resolution(Chunk *ch) {
@@ -200,14 +220,28 @@ struct ftkb_group {
   }
   void finish_chunk(Chunk *ch) {
     ftkb_stats st{};
-    int rc = ftkb_get_stats(ch->ctx, &st);
-    uint64_t n = 0;
-    if (!rc) rc = ftkb_num_points(ch->ctx, &n);
-    if (!rc) { ch->points.resize(n); rc = ftkb_get_points(ch->ctx, ch->points.data(), n); }
-    if (rc) fail(rc, std::string("chunk ") + std::to_string(ch->index) + ": " + ftkb_last_error(ch->ctx));
+    int rc, last = INT_MIN;
+    {
+      std::lock_guard<std::mutex> lk(ch->m);
+      rc = ftkb_get_stats(ch->ctx, &st);              // (confirms every sweep)
+      last = ftkb::confirmed_through(ch->ctx);
+      uint64_t n = 0;
+      if (!rc && !streaming) rc = ftkb_num_points(ch->ctx, &n);
+      if (!rc && !streaming) { ch->points.resize(n); rc = ftkb_get_points(ch->ctx, ch->points.data(), n); }
+      if (rc) fail(rc, std::string("chunk ") + std::to_string(ch->index) + ": " + ftkb_last_error(ch->ctx));
+    }
+    if (streaming && !rc) {
+      // the grower copies the points of every sweep from the chunk's device: the context stays until it has
+      note_confirmed(ch, last);
+      std::unique_lock<std::mutex> lk(m);
+      cv.wait(lk, [&] { return failed.load() != FTKB_OK || cfg.start_timestep + imported > last; });
+    }
     ch->stats = st;
-    ftkb_destroy(ch->ctx);            // its layers and buffers go back to the device; the points stay on the host
-    ch->ctx = nullptr;
+    {
+      std::lock_guard<std::mutex> lk(ch->m);
+      ftkb_destroy(ch->ctx);            // its layers and buffers go back to the device; the points stay on the host (or in root)
+      ch->ctx = nullptr;
+    }
     { std::lock_guard<std::mutex> lk(m); ch->resolution_out = st.resolution; ch->finished = true; }
     cv.notify_all();
   }
@@ -274,12 +308,83 @@ extern "C" void ftkb_group_destroy(ftkb_group *g) {
   if (!g) return;
   g->fail(FTKB_ERR_INVALID, "group destroyed");            // releases workers that wait for a predecessor
   for (auto &w : g->workers) w->join();
+  if (g->grower.joinable()) g->grower.join();
   for (auto &ch : g->chunks) if (ch->ctx) ftkb_destroy(ch->ctx);
   for (auto &sl : g->slabs) if (sl.ctx) ftkb_destroy(sl.ctx);
   if (g->root) ftkb_destroy(g->root);
   g->ev_producer.destroy();
   for (auto &e : g->ev_pieces) e.destroy();
   delete g;
+}
+
+// ---- streaming: the merged context grows during the run ---------------------------------------------------------------------
+// one timestep into the merged context: the points of its sweep from every context that swept it, then the grow step if that sweep
+// covered an interval (the last ordinal sweep's points are imported and never grown)
+static int import_and_grow(ftkb_group *g, const std::vector<ftkb_ctx *> &from, int t) {
+  bool interval = false;
+  for (ftkb_ctx *c : from) {
+    bool iv = false;
+    const int rc = ftkb::import_step(g->root, c, t, &iv);
+    if (rc) return rc;
+    interval = interval || iv;
+  }
+  return interval ? ftkb::grow_imported(g->root, t) : FTKB_OK;
+}
+
+// time chunks: the grower thread.  Timestep t is imported and grown once the chunk that owns it has confirmed its sweep and t-1
+// is done; it stops when finalize says every chunk has been imported, or at the first failure.
+static void grow_in_time_order(ftkb_group *g) {
+  for (;;) {
+    const int t = g->cfg.start_timestep + g->imported;
+    const size_t c = (size_t)(g->imported / g->B);
+    Chunk *ch = nullptr;
+    {
+      std::unique_lock<std::mutex> lk(g->m);
+      auto ready = [&] { return c < g->chunks.size() && g->chunks[c]->confirmed >= t; };
+      g->cv.wait(lk, [&] { return g->failed.load() != FTKB_OK || g->grower_stop || ready(); });
+      if (g->failed.load() != FTKB_OK || !ready()) return;
+      ch = g->chunks[c].get();
+    }
+    int rc;
+    std::string msg;
+    {
+      std::lock_guard<std::mutex> rl(g->root_m);
+      std::lock_guard<std::mutex> cl(ch->m);
+      // (no context: a failure elsewhere let its chunk finish without waiting)
+      rc = ch->ctx ? import_and_grow(g, {ch->ctx}, t) : FTKB_ERR_INVALID;
+      if (rc) msg = ch->ctx ? ftkb_last_error(g->root) : "the chunk's context is gone";
+    }
+    if (rc) { g->fail(rc, "streaming grow of timestep " + std::to_string(t) + ": " + msg); return; }
+    { std::lock_guard<std::mutex> lk(g->m); g->imported++; }
+    g->cv.notify_all();
+  }
+}
+
+// the merged context of a streaming group, from its first push on (and, for time chunks, its grower)
+static int ensure_root(ftkb_group *g) {
+  if (!g->streaming || g->root) return FTKB_OK;
+  ftkb_config c = g->cfg;
+  c.device = g->devices[0];
+  int rc = ftkb_create(&c, &g->root);
+  if (rc) { g->error = std::string("merged context: ") + ftkb_last_error(nullptr); return rc; }
+  if ((rc = ftkb_set_streaming_trajectories(g->root, 1))) { g->error = std::string("merged context: ") + ftkb_last_error(g->root); return rc; }
+  if (!g->spatial) g->grower = std::thread(grow_in_time_order, g);
+  return FTKB_OK;
+}
+
+// z-slabs, on the caller's thread while the workers are idle: every timestep that all slabs have confirmed since the last call,
+// in time order, the slabs' points in slab order (the flat simplices of a cut plane come twice: the grow step's sort drops one)
+static int slabs_grow(ftkb_group *g) {
+  if (!g->streaming) return FTKB_OK;
+  std::vector<ftkb_ctx *> from;
+  for (Slab &sl : g->slabs) from.push_back(sl.ctx);
+  for (;;) {
+    const int t = g->cfg.start_timestep + g->imported;
+    for (ftkb_ctx *c : from) if (ftkb::confirmed_through(c) < t) return FTKB_OK;
+    const int rc = import_and_grow(g, from, t);
+    if (rc) { g->error = "streaming grow of timestep " + std::to_string(t) + ": " + ftkb_last_error(g->root); return rc; }
+    g->imported++;
+  }
 }
 
 // ---- spatial mode: every device works on every step ------------------------------------------------------------------------
@@ -358,6 +463,7 @@ static void post_push(ftkb_group *g, int c, std::function<int(ftkb_ctx *)> push,
     int rc = g->failed.load();
     if (!rc) rc = g->ensure_ctx(ch);
     if (!rc) {
+      std::lock_guard<std::mutex> lk(ch->m);
       rc = push(ch->ctx);
       if (rc) g->fail(rc, std::string("push: ") + ftkb_last_error(ch->ctx));
     }
@@ -421,6 +527,7 @@ struct Source {
 struct Staged { double *S = nullptr, *V = nullptr, *J = nullptr; };
 
 static int push_snapshot(ftkb_group *g, const Source src) {
+  { const int rc = ensure_root(g); if (rc) return rc; }
   const int last = src.extent() - 1;
   if (g->spatial)
     // every device copies its planes (ghost planes included) over its own link, concurrently
@@ -472,6 +579,7 @@ static int push_snapshot(ftkb_group *g, const Source src) {
     int rc = g->failed.load();
     if (!rc) rc = g->ensure_ctx(ch);
     if (!rc) {
+      std::lock_guard<std::mutex> lk(ch->m);
       rc = ftkb_push_snapshot(ch->ctx, st->S, st->V, st->J, FTKB_MEM_DEVICE);      // copied (and synchronised) before it returns
       if (rc) g->fail(rc, std::string("push: ") + ftkb_last_error(ch->ctx));
     }
@@ -655,6 +763,7 @@ extern "C" int ftkb_group_get_slab(const ftkb_group *g, int32_t s, int32_t plane
 extern "C" int ftkb_group_push_synthetic(ftkb_group *g, int kind, const double *params, int nparams, double t) {
   if (!g || nparams < 0 || nparams > 8 || (nparams && !params)) return FTKB_ERR_INVALID;
   std::vector<double> p(params, params + nparams);
+  { const int rc = ensure_root(g); if (rc) return rc; }
   if (g->spatial) return spatial_push(g, [=](Slab &sl) { return ftkb_push_synthetic(sl.ctx, kind, p.data(), (int)p.size(), t); });
   return push_layer(g, [=](ftkb_ctx *c) { return ftkb_push_synthetic(c, kind, p.data(), (int)p.size(), t); }, false);
 }
@@ -669,9 +778,15 @@ static int post_sweep(ftkb_group *g, int step, bool advance) {
     int rc = g->failed.load();
     if (!rc) rc = g->ensure_ctx(ch);
     if (rc) return;
-    rc = advance ? ftkb_advance_timestep(ch->ctx) : ftkb_update_timestep(ch->ctx);
-    if (rc) { g->fail(rc, std::string("sweep: ") + ftkb_last_error(ch->ctx)); return; }
-    g->publish_resolution(ch);
+    int ct = INT_MIN;
+    {
+      std::lock_guard<std::mutex> lk(ch->m);
+      rc = advance ? ftkb_advance_timestep(ch->ctx) : ftkb_update_timestep(ch->ctx);
+      if (rc) { g->fail(rc, std::string("sweep: ") + ftkb_last_error(ch->ctx)); return; }
+      g->publish_resolution(ch);
+      ct = ftkb::confirmed_through(ch->ctx);
+    }
+    if (g->streaming) g->note_confirmed(ch, ct);
     if (last_of_chunk || !advance) g->finish_chunk(ch);
   });
   return FTKB_OK;
@@ -681,7 +796,11 @@ extern "C" int ftkb_group_advance_timestep(ftkb_group *g) {
   if (!g) return FTKB_ERR_INVALID;
   if (g->npushed < g->nadvanced + 2) { g->error = "advance_timestep: two snapshots are needed"; return FTKB_ERR_INVALID; }
   g->nintervals = std::max(g->nintervals, g->nadvanced + 1);
-  if (g->spatial) { g->nadvanced++; return on_all_slabs(g, [](Slab &sl) { return ftkb_advance_timestep(sl.ctx); }, "sweep"); }
+  if (g->spatial) {
+    g->nadvanced++;
+    const int rc = on_all_slabs(g, [](Slab &sl) { return ftkb_advance_timestep(sl.ctx); }, "sweep");
+    return rc ? rc : slabs_grow(g);
+  }
   return post_sweep(g, g->nadvanced++, true);
 }
 
@@ -689,31 +808,25 @@ extern "C" int ftkb_group_update_timestep(ftkb_group *g) {
   if (!g) return FTKB_ERR_INVALID;
   if (g->npushed < g->nadvanced + 1) { g->error = "update_timestep: no snapshot has been pushed"; return FTKB_ERR_INVALID; }
   if (g->npushed >= g->nadvanced + 2) g->nintervals = std::max(g->nintervals, g->nadvanced + 1);     // the next snapshot is there
-  if (g->spatial) return on_all_slabs(g, [](Slab &sl) { return ftkb_update_timestep(sl.ctx); }, "sweep");
+  if (g->spatial) {
+    const int rc = on_all_slabs(g, [](Slab &sl) { return ftkb_update_timestep(sl.ctx); }, "sweep");
+    return rc ? rc : slabs_grow(g);
+  }
   return post_sweep(g, g->nadvanced, false);
 }
 
 // The merged context on the first device: the punctured simplices of every chunk or slab, sorted and deduplicated there, then
-// traced offline -- or, with streaming trajectories, grown once per swept interval t, in time order, over the points of
-// timestep t.  The points of the last ordinal sweep are imported but never grown.
+// traced offline -- or, with streaming trajectories, the context that has grown them during the run: it publishes what it grew.
 static int build_root(ftkb_group *g, const std::vector<const std::vector<ftkb_point> *> &parts) {
-  if (g->root) { ftkb_destroy(g->root); g->root = nullptr; }
-  ftkb_config c = g->cfg;
-  c.device = g->devices[0];
-  int rc = ftkb_create(&c, &g->root);
-  if (rc) { g->error = ftkb_last_error(nullptr); return rc; }
+  int rc = FTKB_OK;
   if (g->streaming) {
-    std::vector<ftkb_point> all;
-    for (auto *p : parts) all.insert(all.end(), p->begin(), p->end());
-    std::stable_sort(all.begin(), all.end(), [](const ftkb_point &a, const ftkb_point &b) { return a.timestep < b.timestep; });
-    rc = ftkb_set_streaming_trajectories(g->root, 1);
-    if (!rc) rc = ftkb_import_points(g->root, all.data(), all.size());
-    for (int k = 0; !rc && k < g->nintervals; k++) {
-      const int t = g->cfg.start_timestep + k;
-      const auto end = std::upper_bound(all.begin(), all.end(), t, [](int s, const ftkb_point &p) { return s < p.timestep; });
-      rc = ftkb::grow_imported(g->root, (uint64_t)(end - all.begin()));
-    }
+    if ((rc = ensure_root(g))) return rc;
   } else {
+    if (g->root) { ftkb_destroy(g->root); g->root = nullptr; }
+    ftkb_config c = g->cfg;
+    c.device = g->devices[0];
+    rc = ftkb_create(&c, &g->root);
+    if (rc) { g->error = ftkb_last_error(nullptr); return rc; }
     // (the flat simplices of a cut plane were found by both neighbouring slabs: the root's sort drops the duplicates)
     for (auto *p : parts)
       if (!rc && !p->empty()) rc = ftkb_import_points(g->root, p->data(), p->size());
@@ -727,13 +840,15 @@ extern "C" int ftkb_group_finalize(ftkb_group *g, ftkb_ctx **root) {
   if (!g || !root) return FTKB_ERR_INVALID;
   *root = nullptr;
   if (g->spatial) {
-    int rc = on_all_slabs(g, [](Slab &sl) {
+    const bool streaming = g->streaming;
+    int rc = on_all_slabs(g, [streaming](Slab &sl) {
       uint64_t n = 0;
       int r = ftkb_get_stats(sl.ctx, &sl.stats);
-      if (!r) r = ftkb_num_points(sl.ctx, &n);
-      if (!r) { sl.points.resize(n); r = ftkb_get_points(sl.ctx, sl.points.data(), n); }
+      if (!r && !streaming) r = ftkb_num_points(sl.ctx, &n);
+      if (!r && !streaming) { sl.points.resize(n); r = ftkb_get_points(sl.ctx, sl.points.data(), n); }
       return r;
     }, "collect");
+    if (!rc) rc = slabs_grow(g);     // streaming: what the last sweeps confirmed, the last ordinal sweep included
     if (rc) return rc;
     std::vector<const std::vector<ftkb_point> *> parts;
     for (auto &sl : g->slabs) parts.push_back(&sl.points);
@@ -753,6 +868,12 @@ extern "C" int ftkb_group_finalize(ftkb_group *g, ftkb_ctx **root) {
   // chunks that never reached their last sweep (the series ended inside them, without a final update): collect them as they are
   for (auto &ch : g->chunks)
     if (ch->ctx && !ch->finished) g->finish_chunk(ch.get());
+  if (g->grower.joinable()) {
+    // every chunk has finished, so every sweep has been imported: the grower has nothing left to wait for
+    { std::lock_guard<std::mutex> lk(g->m); g->grower_stop = true; }
+    g->cv.notify_all();
+    g->grower.join();
+  }
   if (g->failed.load()) return g->failed.load();
   std::vector<const std::vector<ftkb_point> *> parts;
   for (auto &ch : g->chunks) parts.push_back(&ch->points);
@@ -760,6 +881,45 @@ extern "C" int ftkb_group_finalize(ftkb_group *g, ftkb_ctx **root) {
   if (rc) return rc;
   *root = g->root;
   return FTKB_OK;
+}
+
+extern "C" int ftkb_group_get_live_curveset(ftkb_group *g, int32_t *grown_through, ftkb_curveset **out) {
+  if (!g) return FTKB_ERR_INVALID;
+  auto refuse = [g](const std::string &msg) { std::lock_guard<std::mutex> lk(g->m); g->error = "get_live_curveset: " + msg; return FTKB_ERR_INVALID; };
+  if (!grown_through || !out) return refuse("null argument");
+  *out = nullptr;
+  if (!g->streaming) return refuse("streaming trajectories are off (ftkb_group_set_streaming_trajectories)");
+  if (g->failed.load()) return g->failed.load();
+  int rc = ensure_root(g);
+  if (rc) return rc;
+  if (g->spatial) {
+    // confirm the slabs' deferred sweeps, then import and grow them
+    rc = on_all_slabs(g, [](Slab &sl) { ftkb_stats st; return ftkb_get_stats(sl.ctx, &st); }, "confirm");
+    if (!rc) rc = slabs_grow(g);
+    if (rc) return rc;
+  } else if (g->nintervals > 0) {
+    // the chunk that swept the last interval confirms it (its worker runs this behind that sweep), then the grower catches up
+    Chunk *ch = g->chunk((g->nintervals - 1) / g->B);
+    g->workers[ch->index % g->workers.size()]->post([g, ch] {
+      int ct = INT_MIN;
+      {
+        std::lock_guard<std::mutex> lk(ch->m);
+        if (!ch->ctx) return;
+        ftkb_stats st;
+        const int r = ftkb_get_stats(ch->ctx, &st);
+        if (r) { g->fail(r, std::string("confirm: ") + ftkb_last_error(ch->ctx)); return; }
+        ct = ftkb::confirmed_through(ch->ctx);
+      }
+      g->note_confirmed(ch, ct);
+    });
+    std::unique_lock<std::mutex> lk(g->m);
+    g->cv.wait(lk, [g] { return g->failed.load() != FTKB_OK || g->imported >= g->nintervals; });
+    if (g->failed.load()) return g->failed.load();
+  }
+  std::lock_guard<std::mutex> rl(g->root_m);
+  rc = ftkb_get_live_curveset(g->root, grown_through, out);
+  if (rc) { std::lock_guard<std::mutex> lk(g->m); g->error = std::string("get_live_curveset: ") + ftkb_last_error(g->root); }
+  return rc;
 }
 
 extern "C" int ftkb_group_get_stats(ftkb_group *g, ftkb_stats *sum, int32_t *chunks_done) {

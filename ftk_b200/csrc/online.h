@@ -68,9 +68,9 @@ class OnlineTracer {
   bool have_points_ = true;
 };
 
-// (context.cpp) one grow step of a streaming context over its imported points [grown so far, end): how a device group's merged
-// context replays the grow steps of the chunks or slabs that swept for it (group.cpp)
-int grow_imported(ftkb_ctx *c, uint64_t end);
+// (context.cpp) one grow step of a streaming context over the points imported since its last one, as the batch of timestep t:
+// how a device group's merged context grows the trajectories of the chunks or slabs that sweep for it (group.cpp)
+int grow_imported(ftkb_ctx *c, int t);
 
 // One source of a layer's planes [first, first + count) along the slowest axis (z in 3D, y in 2D) of the context's array: the
 // arrays start at plane `first` and live on `device`; every copy from them waits for `after` unless it is null.
@@ -85,6 +85,13 @@ struct Segment {
 // is on another device than the context's.  How a device group feeds its contexts from a device snapshot (one segment) or from
 // snapshot pieces (group.cpp); ftkb_push_snapshot is the one-segment case for its own memory kinds.
 int push_segments(ftkb_ctx *c, const Segment *segs, int n);
+// (context.cpp) the last timestep whose sweep `c` has confirmed (start_timestep - 1: none yet); waits for nothing
+int confirmed_through(const ftkb_ctx *c);
+// (context.cpp) appends the points `src` found in its confirmed sweep of timestep t to the imported points of the streaming
+// context `dst`, device to device: a peer copy when the two live on different devices, never through the host.  *interval: that
+// sweep covered the interval [t, t+1] (an advance), so the points make up a grow step.  The copy is complete on return; neither
+// context may be used by another thread meanwhile.
+int import_step(ftkb_ctx *dst, ftkb_ctx *src, int t, bool *interval);
 // (context.cpp) lets `device` read `peer`'s memory where the hardware allows it, once per pair; makes `device` current
 cudaError_t enable_peer_access(int device, int peer);
 

@@ -40,6 +40,14 @@ class CurveSet:
         tracker._check(L.lib().ftkb_get_curveset(tracker._h, C.byref(h)))
         return cls(h)
 
+    @classmethod
+    def live(cls, get, handle, check):
+        """(grown_through, CurveSet) of a streaming tracker or group at any time: `get` is ftkb_get_live_curveset or
+        ftkb_group_get_live_curveset, `check` turns its return code into an exception"""
+        h, t = C.c_void_p(), C.c_int32()
+        check(get(handle, C.byref(t), C.byref(h)))
+        return t.value, cls(h)
+
     def post_process(self, ops):
         rc = L.lib().ftkb_curveset_post_process(self._h, ops.encode())
         if rc:

@@ -199,6 +199,12 @@ class GroupTracker:
         self._root = view
         return view
 
+    def live_curveset(self):
+        """streaming groups, at any time: (grown_through, CurveSet) after the grow steps of every interval swept so far --
+        call for call what Tracker.live_curveset of one tracker fed the same series returns"""
+        from .curves import CurveSet
+        return CurveSet.live(L.lib().ftkb_group_get_live_curveset, self._g, self._check)
+
     def stats(self):
         s, n = L.Stats(), C.c_int32()
         self._check(L.lib().ftkb_group_get_stats(self._g, C.byref(s), C.byref(n)))

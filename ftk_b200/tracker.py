@@ -374,6 +374,13 @@ class _RegularTracker:
         self._check(L.lib().ftkb_get_trajectory_complete(self._h, out.ctypes.data))
         return out[:nt.value].astype(bool)
 
+    def live_curveset(self):
+        """streaming trackers, at any time: (grown_through, CurveSet) -- the trajectories grown so far (the reference's
+        traced_critical_points) and the last timestep whose grow step has run (start timestep - 1 before the first);
+        CurveSet.slice(t) holds the points of timestep t once t <= grown_through.  Equal to CurveSet.from_tracker after finalize."""
+        from .curves import CurveSet
+        return CurveSet.live(L.lib().ftkb_get_live_curveset, self._h, self._check)
+
     def get_traced_critical_points(self):
         """list of trajectories, each a structured array of points in trace order (with .loop in the
         second tuple member); the counterpart of feature_curve_set_t"""

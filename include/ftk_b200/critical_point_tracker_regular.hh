@@ -397,6 +397,8 @@ class critical_point_tracker_regular {
     if (ctx_) { ftkb_destroy(ctx_); ctx_ = nullptr; }
     traced_.clear();
     points_valid_ = false;
+    finalized_ = false;
+    sweeps_ = refreshed_sweeps_ = 0;
   }
 
   // ---- inputs: critical_point_tracker.hh:202-229 ------------------------------------------------
@@ -474,8 +476,8 @@ class critical_point_tracker_regular {
   }
 
   // ---- stepping: critical_point_tracker.hh:841-848, *_regular.hh update_timestep ------------------
-  void update_timestep() { need(); if (group_) gcheck(ftkb_group_update_timestep(group_)); else check(ftkb_update_timestep(ctx_)); points_valid_ = false; }
-  bool advance_timestep() { need(); if (group_) gcheck(ftkb_group_advance_timestep(group_)); else check(ftkb_advance_timestep(ctx_)); points_valid_ = false; return true; }
+  void update_timestep() { need(); if (group_) gcheck(ftkb_group_update_timestep(group_)); else check(ftkb_update_timestep(ctx_)); points_valid_ = false; sweeps_++; }
+  bool advance_timestep() { need(); if (group_) gcheck(ftkb_group_advance_timestep(group_)); else check(ftkb_advance_timestep(ctx_)); points_valid_ = false; sweeps_++; return true; }
   int get_current_timestep() const { int32_t t = start_timestep_; if (ctx_) ftkb_current_timestep(ctx_, &t); return t; }
 
   // ---- finalize: critical_point_tracker_2d_regular.hh:143-225, critical_point_tracker.hh:668-817 --
@@ -483,6 +485,7 @@ class critical_point_tracker_regular {
     need();
     ensure_root();     // several devices: merged into one context on the first device, traced there
     check(ftkb_finalize(ctx_));
+    finalized_ = true;
     fetch_points();
     uint64_t nt = 0;
     check(ftkb_num_trajectories(ctx_, &nt));
@@ -516,33 +519,27 @@ class critical_point_tracker_regular {
       ftkb_curveset_destroy(cs);
       throw std::runtime_error("ftk_b200: " + msg);
     }
-    uint64_t nc = 0, np = 0;
-    ftkb_curveset_size(cs, &nc, &np);
-    std::vector<ftkb_curve_info> infos(nc ? nc : 1);
-    std::vector<ftkb_curve_point> pts(np ? np : 1);
-    ftkb_curveset_get(cs, infos.data(), pts.data());
+    load_curveset(cs);
     ftkb_curveset_destroy(cs);
-    traced_.clear();
-    for (uint64_t i = 0; i < nc; i++) {
-      const ftkb_curve_info &in = infos[i];
-      feature_curve_t c;
-      for (uint64_t k = in.first; k < in.first + in.count; k++) {
-        feature_point_t p = to_feature_point(pts[k].p);
-        p.v = {{pts[k].v[0], pts[k].v[1], pts[k].v[2]}};
-        p.id = (unsigned long long)pts[k].id;
-        c.push_back(p);
-      }
-      c.id = in.id; c.loop = in.loop != 0; c.complete = in.complete != 0; c.consistent_type = in.consistent_type;
-      c.tmin = in.tmin; c.tmax = in.tmax;
-      c.min = {{in.smin, 0, 0}}; c.max = {{in.smax, 0, 0}}; c.persistence = {{in.persistence, 0, 0}};
-      c.bbmin = {{in.bbmin[0], in.bbmin[1], in.bbmin[2]}}; c.bbmax = {{in.bbmax[0], in.bbmax[1], in.bbmax[2]}};
-      traced_.insert(std::make_pair(in.id, c));
-    }
   }
 
   // ---- results: critical_point_tracker.hh:68-69,105, critical_point_tracker_regular.hh:24-38 ------
   const feature_curve_set_t &get_traced_critical_points() const { return traced_; }
-  feature_curve_set_t &get_traced_critical_points() { return traced_; }
+  // With streaming trajectories the reference's traced set is live: trace_critical_points_online updates it after every interval
+  // sweep.  So before finalize, after any sweep since the last call, this refreshes it from the trajectories grown so far (the
+  // const overload returns it as last refreshed).
+  feature_curve_set_t &get_traced_critical_points() {
+    if (streaming_ && !finalized_ && (ctx_ || group_) && refreshed_sweeps_ != sweeps_) {
+      ftkb_curveset *cs = nullptr;
+      int32_t grown_through = 0;
+      if (group_) gcheck(ftkb_group_get_live_curveset(group_, &grown_through, &cs));
+      else check(ftkb_get_live_curveset(ctx_, &grown_through, &cs));
+      load_curveset(cs);
+      ftkb_curveset_destroy(cs);
+      refreshed_sweeps_ = sweeps_;
+    }
+    return traced_;
+  }
   std::vector<feature_point_t> get_critical_points() { need(); fetch_points(); return points_; }
   std::vector<feature_point_t> get_discrete_critical_points() { return get_critical_points(); }
 
@@ -610,6 +607,31 @@ class critical_point_tracker_regular {
   void ensure_root() { if (group_ && !ctx_) gcheck(ftkb_group_finalize(group_, &ctx_)); }
   void gcheck(int rc) const { if (rc != FTKB_OK) throw std::runtime_error(std::string("ftk_b200: ") + ftkb_group_last_error(group_)); }
   void check(int rc) const { if (rc != FTKB_OK) throw std::runtime_error(std::string("ftk_b200: ") + ftkb_last_error(ctx_)); }
+  // the curves of a library curve set, in its multimap order, as the traced set
+  void load_curveset(const ftkb_curveset *cs) {
+    uint64_t nc = 0, np = 0;
+    ftkb_curveset_size(cs, &nc, &np);
+    std::vector<ftkb_curve_info> infos(nc ? nc : 1);
+    std::vector<ftkb_curve_point> pts(np ? np : 1);
+    ftkb_curveset_get(cs, infos.data(), pts.data());
+    traced_.clear();
+    for (uint64_t i = 0; i < nc; i++) {
+      const ftkb_curve_info &in = infos[i];
+      feature_curve_t c;
+      for (uint64_t k = in.first; k < in.first + in.count; k++) {
+        feature_point_t p = to_feature_point(pts[k].p);
+        p.v = {{pts[k].v[0], pts[k].v[1], pts[k].v[2]}};
+        p.id = (unsigned long long)pts[k].id;
+        c.push_back(p);
+      }
+      c.id = in.id; c.loop = in.loop != 0; c.complete = in.complete != 0; c.consistent_type = in.consistent_type;
+      c.tmin = in.tmin; c.tmax = in.tmax;
+      c.min = {{in.smin, 0, 0}}; c.max = {{in.smax, 0, 0}}; c.persistence = {{in.persistence, 0, 0}};
+      c.bbmin = {{in.bbmin[0], in.bbmin[1], in.bbmin[2]}}; c.bbmax = {{in.bbmax[0], in.bbmax[1], in.bbmax[2]}};
+      traced_.insert(std::make_pair(in.id, c));
+    }
+  }
+
 
   void fetch_points() {
     if (points_valid_) return;
@@ -664,6 +686,8 @@ class critical_point_tracker_regular {
   std::vector<std::string> scalar_components_{"scalar"};
   std::vector<feature_point_t> points_;
   bool points_valid_ = false;
+  bool finalized_ = false;
+  uint64_t sweeps_ = 0, refreshed_sweeps_ = 0;     // update / advance calls; their count at the last refresh of traced_
   feature_curve_set_t traced_;
   std::map<int, std::vector<feature_point_t>> sliced_;
 };

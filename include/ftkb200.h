@@ -240,11 +240,15 @@ int ftkb_push_snapshot_remote(ftkb_ctx *, const double *scalar, const double *ve
  * Options, valid only before the first push (afterwards FTKB_ERR_INVALID):
  *   ftkb_group_set_coords                   ftkb_set_coords for the whole array: same modes and sizes, host data copied before
  *                                           the call returns; every chunk / slab context sweeps with it.
- *   ftkb_group_set_streaming_trajectories   chunks and slabs still sweep offline; ftkb_group_finalize then runs the grow step
- *                                           of ftkb_set_streaming_trajectories on the merged context once per swept interval t,
- *                                           in time order, over its sorted points of timestep t -- the batch a single streaming
- *                                           context grows at t -- and publishes trajectories, loop and complete flags as a
- *                                           streaming context's ftkb_finalize does.
+ *   ftkb_group_set_streaming_trajectories   the merged context on device_ids[0] exists from the first push and grows during the
+ *                                           run: once the sweep of interval t is confirmed (by every z-slab, or by the chunk that
+ *                                           owns t) and t-1 has been grown, its points are copied there device to device and the
+ *                                           grow step of ftkb_set_streaming_trajectories runs over them -- the batch a single
+ *                                           streaming context grows at t.  Grows run in time order, may lag the sweeps by a step
+ *                                           or two (time chunks grow on a thread of their own), and ftkb_group_get_live_curveset
+ *                                           reads them at any time.  ftkb_group_finalize waits for the last grow, imports the
+ *                                           last ordinal sweep's points (they join no trajectory) and publishes trajectories,
+ *                                           loop and complete flags as a streaming context's ftkb_finalize does.
  *
  * chunk_timesteps = 0 selects the SPATIAL decomposition instead (3D only; the reference's own, regular_tracker.hh:126-149):
  * device s holds a z-slab of every snapshot -- its share of the domain's corner planes, the corner plane above (whose flat
@@ -357,8 +361,18 @@ typedef struct ftkb_curveset ftkb_curveset;
 /* trajectories as CSR over a point array (what ftkb_get_trajectories returns); curves get ids 0 .. ntraj-1 */
 int ftkb_curveset_create(const ftkb_point *pts, uint64_t npts, const uint64_t *offsets, const uint64_t *point_idx,
                          const uint8_t *loop, uint64_t ntraj, ftkb_curveset **out);
-/* get_traced_critical_points() of a finalized context; the caller destroys the set */
+/* get_traced_critical_points() of a finalized context (mid-run, of a streaming one: ftkb_get_live_curveset); the caller
+ * destroys the set */
 int ftkb_get_curveset(ftkb_ctx *, ftkb_curveset **out);
+/* the trajectories a streaming context has grown so far, at any time during the run (the reference's traced_critical_points,
+ * which trace_critical_points_online keeps current): the curve set ftkb_get_curveset builds after ftkb_finalize -- curves in id
+ * order, points in trace order, loop and complete flags, statistics -- and, after ftkb_finalize, equal to it.  *grown_through
+ * receives the last timestep whose grow step has run (start_timestep - 1 before the first).  The query changes no later
+ * result.  A context without streaming trajectories, or a NULL argument, gets FTKB_ERR_INVALID.  The caller destroys the set. */
+int ftkb_get_live_curveset(ftkb_ctx *, int32_t *grown_through, ftkb_curveset **out);
+/* the same for a group with ftkb_group_set_streaming_trajectories: first waits for the grow steps of every interval the caller
+ * has swept (advanced over), so that the answer equals, call for call, that of one context fed the same series */
+int ftkb_group_get_live_curveset(ftkb_group *, int32_t *grown_through, ftkb_curveset **out);
 void ftkb_curveset_destroy(ftkb_curveset *);
 int ftkb_curveset_post_process(ftkb_curveset *, const char *ops);
 int ftkb_curveset_size(const ftkb_curveset *, uint64_t *ncurves, uint64_t *npoints);
